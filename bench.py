@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (default)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU code on the host cores
+    python bench.py --gpus N --steps K --dump-outputs DIR    # default workload: also write rank 0's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[3]): 65,536-column synthetic perturbed-profile ensemble PER GPU,
 repwvl-100 table (100 wavelengths x 20 layers x 30 angles), one "step" = one full reference loop
@@ -279,6 +280,24 @@ def timed_loop(torch, rdist, stream, world, steps, one_step, finish):
     return (rdist.max_over_ranks(ms) if world > 1 else ms), res
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6 - (1 << 16)  # 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, state, scalars, seed=2024):
+    """Writes the solver state after the last timed step (per-column arrays, as rcm_get_state returns them) and that step's
+    ensemble scalars as <out_dir>/<name>.npy, so that two builds run with the same arguments can be compared array for
+    array.  Above DUMP_LIMIT_BYTES a fixed, seeded sample of the columns is written; columns.npy names the ones kept."""
+    ncol = next(iter(state.values())).shape[0]
+    per_col = sum(a.nbytes for a in state.values()) // ncol + 8  # + the float64 column index
+    keep = max(1, (DUMP_LIMIT_BYTES - scalars.nbytes) // per_col)
+    cols = np.arange(ncol) if ncol <= keep else np.sort(np.random.default_rng(seed).choice(ncol, size=keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in state.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[cols])
+    np.save(os.path.join(out_dir, "columns.npy"), cols.astype(np.float64))
+    np.save(os.path.join(out_dir, "step_scalars.npy"), scalars.astype(np.float64))
+
+
 def oracle_parity(rcm, st, solver, nsteps, nwvl, n_check=64, seed=2024):
     """Ties the timed run to the oracle: n_check seeded members of THIS run's ensemble are taken through the same
     `nsteps` iterations by the reference (oracle/_ref, else the C port) from the initial state and compared with
@@ -360,6 +379,8 @@ def run_b200(args, rank, world, local_rank):
     k_ms, k_n = solver.kernel_time_ms(reset=True)
     value = world * units_per_step * args.steps / (ms_total * 1e-3)
     k_ms_ranks = gather_floats(rdist, torch, k_ms, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, solver.get_state(), scal.cpu().numpy())
 
     # ---- parity of THIS run against the oracle (rank 0, 64 seeded members, all the steps done so far) ------------
     parity = oracle_parity(rcm, st, solver, args.warmup + args.steps, nwvl) if rank == 0 and not args.no_parity else None
@@ -673,7 +694,11 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling block (one ensemble over the ranks)")
     ap.add_argument("--strong-total", type=int, default=65536, help="columns of the strong-scaling ensemble (N > 1)")
     ap.add_argument("--ring", type=int, default=32, help="slots of the asynchronous scalar exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's state and last-step scalars as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "repwvl"):
+        ap.error("--dump-outputs writes the outputs of the default workload (--impl b200 --workload repwvl)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     rank, world, local_rank = _env_int("RANK", 0), _env_int("WORLD_SIZE", 1), _env_int("LOCAL_RANK", 0)

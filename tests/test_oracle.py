@@ -116,16 +116,23 @@ def test_golden_survey_anchor_values(golden):
     assert abs(golden["s1_dt_100"][0] - 13205.7) < 0.05 and abs(golden["s1_Tsurf_100"][0] - 293.919442) < 1e-6
 
 
-@needs_ref
-def test_reference_live_equals_golden_and_port(port, golden):
+def test_reference_live_equals_golden_and_port(port, golden, golden_misc):
+    """The reference-built oracle when oracle/_ref is built; otherwise the outputs the reference stored in the golden files
+    (solar setup, initial state) stand in for it and the port's run is the one checked."""
     g = golden
-    sol = R.solar()
-    assert sol["solar_irr"] == float(g["solar_irr"]) == port.solar_setup()["solar_irr"]
-    r = R.advance(table_path(100), g["plevel"], g["rel_hum"][:3], sol["solar_irr"], g["Tlayer"][:3], g["Tsurf"][:3],
-                  g["vmr9"][:3], 5)
+    if R.available():
+        sol = R.solar()
+    else:
+        sol = {k: float(golden_misc["solar_" + k]) for k in port.solar_setup()}
+    assert sol == port.solar_setup() and sol["solar_irr"] == float(g["solar_irr"])
+    args = (g["plevel"], g["rel_hum"][:3], sol["solar_irr"], g["Tlayer"][:3], g["Tsurf"][:3], g["vmr9"][:3], 5)
+    r = R.advance(table_path(100), *args) if R.available() else port.advance(port.load_rcmtab(table_path(100)), *args)
     for k in ("E_down", "E_up", "dE", "Tlayer", "Tsurf"):
         assert np.array_equal(r[k], g[f"s5_{k}_100"][:3]), k
-    st = R.init_columns(g["plevel"], g["Tlevel"], g["vmr_ppm_level"])
+    if R.available():
+        st = R.init_columns(g["plevel"], g["Tlevel"], g["vmr_ppm_level"])
+    else:
+        st = {k: g["init_" + k] if "init_" + k in g.files else g[k] for k in ("Tlayer", "vmr9", "rel_hum", "player", "conv")}
     sp = port.init_columns(g["plevel"], g["Tlevel"], g["vmr_ppm_level"])
     for k in st:
         assert np.array_equal(st[k], sp[k]) and np.array_equal(st[k][:14] if st[k].ndim > 1 else st[k],
@@ -183,7 +190,6 @@ def test_lbl_step_sweeps_equal_the_reference_radiative_transfer_by_linearity(por
     assert Eu[0] > 1.0 and Ed[20] > 1.0                          # a real thermal spectrum, not zeros
 
 
-@needs_ref
 def test_port_reaches_the_reference_equilibrium_for_a_perturbed_member(port, golden, golden_eq):
     """The C port over 6,000 iterations == the unmodified reference (tests/golden/ref_equilibrium.npz), bit for bit, for the
     most strongly perturbed member of the fixture (T_surface 297.8 K at equilibrium)."""
