@@ -225,6 +225,21 @@ int rcm_get_state(rcm_solver* s, double* Tlayer, double* Tsurf, double* h2o, flo
 int rcm_save_checkpoint(rcm_solver* s, const char* path);
 int rcm_load_checkpoint(rcm_solver* s, const char* path);
 int rcm_column_count(const rcm_solver* s); /* columns currently loaded (rcm_set_columns / rcm_load_checkpoint) */
+/* Diagnostic radiation call: the thermal fluxes the NEXT step of the resident ensemble would compute - after its theta-sort
+ * and water-vapour feedback, with its grey cloud and solar forcing (main.cpp:536-574) - for the columns [col0, col0 + ncol),
+ * per wavelength, optionally with the active species' VMRs scaled.  Changes nothing: state, step counter, scalars and every
+ * later step stay bit-identical.  With step_index 0 tau comes from the initial, unsorted profile as in the first step.
+ * vmr_scale [nactive] (ascending species index, as vmr_active; NULL = all 1): factor on each active species' layer VMRs as
+ * that step would use them (H2O: after the feedback), one rounded multiplication.
+ * Outputs (host, any may be NULL): E_down_spec / E_up_spec [ncol][nwvl][21], the contribution of each wavelength (its
+ * spectral weight included); E_down / E_up [ncol][21] = those summed over the wavelengths in index order; dE [ncol][20] from
+ * them as main.cpp:337-341 (the column's own solar_irr in the lowest layer).  Synchronous.  Works through the range in
+ * chunks of at most 8,192 columns with device scratch of its own (about 0.6 GB for 100 wavelengths).
+ * Errors: RCM_ERR_ARG for a range outside the loaded columns or a scale that is negative or not finite; RCM_ERR_STATE without
+ * table or columns, on the line-by-line path, with another species_mask than the default's five species, or with
+ * RCM_OPT_PATH 1. */
+int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
+                        double* E_down, double* E_up, double* dE);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

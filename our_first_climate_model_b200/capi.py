@@ -394,6 +394,26 @@ class Solver:
         _check(_lib.rcm_radiative_transfer(self._h, _p(t), _p(Ed), _p(Eu), _p(dE)), self._h)
         return Ed, Eu, dE
 
+    def diagnose_fluxes(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, spectral: bool = True) -> dict:
+        """rcm_diagnose_fluxes: the fluxes the next step would compute for columns [col0, col0 + ncol), without changing
+        anything.  vmr_scale [nactive]: factors on the active species' VMRs (ascending species index; None = unscaled).
+        -> E_down, E_up [ncol, 21], dE [ncol, 20] and, with spectral, E_down_spec / E_up_spec [ncol, nwvl, 21]."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = None
+        if vmr_scale is not None:
+            sc = _f64(vmr_scale).ravel()
+            if sc.size != self.nactive:
+                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        m = max(n, 0)
+        out = dict(E_down=np.zeros((m, NLEV)), E_up=np.zeros((m, NLEV)), dE=np.zeros((m, NLAY)))
+        if spectral:
+            out["E_down_spec"] = np.zeros((m, self.nwvl, NLEV))
+            out["E_up_spec"] = np.zeros((m, self.nwvl, NLEV))
+        _check(_lib.rcm_diagnose_fluxes(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(out.get("E_down_spec")),
+                                        _p(out.get("E_up_spec")), _p(out["E_down"]), _p(out["E_up"]), _p(out["dE"])),
+               self._h)
+        return out
+
     def advance(self, nsteps: int, want_scalars=True):
         sc = (StepScalars * nsteps)() if want_scalars else None
         _check(_lib.rcm_advance(self._h, C.c_int(nsteps), sc), self._h)

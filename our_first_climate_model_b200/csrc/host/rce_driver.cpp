@@ -8,6 +8,7 @@
 //
 //   rcm_rce --atm test.atm --table Reduced100Forcing.nc [--ncol N] [--seed S] [--max-steps M] [--check-every K]
 //           [--dT 1e-3] [--device D] [--out output.txt] [--checkpoint file] [--resume file] [--steps-exact]
+//           [--spectral-out spectrum.csv]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
@@ -21,8 +22,14 @@
 // reference's only call of that reader); a six-column .atm (lbl.arts/README:1-3) gets the well-mixed CO2 / CH4 / N2O of
 // lbl.arts/README:13-16.  The tables hold the optical depths of the file's own column: member 0's H2O and O3.
 //
+// --spectral-out FILE (repwvl tables only): after the run, the radiation the next step would see (rcm_diagnose_fluxes) per
+// wavelength - header "wvl_nm,weight,olr,surface_down", then one row per wavelength with the ensemble means of the TOA upward
+// and the surface downward flux of that wavelength (W/m2, its spectral weight included), summed in column order: the file is
+// byte-identical for any --gpus N.
+//
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <cstdio>
@@ -70,9 +77,52 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     std::string resume, ckpt;
     double *T_out, *Ts_out, *Eu_out;
     float* time_out;
+    int spec_nwvl;            // > 0: --spectral-out, rows [ncol][spec_nwvl] of olr / sfc
+    double *olr_out, *sfc_out;
 };
 
 std::atomic<int> g_failed{0};
+
+// TOA E_up and surface E_down of every (column, wavelength) of the n columns of s: olr / sfc [n][nwvl]
+int diagnose_spectrum(rcm_solver* s, int n, int nwvl, double* olr, double* sfc) {
+    constexpr int NLEV = RCM_NLEVEL, CHUNK = 4096;
+    std::vector<double> dn((size_t)std::min(n, CHUNK) * nwvl * NLEV), up(dn.size());
+    for (int c0 = 0; c0 < n; c0 += CHUNK) {
+        const int m = std::min(CHUNK, n - c0);
+        const int st = rcm_diagnose_fluxes(s, c0, m, nullptr, dn.data(), up.data(), nullptr, nullptr, nullptr);
+        if (st != RCM_OK) return st;
+        for (size_t c = 0; c < (size_t)m; ++c)
+            for (size_t w = 0; w < (size_t)nwvl; ++w) {
+                olr[(c0 + c) * nwvl + w] = up[(c * nwvl + w) * NLEV];
+                sfc[(c0 + c) * nwvl + w] = dn[(c * nwvl + w) * NLEV + NLEV - 1];
+            }
+    }
+    return RCM_OK;
+}
+
+// ensemble means per wavelength, summed in column order
+int write_spectrum(const std::string& path, int ncol, int nwvl, const double* wvl, const double* weight, const double* olr,
+                   const double* sfc) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    std::fprintf(f, "wvl_nm,weight,olr,surface_down\n");
+    for (int w = 0; w < nwvl; ++w) {
+        double so = 0.0, ss = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) {
+            so += olr[c * nwvl + w];
+            ss += sfc[c * nwvl + w];
+        }
+        std::fprintf(f, "%.17g,%.17g,%.17g,%.17g\n", wvl[w], weight[w], so / ncol, ss / ncol);
+    }
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
 
 void run_shard(Shard* sh, const Job* j) {
     auto fail = [&](const char* what, int st) {
@@ -140,12 +190,16 @@ void run_shard(Shard* sh, const Job* j) {
         st = rcm_save_checkpoint(sh->s, (j->ckpt + ".gpu" + std::to_string(sh->dev)).c_str());
         if (st != RCM_OK) return fail("rcm_save_checkpoint", st);
     }
+    if (j->spec_nwvl > 0) {
+        st = diagnose_spectrum(sh->s, (int)n, j->spec_nwvl, j->olr_out + lo * j->spec_nwvl, j->sfc_out + lo * j->spec_nwvl);
+        if (st != RCM_OK) return fail("rcm_diagnose_fluxes", st);
+    }
 }
 
 }  // namespace
 
 int main(int argc, char** argv) {
-    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path;
+    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -169,6 +223,7 @@ int main(int argc, char** argv) {
         else if (a == "--resume") resume_path = val();
         else if (a == "--steps-exact") steps_exact = 1;
         else if (a == "--gpus") gpus = std::atoi(val());
+        else if (a == "--spectral-out") spectral_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -177,7 +232,12 @@ int main(int argc, char** argv) {
     if (atm_path.empty() || (table_path.empty() == lbl_dir.empty()) || ncol < 1 || max_steps < 1 || check_every < 1 || gpus < 1 ||
         gpus > ncol) {
         std::fprintf(stderr, "usage: rcm_rce --atm FILE (--table FILE | --lbl DIR [--co2-factor F]) [--ncol N] [--seed S] [--max-steps M] [--check-every K] "
-                             "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N]\n");
+                             "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
+                             "[--spectral-out FILE]\n");
+        return 1;
+    }
+    if (!lbl_dir.empty() && !spectral_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --spectral-out needs a repwvl table (--table): the line-by-line path has no diagnostic call\n");
         return 1;
     }
 
@@ -255,8 +315,16 @@ int main(int argc, char** argv) {
         }
         std::vector<double> T(n * NLAY), Ts(n), Eu(n * NLEV);
         std::vector<float> time_h(n);
+        int dims[4] = {0, 0, 0, 0};
+        std::vector<double> olr, sfc;
+        if (!spectral_path.empty()) {
+            rcm_table_dims(table, dims);
+            olr.resize(n * dims[2]);
+            sfc.resize(n * dims[2]);
+        }
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
-                max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data()};
+                max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
+                dims[2], olr.data(), sfc.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -285,8 +353,16 @@ int main(int argc, char** argv) {
             if (sh.s) rcm_destroy(sh.s);
             if (sh.comm) ncclCommDestroy(sh.comm);
         }
+        if (bad) {
+            if (table) rcm_table_free(table);
+            return 1;
+        }
+        if (!spectral_path.empty() &&
+            write_spectrum(spectral_path, ncol, dims[2], rcm_table_array(table, 1), rcm_table_array(table, 2), olr.data(), sfc.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
         if (table) rcm_table_free(table);
-        if (bad) return 1;
         st = rcm_write_profiles(out_path.c_str(), 0, 1, ncol, plevel, T.data(), time_h.data(), ncol > 1);
         if (st != RCM_OK) return die(out_path.c_str(), st, nullptr);
         const rcm_step_scalars& last = shards[0].last;
@@ -301,6 +377,7 @@ int main(int argc, char** argv) {
         std::printf("rcm_rce: time loop %.4f s on the slowest GPU = %.4f ms per iteration\n", loop_s, 1e3 * loop_s / (double)shards[0].done);
         return 0;
     }
+    std::vector<double> spec_wvl, spec_weight;  // --spectral-out: the table's wavelengths and weights
     rcm_solver* s = nullptr;
     st = rcm_create(device, &p, &s);
     if (st != RCM_OK) return die("rcm_create", st, nullptr);
@@ -339,6 +416,10 @@ int main(int argc, char** argv) {
         st = rcm_table_load(table_path.c_str(), &t);
         if (st != RCM_OK) return die(table_path.c_str(), st, s);
         st = rcm_set_repwvl_table_from(s, t);
+        int dims[4] = {0, 0, 0, 0};
+        rcm_table_dims(t, dims);
+        spec_wvl.assign(rcm_table_array(t, 1), rcm_table_array(t, 1) + dims[2]);
+        spec_weight.assign(rcm_table_array(t, 2), rcm_table_array(t, 2) + dims[2]);
         rcm_table_free(t);
         if (st != RCM_OK) return die("rcm_set_repwvl_table_from", st, s);
     }
@@ -384,6 +465,13 @@ int main(int argc, char** argv) {
     if (!ckpt_path.empty()) {
         st = rcm_save_checkpoint(s, ckpt_path.c_str());
         if (st != RCM_OK) return die(ckpt_path.c_str(), st, s);
+    }
+    if (!spectral_path.empty()) {
+        const int nw = (int)spec_wvl.size();
+        std::vector<double> olr(m * nw), sfc(m * nw);
+        st = diagnose_spectrum(s, ncol, nw, olr.data(), sfc.data());
+        if (st != RCM_OK) return die("rcm_diagnose_fluxes", st, s);
+        if (write_spectrum(spectral_path, ncol, nw, spec_wvl.data(), spec_weight.data(), olr.data(), sfc.data())) return 1;
     }
     double ts_mean = 0.0;
     for (size_t c = 0; c < m; ++c) ts_mean += Ts[c];

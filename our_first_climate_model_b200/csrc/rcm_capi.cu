@@ -11,7 +11,7 @@
 #include <string>
 #include <vector>
 
-#include "rcm_kernels.cuh"
+#include "rcm_diag.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -98,6 +98,10 @@ struct rcm_solver {
     cudaEvent_t sp_prep[24] = {}, sp_rtdone[24] = {}, sp_end = nullptr;
     double kt_ms = 0.0;
     long kt_n = 0;
+    unsigned char* d_diagnose = nullptr;  // rcm_diagnose_fluxes: two sets of (copies of a chunk's state, its tile blocks, fluxes)
+    size_t diagnose_bytes = 0;
+    cudaStream_t dg_stream[2] = {nullptr, nullptr};  // ... the chunks alternate between two streams and the two sets
+    cudaEvent_t dg_fork = nullptr, dg_join[2] = {nullptr, nullptr};
 };
 
 namespace {
@@ -903,7 +907,7 @@ int rcm_destroy(rcm_solver* s) {
     void* ptrs[] = {s->d_coef3, s->d_xsec_file, s->d_coef, s->d_species, s->d_planck_c, s->d_planck_k, s->d_exp_tab, s->d_T, s->d_Ts, s->d_vmr, s->d_rh,
                     s->d_Tprev, s->d_time, s->d_lbl_lo, s->d_lbl_hi, s->d_lbl_tau5, s->d_lbl_h2o_ref, s->d_lbl_o3_ref, s->d_sH, s->d_sO,
                     s->d_dTstat, s->d_part, s->d_Ed, s->d_Eu, s->d_dE, s->d_dt, s->d_diag, s->d_scalars, s->d_red, s->d_tau,
-                    s->d_lowpos, s->d_solar_col, s->d_cloud_col, s->d_ticket, s->d_tile, s->d_spart, s->d_counter, s->d_multi};
+                    s->d_lowpos, s->d_solar_col, s->d_cloud_col, s->d_ticket, s->d_tile, s->d_spart, s->d_counter, s->d_multi, s->d_diagnose};
     for (void* q : ptrs)
         if (q) cudaFree(q);
     for (auto& e : s->ev_free) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
@@ -920,6 +924,11 @@ int rcm_destroy(rcm_solver* s) {
         if (s->sp_rtdone[i]) cudaEventDestroy(s->sp_rtdone[i]);
     }
     if (s->sp_end) cudaEventDestroy(s->sp_end);
+    for (int i = 0; i < 2; ++i) {
+        if (s->dg_stream[i]) cudaStreamDestroy(s->dg_stream[i]);
+        if (s->dg_join[i]) cudaEventDestroy(s->dg_join[i]);
+    }
+    if (s->dg_fork) cudaEventDestroy(s->dg_fork);
     if (s->hg.exec) cudaGraphExecDestroy(s->hg.exec);
     if (s->own_stream) cudaStreamDestroy(s->own_stream);
     delete s;
@@ -1425,6 +1434,136 @@ int rcm_get_state(rcm_solver* s, double* Tlayer, double* Tsurf, double* h2o, flo
         CU(cudaMemcpy2DAsync(h2o, NLAY * sizeof(double), s->d_vmr + (size_t)s->h2o_slot * NLAY,
                              (size_t)s->nactive * NLAY * sizeof(double), NLAY * sizeof(double), n, cudaMemcpyDeviceToHost,
                              s->stream));
+    }
+    CU(cudaStreamSynchronize(s->stream));
+    return RCM_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Diagnostic radiation call.  The split path's prep kernel - the sort, the water-vapour feedback and the table indices of
+// the next step - runs on COPIES of a chunk's T, previous profile and VMRs and writes its tile blocks into a scratch
+// buffer; the solver's state, its tile blocks and every flag stay as they are.  Chunks of at most 8,192 columns alternate
+// between two streams with a scratch set each (about 0.6 GB with 100 wavelengths): the memory-bound sum kernel and the copies
+// of one chunk overlap the radiative transfer of the next, and the last round of one chunk's units the first of the next.
+// ------------------------------------------------------------------------------------------
+int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
+                        double* E_down, double* E_up, double* dE) {
+    if (!s) return RCM_ERR_ARG;
+    if (s->lbl_mode) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: the line-by-line path is not supported");
+    if (!s->has_table) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: no lookup table loaded");
+    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: no columns loaded");
+    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: needs the five active species of the default species_mask");
+    if (!use_split(s)) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: needs the split path (RCM_OPT_PATH 0, no forced tile shape)");
+    if (col0 < 0 || ncol <= 0 || (long long)col0 + ncol > s->ncol)
+        return fail(s, RCM_ERR_ARG, "rcm_diagnose_fluxes: columns [" + std::to_string(col0) + ", " + std::to_string((long long)col0 + ncol) +
+                                        ") outside the " + std::to_string(s->ncol) + " loaded");
+    DiagScale sc{};
+    for (int k = 0; k < 5; ++k) {
+        sc.f[k] = vmr_scale ? vmr_scale[k] : 1.0;
+        if (!(sc.f[k] >= 0.0) || !std::isfinite(sc.f[k]))
+            return fail(s, RCM_ERR_ARG, "rcm_diagnose_fluxes: vmr_scale[" + std::to_string(k) + "] must be finite and >= 0");
+    }
+    CU(cudaSetDevice(s->device));
+    int st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    constexpr int kMaxChunk = 8192;
+    const int nwvl = s->dc.nwvl, na = s->nactive;
+    const size_t ch = (size_t)std::min(kMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
+    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], E_down, E_up [ch][21], dE [ch][20], spectral [2][ch][nwvl][21],
+    // then the tile blocks
+    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 2 * NLEV + NLAY) + 2 * ch * nwvl * NLEV;
+    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    if (2 * set_bytes > s->diagnose_bytes) {
+        CU(dalloc(s->d_diagnose, 2 * set_bytes));
+        s->diagnose_bytes = 2 * set_bytes;
+    }
+    if (!s->dg_fork) {
+        for (int i = 0; i < 2; ++i) {
+            CU(cudaStreamCreateWithFlags(&s->dg_stream[i], cudaStreamNonBlocking));
+            CU(cudaEventCreateWithFlags(&s->dg_join[i], cudaEventDisableTiming));
+        }
+        CU(cudaEventCreateWithFlags(&s->dg_fork, cudaEventDisableTiming));
+    }
+    CU(cudaEventRecord(s->dg_fork, s->stream));  // work queued on the solver's stream comes first
+    for (int i = 0; i < 2; ++i) CU(cudaStreamWaitEvent(s->dg_stream[i], s->dg_fork, 0));
+    const bool scaled = vmr_scale != nullptr;
+    const int nsm = nsm_of(s);
+    // the downloads of chunk k are issued after the kernels of chunk k + 1: into pageable memory they block the host
+    struct Pending { cudaStream_t q; size_t r; int n; const double *dn, *up, *Ed, *Eu, *dE; } pend{};
+    auto download = [&](const Pending& c) -> int {
+        const size_t nspec = (size_t)c.n * nwvl * NLEV;
+        if (E_down_spec) CU(cudaMemcpyAsync(E_down_spec + c.r * nwvl * NLEV, c.dn, nspec * D, cudaMemcpyDeviceToHost, c.q));
+        if (E_up_spec) CU(cudaMemcpyAsync(E_up_spec + c.r * nwvl * NLEV, c.up, nspec * D, cudaMemcpyDeviceToHost, c.q));
+        if (E_down) CU(cudaMemcpyAsync(E_down + c.r * NLEV, c.Ed, c.n * NLEV * D, cudaMemcpyDeviceToHost, c.q));
+        if (E_up) CU(cudaMemcpyAsync(E_up + c.r * NLEV, c.Eu, c.n * NLEV * D, cudaMemcpyDeviceToHost, c.q));
+        if (dE) CU(cudaMemcpyAsync(dE + c.r * NLAY, c.dE, c.n * NLAY * D, cudaMemcpyDeviceToHost, c.q));
+        return RCM_OK;
+    };
+    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
+        const int n = std::min((int)ch, col0 + ncol - c0);
+        const size_t o = (size_t)c0, r = (size_t)(c0 - col0);
+        cudaStream_t q = s->dg_stream[k % 2];  // chunk k + 2 reuses the set of chunk k after it on the same stream
+        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
+        double* dT = p; p += ch * NLAY;
+        double* dTprev = p; p += ch * NLAY;
+        double* dvmr = p; p += ch * na * NLAY;
+        double* dstat = p; p += ch;
+        double* dEd = p; p += ch * NLEV;
+        double* dEu = p; p += ch * NLEV;
+        double* ddE = p; p += ch * NLAY;
+        double* dspec_dn = p; p += ch * nwvl * NLEV;
+        double* dspec_up = p;
+        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
+        CU(cudaMemcpyAsync(dT, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+        CU(cudaMemcpyAsync(dTprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+        CU(cudaMemcpyAsync(dvmr, s->d_vmr + o * na * NLAY, (size_t)n * na * NLAY * D, cudaMemcpyDeviceToDevice, q));
+        SplitArgs a = split_args(s, c0, n, 0);
+        a.Tlayer = dT;
+        a.Tprev = dTprev;
+        a.vmr = dvmr;
+        a.dTstat = dstat;
+        a.tile = dtile;
+        a.counter = nullptr;
+        a.part = nullptr;
+        a.diag = nullptr;
+        a.E_down = a.E_up = a.dE = a.dt = nullptr;
+        a.time_h = nullptr;
+        SplitColFlags f{};
+        f.prep = 1;
+        f.first = (s->step_index == 0);
+        f.write_all_vmr = 1;
+        CU(rcm_launch_split_col(a, f, q));
+        if (scaled) CU(rcm_launch_diag_scale(dtile, a.ntiles, sc, q));
+        DiagArgs g{};
+        g.ncol = n;
+        g.ntiles = a.ntiles;
+        g.nsplit = a.nsplit;
+        g.ipu = a.ipu;
+        g.nitem = a.nitem;
+        g.nunits = a.nunits;
+        g.clampk = s->clampk;
+        g.tau_clamp = s->tau_clamp;
+        g.coef = s->d_coef3;
+        g.planck_c = s->d_planck_c;
+        g.planck_k = s->d_planck_k;
+        g.exp_tab = s->d_exp_tab;
+        g.tile = dtile;
+        g.spec_dn = dspec_dn;
+        g.spec_up = dspec_up;
+        g.E_down = dEd;
+        g.E_up = dEu;
+        g.dE = ddE;
+        g.solar_col = a.solar_col;
+        CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm), q));
+        CU(rcm_launch_diag_sum(g, q));
+        s->launches += scaled ? 4 : 3;
+        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
+        pend = {q, r, n, dspec_dn, dspec_up, dEd, dEu, ddE};
+    }
+    if ((st = download(pend)) != RCM_OK) return st;
+    for (int i = 0; i < 2; ++i) {
+        CU(cudaEventRecord(s->dg_join[i], s->dg_stream[i]));
+        CU(cudaStreamWaitEvent(s->stream, s->dg_join[i], 0));
     }
     CU(cudaStreamSynchronize(s->stream));
     return RCM_OK;

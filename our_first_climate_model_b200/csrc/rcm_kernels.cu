@@ -21,6 +21,7 @@
 #include <cstdio>
 
 #include "rcm_kernels.cuh"
+#include "rcm_diag.cuh"
 
 __constant__ DevConst cst;
 
@@ -191,6 +192,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 
 #include "rcm_lbl_kernels.cuh"
 #include "rcm_split_kernels.cuh"
+#include "rcm_diag_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -381,5 +383,23 @@ cudaError_t rcm_launch_lbl_step(const LblArgs& a, cudaStream_t st, cudaEvent_t e
     kern<<<a.ntiles * a.nchunks, NT, smem, st>>>(a);
     if (ev1) cudaEventRecord(ev1, st);
     rcm_lbl_finish_kernel<<<a.ncol, LBL_FIN_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_diag_scale(unsigned char* tile, int ntiles, const DiagScale& sc, cudaStream_t st) {
+    rcm_diag_scale_kernel<<<296, 256, 0, st>>>(tile, ntiles, sc);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_diag_rt(const DiagArgs& a, int grid, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_diag_rt_kernel<true> : rcm_diag_rt_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DIAG_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, DIAG_NT, DIAG_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_diag_sum(const DiagArgs& a, cudaStream_t st) {
+    rcm_diag_sum_kernel<<<(a.ncol + DIAG_SUM_COLS - 1) / DIAG_SUM_COLS, 128, 0, st>>>(a);
     return cudaGetLastError();
 }
