@@ -240,6 +240,20 @@ int rcm_column_count(const rcm_solver* s); /* columns currently loaded (rcm_set_
  * RCM_OPT_PATH 1. */
 int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
                         double* E_down, double* E_up, double* dE);
+/* Radiative kernels (Soden et al. 2008) of the columns [col0, col0 + ncol): analytic derivatives of two fluxes of the NEXT
+ * step - output o = 0: E_up[0], the OLR; o = 1: E_down[20], the surface downward flux - at exactly the state
+ * rcm_diagnose_fluxes radiates with (after the theta-sort and the water-vapour feedback, with the grey cloud, per-column cloud
+ * tau of rcm_set_column_solar included; at step 0 with tau from the initial, unsorted profile), vmr_scale as there.
+ * Entries of each output [41]: 0..19 dF/dT_l (W m-2 K-1, layers top-down); 20 dF/dT_surf (exactly 0.0 for o = 1: the surface
+ * is black); 21..40 dF/d ln q_l (W m-2 per unit ln q), q_l = H2O VMR of layer l as the step uses it.
+ * Definitions: d/dT_l perturbs layer l's temperature in both places it enters - its Planck source and the temperature its tau
+ * is interpolated at (the same value except at step 0); d/d ln q_l is taken at fixed T.  Where a clamp is active the derivative
+ * is 0: tau at its floor or ceiling, a temperature at or below T_floor in the Planck source.  Exactly on a table temperature
+ * node the slope is that of the interval LowerPos picks.
+ * Outputs (host, either may be NULL): K_spec [ncol][nwvl][2][41], the contribution of each wavelength (its spectral weight
+ * included); K [ncol][2][41] = K_spec summed over the wavelengths in index order.  Synchronous; changes nothing.  Device scratch
+ * of its own (about 1.1 GB for 100 wavelengths).  Errors as rcm_diagnose_fluxes; also RCM_ERR_STATE when H2O is not active. */
+int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* K_spec, double* K);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

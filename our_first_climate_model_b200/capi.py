@@ -414,6 +414,28 @@ class Solver:
                self._h)
         return out
 
+    def radiative_kernels(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, spectral: bool = False) -> dict:
+        """rcm_radiative_kernels: derivatives of the next step's OLR (output 0) and surface downward flux (output 1) for
+        columns [col0, col0 + ncol), without changing anything.  vmr_scale as in diagnose_fluxes.
+        -> K [ncol, 2, 41] (entries: dF/dT_l for the 20 layers top-down, dF/dT_surf, dF/dln q_l for the 20 layers) with the
+        views dOLR_dT [ncol, 20], dOLR_dTs [ncol], dOLR_dlnq [ncol, 20], dSFC_dT, dSFC_dlnq, and with spectral
+        K_spec [ncol, nwvl, 2, 41] (each wavelength's contribution; K is its sum over the wavelengths in index order)."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = None
+        if vmr_scale is not None:
+            sc = _f64(vmr_scale).ravel()
+            if sc.size != self.nactive:
+                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        m = max(n, 0)
+        K = np.zeros((m, 2, 2 * NLAY + 1))
+        Ks = np.zeros((m, self.nwvl, 2, 2 * NLAY + 1)) if spectral else None
+        _check(_lib.rcm_radiative_kernels(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(Ks), _p(K)), self._h)
+        out = dict(K=K, dOLR_dT=K[:, 0, :NLAY], dOLR_dTs=K[:, 0, NLAY], dOLR_dlnq=K[:, 0, NLAY + 1:],
+                   dSFC_dT=K[:, 1, :NLAY], dSFC_dlnq=K[:, 1, NLAY + 1:])
+        if spectral:
+            out["K_spec"] = Ks
+        return out
+
     def advance(self, nsteps: int, want_scalars=True):
         sc = (StepScalars * nsteps)() if want_scalars else None
         _check(_lib.rcm_advance(self._h, C.c_int(nsteps), sc), self._h)

@@ -8,7 +8,7 @@
 //
 //   rcm_rce --atm test.atm --table Reduced100Forcing.nc [--ncol N] [--seed S] [--max-steps M] [--check-every K]
 //           [--dT 1e-3] [--device D] [--out output.txt] [--checkpoint file] [--resume file] [--steps-exact]
-//           [--spectral-out spectrum.csv]
+//           [--spectral-out spectrum.csv] [--kernels-out kernels.csv]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
@@ -26,6 +26,12 @@
 // wavelength - header "wvl_nm,weight,olr,surface_down", then one row per wavelength with the ensemble means of the TOA upward
 // and the surface downward flux of that wavelength (W/m2, its spectral weight included), summed in column order: the file is
 // byte-identical for any --gpus N.
+//
+// --kernels-out FILE (repwvl tables only): after the run, the radiative kernels of the next step (rcm_radiative_kernels) -
+// header "layer,p_layer,dOLR_dT,dOLR_dlnq,dSFC_dT,dSFC_dlnq", then one row per layer (top-down; p_layer in hPa) with the
+// ensemble means of the derivatives of the OLR and of the surface downward flux with respect to the layer's temperature
+// (W/m2/K) and ln(H2O VMR) (W/m2), then the row "surface" with the surface pressure and the derivatives with respect to the
+// surface temperature (the ln q fields 0).  Summed in column order: the file is byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -79,6 +85,8 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     float* time_out;
     int spec_nwvl;            // > 0: --spectral-out, rows [ncol][spec_nwvl] of olr / sfc
     double *olr_out, *sfc_out;
+    int kernels;              // --kernels-out: rows [ncol][2][41] of rcm_radiative_kernels into K_out
+    double* K_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -117,6 +125,33 @@ int write_spectrum(const std::string& path, int ncol, int nwvl, const double* wv
         }
         std::fprintf(f, "%.17g,%.17g,%.17g,%.17g\n", wvl[w], weight[w], so / ncol, ss / ncol);
     }
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
+
+constexpr int KERN_NE = 2 * RCM_NLAYER + 1, KERN_NK = 2 * KERN_NE;  // rcm_radiative_kernels: [2][41] per column
+
+// ensemble means of the radiative kernels, summed in column order
+int write_kernels(const std::string& path, int ncol, const double* player, double p_surface, const double* K) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    auto mean = [&](int o, int e) {
+        double sum = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) sum += K[c * KERN_NK + o * KERN_NE + e];
+        return sum / ncol;
+    };
+    constexpr int NLAY = RCM_NLAYER;
+    std::fprintf(f, "layer,p_layer,dOLR_dT,dOLR_dlnq,dSFC_dT,dSFC_dlnq\n");
+    for (int l = 0; l < NLAY; ++l)
+        std::fprintf(f, "%d,%.17g,%.17g,%.17g,%.17g,%.17g\n", l, player[l], mean(0, l), mean(0, NLAY + 1 + l), mean(1, l),
+                     mean(1, NLAY + 1 + l));
+    std::fprintf(f, "surface,%.17g,%.17g,0,%.17g,0\n", p_surface, mean(0, NLAY), mean(1, NLAY));
     if (std::fclose(f) != 0) {
         std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
         return 1;
@@ -194,12 +229,16 @@ void run_shard(Shard* sh, const Job* j) {
         st = diagnose_spectrum(sh->s, (int)n, j->spec_nwvl, j->olr_out + lo * j->spec_nwvl, j->sfc_out + lo * j->spec_nwvl);
         if (st != RCM_OK) return fail("rcm_diagnose_fluxes", st);
     }
+    if (j->kernels) {
+        st = rcm_radiative_kernels(sh->s, 0, (int)n, nullptr, nullptr, j->K_out + lo * KERN_NK);
+        if (st != RCM_OK) return fail("rcm_radiative_kernels", st);
+    }
 }
 
 }  // namespace
 
 int main(int argc, char** argv) {
-    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path;
+    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -224,6 +263,7 @@ int main(int argc, char** argv) {
         else if (a == "--steps-exact") steps_exact = 1;
         else if (a == "--gpus") gpus = std::atoi(val());
         else if (a == "--spectral-out") spectral_path = val();
+        else if (a == "--kernels-out") kernels_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -233,11 +273,15 @@ int main(int argc, char** argv) {
         gpus > ncol) {
         std::fprintf(stderr, "usage: rcm_rce --atm FILE (--table FILE | --lbl DIR [--co2-factor F]) [--ncol N] [--seed S] [--max-steps M] [--check-every K] "
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
-                             "[--spectral-out FILE]\n");
+                             "[--spectral-out FILE] [--kernels-out FILE]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --spectral-out needs a repwvl table (--table): the line-by-line path has no diagnostic call\n");
+        return 1;
+    }
+    if (!lbl_dir.empty() && !kernels_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --kernels-out needs a repwvl table (--table): the line-by-line path has no radiative kernels\n");
         return 1;
     }
 
@@ -322,9 +366,10 @@ int main(int argc, char** argv) {
             olr.resize(n * dims[2]);
             sfc.resize(n * dims[2]);
         }
+        std::vector<double> K(kernels_path.empty() ? 0 : n * KERN_NK);
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
-                dims[2], olr.data(), sfc.data()};
+                dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -359,6 +404,10 @@ int main(int argc, char** argv) {
         }
         if (!spectral_path.empty() &&
             write_spectrum(spectral_path, ncol, dims[2], rcm_table_array(table, 1), rcm_table_array(table, 2), olr.data(), sfc.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
+        if (!kernels_path.empty() && write_kernels(kernels_path, ncol, player.data(), plevel[NLAY], K.data())) {
             rcm_table_free(table);
             return 1;
         }
@@ -472,6 +521,12 @@ int main(int argc, char** argv) {
         st = diagnose_spectrum(s, ncol, nw, olr.data(), sfc.data());
         if (st != RCM_OK) return die("rcm_diagnose_fluxes", st, s);
         if (write_spectrum(spectral_path, ncol, nw, spec_wvl.data(), spec_weight.data(), olr.data(), sfc.data())) return 1;
+    }
+    if (!kernels_path.empty()) {
+        std::vector<double> K(m * KERN_NK);
+        st = rcm_radiative_kernels(s, 0, ncol, nullptr, nullptr, K.data());
+        if (st != RCM_OK) return die("rcm_radiative_kernels", st, s);
+        if (write_kernels(kernels_path, ncol, player.data(), plevel[NLAY], K.data())) return 1;
     }
     double ts_mean = 0.0;
     for (size_t c = 0; c < m; ++c) ts_mean += Ts[c];

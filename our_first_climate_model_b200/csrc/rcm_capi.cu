@@ -11,7 +11,7 @@
 #include <string>
 #include <vector>
 
-#include "rcm_diag.cuh"
+#include "rcm_jac.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -1440,39 +1440,37 @@ int rcm_get_state(rcm_solver* s, double* Tlayer, double* Tsurf, double* h2o, flo
 }
 
 // ------------------------------------------------------------------------------------------
-// Diagnostic radiation call.  The split path's prep kernel - the sort, the water-vapour feedback and the table indices of
-// the next step - runs on COPIES of a chunk's T, previous profile and VMRs and writes its tile blocks into a scratch
-// buffer; the solver's state, its tile blocks and every flag stay as they are.  Chunks of at most 8,192 columns alternate
-// between two streams with a scratch set each (about 0.6 GB with 100 wavelengths): the memory-bound sum kernel and the copies
-// of one chunk overlap the radiative transfer of the next, and the last round of one chunk's units the first of the next.
+// Diagnostic calls (rcm_diagnose_fluxes, rcm_radiative_kernels).  The split path's prep kernel - the sort, the water-vapour
+// feedback and the table indices of the next step - runs on COPIES of a chunk's T, previous profile and VMRs and writes its
+// tile blocks into a scratch buffer; the solver's state, its tile blocks and every flag stay as they are.  Chunks of at most
+// 8,192 columns alternate between two streams with a scratch set each (about 0.6 GB with 100 wavelengths for the fluxes,
+// 1.1 GB for the radiative kernels): the memory-bound sum kernel and the copies of one chunk overlap the radiative transfer
+// of the next, and the last round of one chunk's units the first of the next.
 // ------------------------------------------------------------------------------------------
-int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
-                        double* E_down, double* E_up, double* dE) {
-    if (!s) return RCM_ERR_ARG;
-    if (s->lbl_mode) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: the line-by-line path is not supported");
-    if (!s->has_table) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: no lookup table loaded");
-    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: no columns loaded");
-    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: needs the five active species of the default species_mask");
-    if (!use_split(s)) return fail(s, RCM_ERR_STATE, "rcm_diagnose_fluxes: needs the split path (RCM_OPT_PATH 0, no forced tile shape)");
+namespace {
+
+constexpr int kDiagMaxChunk = 8192;
+
+// the checks both calls make; the factors of vmr_scale (NULL = all 1) into sc
+int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
+    if (s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": the line-by-line path is not supported");
+    if (!s->has_table) return fail(s, RCM_ERR_STATE, fn + ": no lookup table loaded");
+    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
+    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
+    if (!use_split(s)) return fail(s, RCM_ERR_STATE, fn + ": needs the split path (RCM_OPT_PATH 0, no forced tile shape)");
     if (col0 < 0 || ncol <= 0 || (long long)col0 + ncol > s->ncol)
-        return fail(s, RCM_ERR_ARG, "rcm_diagnose_fluxes: columns [" + std::to_string(col0) + ", " + std::to_string((long long)col0 + ncol) +
+        return fail(s, RCM_ERR_ARG, fn + ": columns [" + std::to_string(col0) + ", " + std::to_string((long long)col0 + ncol) +
                                         ") outside the " + std::to_string(s->ncol) + " loaded");
-    DiagScale sc{};
     for (int k = 0; k < 5; ++k) {
         sc.f[k] = vmr_scale ? vmr_scale[k] : 1.0;
         if (!(sc.f[k] >= 0.0) || !std::isfinite(sc.f[k]))
-            return fail(s, RCM_ERR_ARG, "rcm_diagnose_fluxes: vmr_scale[" + std::to_string(k) + "] must be finite and >= 0");
+            return fail(s, RCM_ERR_ARG, fn + ": vmr_scale[" + std::to_string(k) + "] must be finite and >= 0");
     }
-    CU(cudaSetDevice(s->device));
-    int st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    constexpr int kMaxChunk = 8192;
-    const int nwvl = s->dc.nwvl, na = s->nactive;
-    const size_t ch = (size_t)std::min(kMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
-    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], E_down, E_up [ch][21], dE [ch][20], spectral [2][ch][nwvl][21],
-    // then the tile blocks
-    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 2 * NLEV + NLAY) + 2 * ch * nwvl * NLEV;
-    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    return RCM_OK;
+}
+
+// two scratch sets of set_bytes each, the two streams; work queued on the solver's stream comes first
+int diag_begin(rcm_solver* s, size_t set_bytes) {
     if (2 * set_bytes > s->diagnose_bytes) {
         CU(dalloc(s->d_diagnose, 2 * set_bytes));
         s->diagnose_bytes = 2 * set_bytes;
@@ -1484,8 +1482,71 @@ int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_sca
         }
         CU(cudaEventCreateWithFlags(&s->dg_fork, cudaEventDisableTiming));
     }
-    CU(cudaEventRecord(s->dg_fork, s->stream));  // work queued on the solver's stream comes first
+    CU(cudaEventRecord(s->dg_fork, s->stream));
     for (int i = 0; i < 2; ++i) CU(cudaStreamWaitEvent(s->dg_stream[i], s->dg_fork, 0));
+    return RCM_OK;
+}
+
+// Copies of columns [c0, c0 + n) - T and Tprev into dT, dTprev [ch][20], VMRs into dvmr [ch][5][20] - and the prep of the
+// next step on them (dstat [ch]: its stationarity diagnostic, unused), tile blocks into dtile, then the VMR factors (sc:
+// NULL = unscaled).  On return dT holds the sorted profile the step radiates with; a carries the chunk's unit plan.
+int diag_prep(rcm_solver* s, cudaStream_t q, int c0, int n, double* dT, double* dTprev, double* dvmr, double* dstat,
+              unsigned char* dtile, const DiagScale* sc, SplitArgs& a) {
+    constexpr size_t D = sizeof(double);
+    const size_t o = (size_t)c0;
+    const int na = s->nactive;
+    CU(cudaMemcpyAsync(dT, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(dTprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(dvmr, s->d_vmr + o * na * NLAY, (size_t)n * na * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    a = split_args(s, c0, n, 0);
+    a.Tlayer = dT;
+    a.Tprev = dTprev;
+    a.vmr = dvmr;
+    a.dTstat = dstat;
+    a.tile = dtile;
+    a.counter = nullptr;
+    a.part = nullptr;
+    a.diag = nullptr;
+    a.E_down = a.E_up = a.dE = a.dt = nullptr;
+    a.time_h = nullptr;
+    SplitColFlags f{};
+    f.prep = 1;
+    f.first = (s->step_index == 0);
+    f.write_all_vmr = 1;
+    CU(rcm_launch_split_col(a, f, q));
+    if (sc) CU(rcm_launch_diag_scale(dtile, a.ntiles, *sc, q));
+    s->launches += sc ? 2 : 1;
+    return RCM_OK;
+}
+
+// the solver's stream waits for both streams; then the host waits
+int diag_end(rcm_solver* s) {
+    for (int i = 0; i < 2; ++i) {
+        CU(cudaEventRecord(s->dg_join[i], s->dg_stream[i]));
+        CU(cudaStreamWaitEvent(s->stream, s->dg_join[i], 0));
+    }
+    CU(cudaStreamSynchronize(s->stream));
+    return RCM_OK;
+}
+
+}  // namespace
+
+int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
+                        double* E_down, double* E_up, double* dE) {
+    if (!s) return RCM_ERR_ARG;
+    DiagScale sc{};
+    int st = diag_check(s, "rcm_diagnose_fluxes", col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    CU(cudaSetDevice(s->device));
+    st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    const int nwvl = s->dc.nwvl, na = s->nactive;
+    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
+    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], E_down, E_up [ch][21], dE [ch][20], spectral [2][ch][nwvl][21],
+    // then the tile blocks
+    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 2 * NLEV + NLAY) + 2 * ch * nwvl * NLEV;
+    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
     const bool scaled = vmr_scale != nullptr;
     const int nsm = nsm_of(s);
     // the downloads of chunk k are issued after the kernels of chunk k + 1: into pageable memory they block the host
@@ -1501,7 +1562,7 @@ int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_sca
     };
     for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
         const int n = std::min((int)ch, col0 + ncol - c0);
-        const size_t o = (size_t)c0, r = (size_t)(c0 - col0);
+        const size_t r = (size_t)(c0 - col0);
         cudaStream_t q = s->dg_stream[k % 2];  // chunk k + 2 reuses the set of chunk k after it on the same stream
         double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
         double* dT = p; p += ch * NLAY;
@@ -1514,26 +1575,8 @@ int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_sca
         double* dspec_dn = p; p += ch * nwvl * NLEV;
         double* dspec_up = p;
         unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
-        CU(cudaMemcpyAsync(dT, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-        CU(cudaMemcpyAsync(dTprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-        CU(cudaMemcpyAsync(dvmr, s->d_vmr + o * na * NLAY, (size_t)n * na * NLAY * D, cudaMemcpyDeviceToDevice, q));
-        SplitArgs a = split_args(s, c0, n, 0);
-        a.Tlayer = dT;
-        a.Tprev = dTprev;
-        a.vmr = dvmr;
-        a.dTstat = dstat;
-        a.tile = dtile;
-        a.counter = nullptr;
-        a.part = nullptr;
-        a.diag = nullptr;
-        a.E_down = a.E_up = a.dE = a.dt = nullptr;
-        a.time_h = nullptr;
-        SplitColFlags f{};
-        f.prep = 1;
-        f.first = (s->step_index == 0);
-        f.write_all_vmr = 1;
-        CU(rcm_launch_split_col(a, f, q));
-        if (scaled) CU(rcm_launch_diag_scale(dtile, a.ntiles, sc, q));
+        SplitArgs a;
+        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, scaled ? &sc : nullptr, a)) != RCM_OK) return st;
         DiagArgs g{};
         g.ncol = n;
         g.ntiles = a.ntiles;
@@ -1556,17 +1599,80 @@ int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_sca
         g.solar_col = a.solar_col;
         CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm), q));
         CU(rcm_launch_diag_sum(g, q));
-        s->launches += scaled ? 4 : 3;
+        s->launches += 2;
         if (k > 0 && (st = download(pend)) != RCM_OK) return st;
         pend = {q, r, n, dspec_dn, dspec_up, dEd, dEu, ddE};
     }
     if ((st = download(pend)) != RCM_OK) return st;
-    for (int i = 0; i < 2; ++i) {
-        CU(cudaEventRecord(s->dg_join[i], s->dg_stream[i]));
-        CU(cudaStreamWaitEvent(s->stream, s->dg_join[i], 0));
+    return diag_end(s);
+}
+
+// Radiative kernels: the same chunks, streams and prep as rcm_diagnose_fluxes; rcm_jac_rt_kernel per (column, wavelength),
+// rcm_jac_sum_kernel for the sum over the wavelengths.
+int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* K_spec, double* K) {
+    if (!s) return RCM_ERR_ARG;
+    DiagScale sc{};
+    int st = diag_check(s, "rcm_radiative_kernels", col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, "rcm_radiative_kernels: needs H2O among the active species");
+    CU(cudaSetDevice(s->device));
+    st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    const int nwvl = s->dc.nwvl, na = s->nactive;
+    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
+    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], K [ch][82], K_spec [ch][nwvl][82], then the tile blocks
+    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + JAC_NK) + ch * nwvl * JAC_NK;
+    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
+    const int grid_max = rcm_jac_ctas_per_sm() * nsm_of(s);
+    struct Pending { cudaStream_t q; size_t r; int n; const double *Ks, *K; } pend{};
+    auto download = [&](const Pending& c) -> int {
+        if (K_spec) CU(cudaMemcpyAsync(K_spec + c.r * nwvl * JAC_NK, c.Ks, (size_t)c.n * nwvl * JAC_NK * D, cudaMemcpyDeviceToHost, c.q));
+        if (K) CU(cudaMemcpyAsync(K + c.r * JAC_NK, c.K, (size_t)c.n * JAC_NK * D, cudaMemcpyDeviceToHost, c.q));
+        return RCM_OK;
+    };
+    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
+        const int n = std::min((int)ch, col0 + ncol - c0);
+        const size_t r = (size_t)(c0 - col0);
+        cudaStream_t q = s->dg_stream[k % 2];
+        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
+        double* dT = p; p += ch * NLAY;
+        double* dTprev = p; p += ch * NLAY;
+        double* dvmr = p; p += ch * na * NLAY;
+        double* dstat = p; p += ch;
+        double* dK = p; p += ch * JAC_NK;
+        double* dKs = p;
+        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
+        SplitArgs a;
+        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, vmr_scale ? &sc : nullptr, a)) != RCM_OK) return st;
+        JacArgs g{};
+        g.ncol = n;
+        g.ntiles = a.ntiles;
+        g.nsplit = a.nsplit;
+        g.ipu = a.ipu;
+        g.nitem = a.nitem;
+        g.nunits = a.nunits;
+        g.clampk = s->clampk;
+        g.tau_clamp = s->tau_clamp;
+        g.T_floor = s->T_floor;
+        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+        g.coef = s->d_coef3;
+        g.planck_c = s->d_planck_c;
+        g.planck_k = s->d_planck_k;
+        g.exp_tab = s->d_exp_tab;
+        g.tile = dtile;
+        g.T = dT;
+        g.Ts = s->d_Ts + c0;
+        g.K_spec = dKs;
+        g.K = dK;
+        CU(rcm_launch_jac_rt(g, std::min(g.nunits, grid_max), q));
+        CU(rcm_launch_jac_sum(g, q));
+        s->launches += 2;
+        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
+        pend = {q, r, n, dKs, dK};
     }
-    CU(cudaStreamSynchronize(s->stream));
-    return RCM_OK;
+    if ((st = download(pend)) != RCM_OK) return st;
+    return diag_end(s);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -22,6 +22,7 @@
 
 #include "rcm_kernels.cuh"
 #include "rcm_diag.cuh"
+#include "rcm_jac.cuh"
 
 __constant__ DevConst cst;
 
@@ -193,6 +194,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_lbl_kernels.cuh"
 #include "rcm_split_kernels.cuh"
 #include "rcm_diag_kernels.cuh"
+#include "rcm_jac_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -401,5 +403,22 @@ cudaError_t rcm_launch_diag_rt(const DiagArgs& a, int grid, cudaStream_t st) {
 
 cudaError_t rcm_launch_diag_sum(const DiagArgs& a, cudaStream_t st) {
     rcm_diag_sum_kernel<<<(a.ncol + DIAG_SUM_COLS - 1) / DIAG_SUM_COLS, 128, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+int rcm_jac_ctas_per_sm() { return JAC_CTAS; }
+
+cudaError_t rcm_launch_jac_rt(const JacArgs& a, int grid, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_jac_rt_kernel<true> : rcm_jac_rt_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JAC_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, JAC_NT, JAC_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_jac_sum(const JacArgs& a, cudaStream_t st) {
+    const size_t blocks = ((size_t)a.ncol * JAC_NK + 255) / 256;
+    const int grid = blocks < 4096 ? (int)blocks : 4096;
+    rcm_jac_sum_kernel<<<grid, 256, 0, st>>>(a);
     return cudaGetLastError();
 }
