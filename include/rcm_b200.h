@@ -254,6 +254,17 @@ int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_sca
  * included); K [ncol][2][41] = K_spec summed over the wavelengths in index order.  Synchronous; changes nothing.  Device scratch
  * of its own (about 1.1 GB for 100 wavelengths).  Errors as rcm_diagnose_fluxes; also RCM_ERR_STATE when H2O is not active. */
 int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* K_spec, double* K);
+/* Flux Jacobians of the columns [col0, col0 + ncol): analytic derivatives of every level's broadband E_down and E_up of the
+ * NEXT step (summed over the wavelengths in index order) and of its heating rates, at exactly the state rcm_radiative_kernels
+ * differentiates (sort, water-vapour feedback, grey cloud, step-0 rule, vmr_scale), with respect to the same 41 entries
+ * x_e and with the same definitions: 0..19 T_l (layers top-down), 20 T_surf, 21..40 ln q_l.
+ * Outputs (host, either may be NULL): J [ncol][2][21][41], J[c][0][k][e] = dE_down[k]/dx_e and J[c][1][k][e] = dE_up[k]/dx_e
+ * (W m-2 per K resp. per unit ln q); dE_jac [ncol][20][41], d dE_l/dx_e computed from J entry by entry as dE from E
+ * (main.cpp:337-341): H[l] = Jd[l] - Jd[l+1] + Ju[l+1] - Ju[l], then H[19] += Jd[20] - Ju[20] (the solar term is constant).
+ * Exactly 0.0 by construction: row E_down[0]; dE_down[k]/d(T_l, ln q_l) for l >= k; dE_down[k]/dT_surf; dE_up[k]/d(T_l,
+ * ln q_l) for l < k (so row E_up[20] has only its T_surf entry).  Synchronous; changes nothing.  Device scratch of its own
+ * (about 0.4 GB, independent of the wavelengths).  Errors as rcm_radiative_kernels. */
+int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

@@ -436,6 +436,23 @@ class Solver:
             out["K_spec"] = Ks
         return out
 
+    def flux_jacobian(self, col0: int = 0, ncol: int | None = None, vmr_scale=None) -> dict:
+        """rcm_flux_jacobian: derivatives of the next step's broadband fluxes at every level and of its heating rates for
+        columns [col0, col0 + ncol), without changing anything.  vmr_scale as in diagnose_fluxes.  Entries as in
+        radiative_kernels (dT_l for the 20 layers top-down, dT_surf, dln q_l for the 20 layers).
+        -> J [ncol, 2, 21, 41] (J[:, 0, k] = dE_down[k], J[:, 1, k] = dE_up[k]) and dE_jac [ncol, 20, 41]."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = None
+        if vmr_scale is not None:
+            sc = _f64(vmr_scale).ravel()
+            if sc.size != self.nactive:
+                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        m = max(n, 0)
+        J = np.zeros((m, 2, NLAY + 1, 2 * NLAY + 1))
+        H = np.zeros((m, NLAY, 2 * NLAY + 1))
+        _check(_lib.rcm_flux_jacobian(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(J), _p(H)), self._h)
+        return dict(J=J, dE_jac=H)
+
     def advance(self, nsteps: int, want_scalars=True):
         sc = (StepScalars * nsteps)() if want_scalars else None
         _check(_lib.rcm_advance(self._h, C.c_int(nsteps), sc), self._h)

@@ -8,7 +8,7 @@
 //
 //   rcm_rce --atm test.atm --table Reduced100Forcing.nc [--ncol N] [--seed S] [--max-steps M] [--check-every K]
 //           [--dT 1e-3] [--device D] [--out output.txt] [--checkpoint file] [--resume file] [--steps-exact]
-//           [--spectral-out spectrum.csv] [--kernels-out kernels.csv]
+//           [--spectral-out spectrum.csv] [--kernels-out kernels.csv] [--jacobian-out jacobian.csv]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
@@ -32,6 +32,11 @@
 // ensemble means of the derivatives of the OLR and of the surface downward flux with respect to the layer's temperature
 // (W/m2/K) and ln(H2O VMR) (W/m2), then the row "surface" with the surface pressure and the derivatives with respect to the
 // surface temperature (the ln q fields 0).  Summed in column order: the file is byte-identical for any --gpus N.
+//
+// --jacobian-out FILE (repwvl tables only): after the run, the derivatives of the next step's heating rates
+// (rcm_flux_jacobian's dE_jac) - header "layer,p_layer,dT_0..dT_19,dT_surf,dlnq_0..dlnq_19", then one row per layer l
+// (top-down; p_layer in hPa) with the ensemble means of d dE_l/dx_e (W/m2 per K resp. per unit ln q) for the 41 entries x_e.
+// Summed in column order: the file is byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -87,6 +92,8 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     double *olr_out, *sfc_out;
     int kernels;              // --kernels-out: rows [ncol][2][41] of rcm_radiative_kernels into K_out
     double* K_out;
+    int jacobian;             // --jacobian-out: rows [ncol][20][41] of rcm_flux_jacobian's dE_jac into H_out
+    double* H_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -152,6 +159,37 @@ int write_kernels(const std::string& path, int ncol, const double* player, doubl
         std::fprintf(f, "%d,%.17g,%.17g,%.17g,%.17g,%.17g\n", l, player[l], mean(0, l), mean(0, NLAY + 1 + l), mean(1, l),
                      mean(1, NLAY + 1 + l));
     std::fprintf(f, "surface,%.17g,%.17g,0,%.17g,0\n", p_surface, mean(0, NLAY), mean(1, NLAY));
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
+
+constexpr int JAC_NH = RCM_NLAYER * KERN_NE;  // rcm_flux_jacobian: dE_jac [20][41] per column
+
+// ensemble means of the heating-rate Jacobians, summed in column order
+int write_jacobian(const std::string& path, int ncol, const double* player, const double* H) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    constexpr int NLAY = RCM_NLAYER;
+    std::fprintf(f, "layer,p_layer");
+    for (int l = 0; l < NLAY; ++l) std::fprintf(f, ",dT_%d", l);
+    std::fprintf(f, ",dT_surf");
+    for (int l = 0; l < NLAY; ++l) std::fprintf(f, ",dlnq_%d", l);
+    std::fprintf(f, "\n");
+    for (int l = 0; l < NLAY; ++l) {
+        std::fprintf(f, "%d,%.17g", l, player[l]);
+        for (int e = 0; e < KERN_NE; ++e) {
+            double sum = 0.0;
+            for (size_t c = 0; c < (size_t)ncol; ++c) sum += H[c * JAC_NH + l * KERN_NE + e];
+            std::fprintf(f, ",%.17g", sum / ncol);
+        }
+        std::fprintf(f, "\n");
+    }
     if (std::fclose(f) != 0) {
         std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
         return 1;
@@ -233,12 +271,17 @@ void run_shard(Shard* sh, const Job* j) {
         st = rcm_radiative_kernels(sh->s, 0, (int)n, nullptr, nullptr, j->K_out + lo * KERN_NK);
         if (st != RCM_OK) return fail("rcm_radiative_kernels", st);
     }
+    if (j->jacobian) {
+        st = rcm_flux_jacobian(sh->s, 0, (int)n, nullptr, nullptr, j->H_out + lo * JAC_NH);
+        if (st != RCM_OK) return fail("rcm_flux_jacobian", st);
+    }
 }
 
 }  // namespace
 
 int main(int argc, char** argv) {
-    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path;
+    std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
+        jacobian_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -264,6 +307,7 @@ int main(int argc, char** argv) {
         else if (a == "--gpus") gpus = std::atoi(val());
         else if (a == "--spectral-out") spectral_path = val();
         else if (a == "--kernels-out") kernels_path = val();
+        else if (a == "--jacobian-out") jacobian_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -273,7 +317,7 @@ int main(int argc, char** argv) {
         gpus > ncol) {
         std::fprintf(stderr, "usage: rcm_rce --atm FILE (--table FILE | --lbl DIR [--co2-factor F]) [--ncol N] [--seed S] [--max-steps M] [--check-every K] "
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
-                             "[--spectral-out FILE] [--kernels-out FILE]\n");
+                             "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -282,6 +326,10 @@ int main(int argc, char** argv) {
     }
     if (!lbl_dir.empty() && !kernels_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --kernels-out needs a repwvl table (--table): the line-by-line path has no radiative kernels\n");
+        return 1;
+    }
+    if (!lbl_dir.empty() && !jacobian_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --jacobian-out needs a repwvl table (--table): the line-by-line path has no flux Jacobians\n");
         return 1;
     }
 
@@ -367,9 +415,10 @@ int main(int argc, char** argv) {
             sfc.resize(n * dims[2]);
         }
         std::vector<double> K(kernels_path.empty() ? 0 : n * KERN_NK);
+        std::vector<double> H(jacobian_path.empty() ? 0 : n * JAC_NH);
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
-                dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data()};
+                dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -408,6 +457,10 @@ int main(int argc, char** argv) {
             return 1;
         }
         if (!kernels_path.empty() && write_kernels(kernels_path, ncol, player.data(), plevel[NLAY], K.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
+        if (!jacobian_path.empty() && write_jacobian(jacobian_path, ncol, player.data(), H.data())) {
             rcm_table_free(table);
             return 1;
         }
@@ -527,6 +580,12 @@ int main(int argc, char** argv) {
         st = rcm_radiative_kernels(s, 0, ncol, nullptr, nullptr, K.data());
         if (st != RCM_OK) return die("rcm_radiative_kernels", st, s);
         if (write_kernels(kernels_path, ncol, player.data(), plevel[NLAY], K.data())) return 1;
+    }
+    if (!jacobian_path.empty()) {
+        std::vector<double> H(m * JAC_NH);
+        st = rcm_flux_jacobian(s, 0, ncol, nullptr, nullptr, H.data());
+        if (st != RCM_OK) return die("rcm_flux_jacobian", st, s);
+        if (write_jacobian(jacobian_path, ncol, player.data(), H.data())) return 1;
     }
     double ts_mean = 0.0;
     for (size_t c = 0; c < m; ++c) ts_mean += Ts[c];

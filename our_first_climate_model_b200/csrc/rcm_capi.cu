@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "rcm_jac.cuh"
+#include "rcm_fjac.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -1440,12 +1441,13 @@ int rcm_get_state(rcm_solver* s, double* Tlayer, double* Tsurf, double* h2o, flo
 }
 
 // ------------------------------------------------------------------------------------------
-// Diagnostic calls (rcm_diagnose_fluxes, rcm_radiative_kernels).  The split path's prep kernel - the sort, the water-vapour
-// feedback and the table indices of the next step - runs on COPIES of a chunk's T, previous profile and VMRs and writes its
-// tile blocks into a scratch buffer; the solver's state, its tile blocks and every flag stay as they are.  Chunks of at most
-// 8,192 columns alternate between two streams with a scratch set each (about 0.6 GB with 100 wavelengths for the fluxes,
-// 1.1 GB for the radiative kernels): the memory-bound sum kernel and the copies of one chunk overlap the radiative transfer
-// of the next, and the last round of one chunk's units the first of the next.
+// Diagnostic calls (rcm_diagnose_fluxes, rcm_radiative_kernels, rcm_flux_jacobian).  The split path's prep kernel - the
+// sort, the water-vapour feedback and the table indices of the next step - runs on COPIES of a chunk's T, previous profile
+// and VMRs and writes its tile blocks into a scratch buffer; the solver's state, its tile blocks and every flag stay as they
+// are.  Chunks of at most 8,192 columns alternate between two streams with a scratch set each (about 0.6 GB with 100
+// wavelengths for the fluxes, 1.1 GB for the radiative kernels, 0.4 GB for the flux Jacobians, whatever the wavelengths):
+// the memory-bound sum kernel and the copies of one chunk overlap the radiative transfer of the next, and the last round of
+// one chunk's units the first of the next.
 // ------------------------------------------------------------------------------------------
 namespace {
 
@@ -1670,6 +1672,67 @@ int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_s
         s->launches += 2;
         if (k > 0 && (st = download(pend)) != RCM_OK) return st;
         pend = {q, r, n, dKs, dK};
+    }
+    if ((st = download(pend)) != RCM_OK) return st;
+    return diag_end(s);
+}
+
+// Flux Jacobians: the same chunks, streams and prep as rcm_diagnose_fluxes; rcm_fjac_kernel sums over the wavelengths
+// itself, one warp per column.
+int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac) {
+    if (!s) return RCM_ERR_ARG;
+    DiagScale sc{};
+    int st = diag_check(s, "rcm_flux_jacobian", col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, "rcm_flux_jacobian: needs H2O among the active species");
+    CU(cudaSetDevice(s->device));
+    st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    const int na = s->nactive;
+    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
+    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], J [ch][2][21][41], dE_jac [ch][20][41], then the tile blocks
+    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + FJAC_NJ + FJAC_NH);
+    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
+    struct Pending { cudaStream_t q; size_t r; int n; const double *J, *H; } pend{};
+    auto download = [&](const Pending& c) -> int {
+        if (J) CU(cudaMemcpyAsync(J + c.r * FJAC_NJ, c.J, (size_t)c.n * FJAC_NJ * D, cudaMemcpyDeviceToHost, c.q));
+        if (dE_jac) CU(cudaMemcpyAsync(dE_jac + c.r * FJAC_NH, c.H, (size_t)c.n * FJAC_NH * D, cudaMemcpyDeviceToHost, c.q));
+        return RCM_OK;
+    };
+    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
+        const int n = std::min((int)ch, col0 + ncol - c0);
+        const size_t r = (size_t)(c0 - col0);
+        cudaStream_t q = s->dg_stream[k % 2];
+        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
+        double* dT = p; p += ch * NLAY;
+        double* dTprev = p; p += ch * NLAY;
+        double* dvmr = p; p += ch * na * NLAY;
+        double* dstat = p; p += ch;
+        double* dJ = p; p += ch * FJAC_NJ;
+        double* dH = p;
+        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
+        SplitArgs a;
+        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, vmr_scale ? &sc : nullptr, a)) != RCM_OK) return st;
+        FjacArgs g{};
+        g.ncol = n;
+        g.clampk = s->clampk;
+        g.tau_clamp = s->tau_clamp;
+        g.T_floor = s->T_floor;
+        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+        g.coef = s->d_coef3;
+        g.planck_c = s->d_planck_c;
+        g.planck_k = s->d_planck_k;
+        g.exp_tab = s->d_exp_tab;
+        g.tile = dtile;
+        g.T = dT;
+        g.Ts = s->d_Ts + c0;
+        g.J = dJ;
+        g.dE_jac = dH;
+        CU(rcm_launch_fjac(g, q));
+        s->launches += 1;
+        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
+        pend = {q, r, n, dJ, dH};
     }
     if ((st = download(pend)) != RCM_OK) return st;
     return diag_end(s);

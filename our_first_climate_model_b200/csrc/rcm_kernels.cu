@@ -23,6 +23,7 @@
 #include "rcm_kernels.cuh"
 #include "rcm_diag.cuh"
 #include "rcm_jac.cuh"
+#include "rcm_fjac.cuh"
 
 __constant__ DevConst cst;
 
@@ -195,6 +196,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_split_kernels.cuh"
 #include "rcm_diag_kernels.cuh"
 #include "rcm_jac_kernels.cuh"
+#include "rcm_fjac_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -420,5 +422,15 @@ cudaError_t rcm_launch_jac_sum(const JacArgs& a, cudaStream_t st) {
     const size_t blocks = ((size_t)a.ncol * JAC_NK + 255) / 256;
     const int grid = blocks < 4096 ? (int)blocks : 4096;
     rcm_jac_sum_kernel<<<grid, 256, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+int rcm_fjac_ctas_per_sm() { return FJAC_CTAS; }
+
+cudaError_t rcm_launch_fjac(const FjacArgs& a, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_fjac_kernel<true> : rcm_fjac_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FJAC_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<(a.ncol + FJAC_WARPS - 1) / FJAC_WARPS, FJAC_NT, FJAC_SMEM, st>>>(a);
     return cudaGetLastError();
 }
