@@ -118,7 +118,9 @@ def init_columns(plevel, Tlevel, vmr_ppm_level, co2_factor=1.0):
     return out
 
 
-def read_tau(tab, plevel, Tlayer, vmr9, cloud_on=True, tau_s=2.0):
+def read_tau(tab, plevel, Tlayer, vmr9, cloud_on=True, tau_s=2.0, cloud_layer=17, tau_floor=None):
+    """tau [nwvl][20] with the grey cloud in cloud_layer (< 0: none); tau_floor: tau = max(tau, tau_floor) after the cloud,
+    the lower clamp the solver's kernels apply where the reference's exp overflows (DESIGN.md section 4)."""
     t = ctable(tab)
     nw = t.n_wvl
     pl = np.ascontiguousarray(plevel, dtype=np.float64)
@@ -127,13 +129,16 @@ def read_tau(tab, plevel, Tlayer, vmr9, cloud_on=True, tau_s=2.0):
     tau = np.zeros((nw, NLAY)); lp = np.zeros(NLAY, dtype=np.int64); lt = np.zeros(NLAY, dtype=np.int64)
     lib().rcmo_read_tau(C.byref(t), C.c_int(NLEV), _p(pl), _p(T), _p(v), _p(tau), _p(lp), _p(lt))
     if cloud_on:
-        lib().rcmo_cloud_into_tau(_p(tau), C.c_int(nw), C.c_int(NLAY), C.c_int(17), C.c_double(tau_s / 2.0))
+        lib().rcmo_cloud_into_tau(_p(tau), C.c_int(nw), C.c_int(NLAY), C.c_int(cloud_layer), C.c_double(tau_s / 2.0))
+    if tau_floor is not None:
+        tau = np.maximum(tau, tau_floor)
     return tau, lp, lt
 
 
-def radiative_transfer(tau, wvl, weight, Tlayer, T_surface, solar_irr):
+def radiative_transfer(tau, wvl, weight, Tlayer, T_surface, solar_irr, nangle=30):
     tau = np.ascontiguousarray(tau, dtype=np.float64)
     p = default_params(solar_irr)
+    p.nangle = nangle
     Ed = np.zeros(NLEV); Eu = np.zeros(NLEV); dE = np.zeros(NLAY)
     lib().rcmo_radiative_transfer(C.byref(p), C.c_int(tau.shape[0]), _p(tau),
                                   _p(np.ascontiguousarray(wvl, dtype=np.float64)),
