@@ -265,6 +265,34 @@ int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_s
  * ln q_l) for l < k (so row E_up[20] has only its T_surf entry).  Synchronous; changes nothing.  Device scratch of its own
  * (about 0.4 GB, independent of the wavelengths).  Errors as rcm_radiative_kernels. */
 int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
+/* Stratosphere-adjusted forcing of the columns [col0, col0 + ncol) by fixed dynamical heating (SARF: Manabe & Wetherald;
+ * Hansen et al. 1997), next to the instantaneous forcing (IRF).
+ * Base state: the state rcm_diagnose_fluxes(..., NULL, ...) radiates (after the theta-sort and the water-vapour feedback,
+ * with the grey or per-column cloud and the step-0 rule).  Perturbed state: the same with vmr_scale applied exactly as the
+ * other calls apply it (NULL = all 1).
+ * Stratosphere: ntrop[c] in [0, 19] (required, never NULL) is the number of stratospheric layers of column c, layers
+ * 0 .. ntrop - 1 top-down; the tropopause is level ntrop[c].
+ * Adjustment dT: dT_l for l < ntrop is added to layer l's temperature in both places it enters, its Planck source and the
+ * temperature its tau is interpolated at (the d/dT_l of rcm_radiative_kernels and rcm_flux_jacobian; at step 0 it moves
+ * both the sorted and the unsorted profile).  Troposphere, surface and all VMRs stay fixed; no re-sort, no feedback.
+ * Solved for: dE_l(perturbed, T + dT) = dE_l(base, T) for every l < ntrop, by Newton on the ntrop x ntrop block of dE_jac
+ * (entries 0 .. ntrop - 1 of rows 0 .. ntrop - 1), re-evaluated at every iterate; FP64 Gaussian elimination with partial
+ * pivoting (lowest row on ties).
+ * Convergence: a column has converged when max_{l < ntrop} |dE_l - dE_l^base| <= tol (W m-2).  From then on it is frozen:
+ * its outputs are those of the evaluation that met the test, and later iterations do not touch it.
+ * iters[c]: the number of Newton updates applied; -1 when max_iter updates did not converge, when the linear solve met a
+ * zero or non-finite pivot, or when the residual is not finite - the outputs then hold the last evaluated iterate and the
+ * call still returns RCM_OK.
+ * Outputs (host, any may be NULL), with N_k = E_down[k] - E_up[k] computed as (Ed'[k] - Eu'[k]) - (Ed[k] - Eu[k]):
+ * F [ncol][4]: 0 IRF at TOA, 1 IRF at the tropopause level, 2 SARF at TOA, 3 SARF at the tropopause level (W m-2);
+ * dT_adj [ncol][20] (K, exactly 0.0 for l >= ntrop); E_down, E_up [ncol][21] broadband fluxes at the adjusted perturbed
+ * state; iters [ncol].  Every value is a function of its column alone: ranges, shards and chunks give bit-identical results.
+ * Synchronous; changes nothing.  Device scratch of its own: 7,113 doubles and 2 ints per column of a chunk (8,192 at most)
+ * plus the tile blocks, twice - 957,219,328 bytes for 8,192 columns and 100 wavelengths (42 x nwvl + 2,913 doubles per
+ * column in general).  Errors as rcm_flux_jacobian; also RCM_ERR_ARG when ntrop is NULL or an entry lies outside [0, 19],
+ * tol is not finite or not > 0, or max_iter < 1. */
+int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol,
+                         int max_iter, double* F, double* dT_adj, double* E_down, double* E_up, int* iters);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

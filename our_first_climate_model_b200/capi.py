@@ -453,6 +453,37 @@ class Solver:
         _check(_lib.rcm_flux_jacobian(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(J), _p(H)), self._h)
         return dict(J=J, dE_jac=H)
 
+    def adjusted_forcing(self, vmr_scale, ntrop, col0: int = 0, ncol: int | None = None, tol: float = 1e-6,
+                         max_iter: int = 20) -> dict:
+        """rcm_adjusted_forcing: stratosphere-adjusted forcing by fixed dynamical heating for columns [col0, col0 + ncol),
+        without changing anything.  vmr_scale as in diagnose_fluxes (None = unscaled: no forcing); ntrop: the stratospheric
+        layers 0 .. ntrop - 1 of every column, an int or an array [ncol] of values in [0, 19]; Newton until
+        max_{l < ntrop} |dE_l - dE_l^base| <= tol (W/m2), at most max_iter updates.
+        -> F [ncol, 4] with the views IRF_toa, IRF_trop, SARF_toa, SARF_trop (W/m2), dT_adj [ncol, 20] (K), E_down, E_up
+        [ncol, 21] at the adjusted perturbed state, iters [ncol] (Newton updates applied, -1: not converged) and
+        converged [ncol] (iters >= 0)."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        m = max(n, 0)
+        sc = None
+        if vmr_scale is not None:
+            sc = _f64(vmr_scale).ravel()
+            if sc.size != self.nactive:
+                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        nt = np.asarray(ntrop)
+        if nt.ndim == 0:
+            nt = np.full(m, int(nt), dtype=np.int32)
+        elif nt.shape != (m,):
+            raise ValueError(f"ntrop needs one entry per column ({m}), got shape {nt.shape}")
+        nt = np.ascontiguousarray(nt, dtype=np.int32)
+        F = np.zeros((m, 4))
+        dT = np.zeros((m, NLAY))
+        Ed, Eu = np.zeros((m, NLEV)), np.zeros((m, NLEV))
+        it = np.zeros(m, dtype=np.int32)
+        _check(_lib.rcm_adjusted_forcing(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(nt), C.c_double(tol),
+                                         C.c_int(max_iter), _p(F), _p(dT), _p(Ed), _p(Eu), _p(it)), self._h)
+        return dict(F=F, IRF_toa=F[:, 0], IRF_trop=F[:, 1], SARF_toa=F[:, 2], SARF_trop=F[:, 3], dT_adj=dT, E_down=Ed,
+                    E_up=Eu, iters=it, converged=it >= 0)
+
     def advance(self, nsteps: int, want_scalars=True):
         sc = (StepScalars * nsteps)() if want_scalars else None
         _check(_lib.rcm_advance(self._h, C.c_int(nsteps), sc), self._h)

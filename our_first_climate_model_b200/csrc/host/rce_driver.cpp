@@ -9,6 +9,7 @@
 //   rcm_rce --atm test.atm --table Reduced100Forcing.nc [--ncol N] [--seed S] [--max-steps M] [--check-every K]
 //           [--dT 1e-3] [--device D] [--out output.txt] [--checkpoint file] [--resume file] [--steps-exact]
 //           [--spectral-out spectrum.csv] [--kernels-out kernels.csv] [--jacobian-out jacobian.csv]
+//           [--forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
@@ -37,6 +38,14 @@
 // (rcm_flux_jacobian's dE_jac) - header "layer,p_layer,dT_0..dT_19,dT_surf,dlnq_0..dlnq_19", then one row per layer l
 // (top-down; p_layer in hPa) with the ensemble means of d dE_l/dx_e (W/m2 per K resp. per unit ln q) for the 41 entries x_e.
 // Summed in column order: the file is byte-identical for any --gpus N.
+//
+// --forcing-out FILE (repwvl tables only): after the run, the stratosphere-adjusted forcing of the next step's state by fixed
+// dynamical heating (rcm_adjusted_forcing, tol 1e-6 W/m2, at most 20 Newton updates) for the factors --forcing-scale on the
+// five active species' VMRs (H2O, CO2, O3, N2O, CH4; default 1,2,1,1,1: doubled CO2) with the --trop-layers top layers
+// (default 4) as the stratosphere - header "layer,p_layer,dT_adj", then one row per layer (top-down; p_layer in hPa) with the
+// ensemble-mean adjustment (K), then the rows "IRF_toa,,v", "IRF_trop,,v", "SARF_toa,,v", "SARF_trop,,v" with the ensemble
+// means (W/m2) and "unconverged,,n" with the number of columns that did not converge.  Summed in column order: the file is
+// byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -94,6 +103,11 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     double* K_out;
     int jacobian;             // --jacobian-out: rows [ncol][20][41] of rcm_flux_jacobian's dE_jac into H_out
     double* H_out;
+    int forcing;              // --forcing-out: rcm_adjusted_forcing's F [ncol][4], dT_adj [ncol][20], iters [ncol]
+    const double* forcing_scale;
+    const int* ntrop;         // [ncol]
+    double *F_out, *dTadj_out;
+    int* iters_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -197,6 +211,39 @@ int write_jacobian(const std::string& path, int ncol, const double* player, cons
     return 0;
 }
 
+constexpr int FORCING_MAX_ITER = 20;
+constexpr double FORCING_TOL = 1e-6;
+
+// ensemble means of the adjusted forcing, summed in column order
+int write_forcing(const std::string& path, int ncol, const double* player, const double* F, const double* dT, const int* iters) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    constexpr int NLAY = RCM_NLAYER;
+    std::fprintf(f, "layer,p_layer,dT_adj\n");
+    for (int l = 0; l < NLAY; ++l) {
+        double sum = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) sum += dT[c * NLAY + l];
+        std::fprintf(f, "%d,%.17g,%.17g\n", l, player[l], sum / ncol);
+    }
+    const char* names[4] = {"IRF_toa", "IRF_trop", "SARF_toa", "SARF_trop"};
+    for (int k = 0; k < 4; ++k) {
+        double sum = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) sum += F[c * 4 + k];
+        std::fprintf(f, "%s,,%.17g\n", names[k], sum / ncol);
+    }
+    int bad = 0;
+    for (size_t c = 0; c < (size_t)ncol; ++c) bad += iters[c] < 0;
+    std::fprintf(f, "unconverged,,%d\n", bad);
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
+
 void run_shard(Shard* sh, const Job* j) {
     auto fail = [&](const char* what, int st) {
         sh->err = std::string(what) + ": " + rcm_status_string(st) + (sh->s ? std::string(" - ") + rcm_last_error(sh->s) : "");
@@ -275,13 +322,18 @@ void run_shard(Shard* sh, const Job* j) {
         st = rcm_flux_jacobian(sh->s, 0, (int)n, nullptr, nullptr, j->H_out + lo * JAC_NH);
         if (st != RCM_OK) return fail("rcm_flux_jacobian", st);
     }
+    if (j->forcing) {
+        st = rcm_adjusted_forcing(sh->s, 0, (int)n, j->forcing_scale, j->ntrop + lo, FORCING_TOL, FORCING_MAX_ITER, j->F_out + lo * 4,
+                                  j->dTadj_out + lo * NLAY, nullptr, nullptr, j->iters_out + lo);
+        if (st != RCM_OK) return fail("rcm_adjusted_forcing", st);
+    }
 }
 
 }  // namespace
 
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
-        jacobian_path;
+        jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4";
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -308,6 +360,9 @@ int main(int argc, char** argv) {
         else if (a == "--spectral-out") spectral_path = val();
         else if (a == "--kernels-out") kernels_path = val();
         else if (a == "--jacobian-out") jacobian_path = val();
+        else if (a == "--forcing-out") forcing_path = val();
+        else if (a == "--forcing-scale") forcing_scale_arg = val();
+        else if (a == "--trop-layers") trop_layers_arg = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -317,7 +372,8 @@ int main(int argc, char** argv) {
         gpus > ncol) {
         std::fprintf(stderr, "usage: rcm_rce --atm FILE (--table FILE | --lbl DIR [--co2-factor F]) [--ncol N] [--seed S] [--max-steps M] [--check-every K] "
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
-                             "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE]\n");
+                             "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE] "
+                             "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -331,6 +387,27 @@ int main(int argc, char** argv) {
     if (!lbl_dir.empty() && !jacobian_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --jacobian-out needs a repwvl table (--table): the line-by-line path has no flux Jacobians\n");
         return 1;
+    }
+    if (!lbl_dir.empty() && !forcing_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --forcing-out needs a repwvl table (--table): the line-by-line path has no adjusted forcing\n");
+        return 1;
+    }
+    double forcing_scale[5];
+    int trop_layers = 0;
+    if (!forcing_path.empty()) {  // --forcing-scale: exactly five numbers; --trop-layers: one integer in [0, 19]
+        int k = 0;
+        const char* q = forcing_scale_arg.c_str();
+        for (char* e = nullptr; k < 5; ++k, q = e + 1) {
+            forcing_scale[k] = std::strtod(q, &e);
+            if (e == q || (k < 4 && *e != ',') || (k == 4 && *e != '\0')) break;
+        }
+        char* e = nullptr;
+        const long tl = std::strtol(trop_layers_arg.c_str(), &e, 10);
+        if (k < 5 || e == trop_layers_arg.c_str() || *e != '\0' || tl < 0 || tl > RCM_NLAYER - 1) {
+            std::fprintf(stderr, "rcm_rce: --forcing-scale needs five comma-separated factors and --trop-layers an integer in [0, 19]\n");
+            return 1;
+        }
+        trop_layers = (int)tl;
     }
 
     // ---- the column of the .atm file (main.cpp:396-430) and its ensemble ---------------------------
@@ -416,9 +493,13 @@ int main(int argc, char** argv) {
         }
         std::vector<double> K(kernels_path.empty() ? 0 : n * KERN_NK);
         std::vector<double> H(jacobian_path.empty() ? 0 : n * JAC_NH);
+        const bool forcing = !forcing_path.empty();
+        std::vector<double> Ff(forcing ? n * 4 : 0), dTf(forcing ? n * NLAY : 0);
+        std::vector<int> itf(forcing ? n : 0), ntrop(n, trop_layers);
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
-                dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data()};
+                dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data(),
+                forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -461,6 +542,10 @@ int main(int argc, char** argv) {
             return 1;
         }
         if (!jacobian_path.empty() && write_jacobian(jacobian_path, ncol, player.data(), H.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
+        if (forcing && write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) {
             rcm_table_free(table);
             return 1;
         }
@@ -586,6 +671,14 @@ int main(int argc, char** argv) {
         st = rcm_flux_jacobian(s, 0, ncol, nullptr, nullptr, H.data());
         if (st != RCM_OK) return die("rcm_flux_jacobian", st, s);
         if (write_jacobian(jacobian_path, ncol, player.data(), H.data())) return 1;
+    }
+    if (!forcing_path.empty()) {
+        std::vector<double> Ff(m * 4), dTf(m * NLAY);
+        std::vector<int> itf(m), ntrop(m, trop_layers);
+        st = rcm_adjusted_forcing(s, 0, ncol, forcing_scale, ntrop.data(), FORCING_TOL, FORCING_MAX_ITER, Ff.data(), dTf.data(), nullptr,
+                                  nullptr, itf.data());
+        if (st != RCM_OK) return die("rcm_adjusted_forcing", st, s);
+        if (write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) return 1;
     }
     double ts_mean = 0.0;
     for (size_t c = 0; c < m; ++c) ts_mean += Ts[c];

@@ -12,7 +12,7 @@
 #include <vector>
 
 #include "rcm_jac.cuh"
-#include "rcm_fjac.cuh"
+#include "rcm_fdh.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -103,6 +103,7 @@ struct rcm_solver {
     size_t diagnose_bytes = 0;
     cudaStream_t dg_stream[2] = {nullptr, nullptr};  // ... the chunks alternate between two streams and the two sets
     cudaEvent_t dg_fork = nullptr, dg_join[2] = {nullptr, nullptr};
+    int* h_fdh_count = nullptr;  // rcm_adjusted_forcing: the active count of each stream's chunk (pinned, read every iteration)
 };
 
 namespace {
@@ -930,6 +931,7 @@ int rcm_destroy(rcm_solver* s) {
         if (s->dg_join[i]) cudaEventDestroy(s->dg_join[i]);
     }
     if (s->dg_fork) cudaEventDestroy(s->dg_fork);
+    if (s->h_fdh_count) cudaFreeHost(s->h_fdh_count);
     if (s->hg.exec) cudaGraphExecDestroy(s->hg.exec);
     if (s->own_stream) cudaStreamDestroy(s->own_stream);
     delete s;
@@ -1735,6 +1737,213 @@ int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale
         pend = {q, r, n, dJ, dH};
     }
     if ((st = download(pend)) != RCM_OK) return st;
+    return diag_end(s);
+}
+
+// Stratosphere-adjusted forcing: the chunks, streams, state copies and prep of the calls above.  Per chunk a base evaluation
+// (unscaled), the VMR scaling, then Newton iterations: retemper, evaluation (rcm_diag_rt_kernel + rcm_diag_sum_kernel),
+// check; while columns are active, the flux Jacobian (rcm_fjac_kernel) and the Newton step.  The host reads a chunk's active
+// count after every check.  The chunks of the two streams take turns: one chunk's kernels run while the host waits for the
+// other's count.
+int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol, int max_iter,
+                         double* F, double* dT_adj, double* E_down, double* E_up, int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_adjusted_forcing";
+    DiagScale sc{};
+    int st = diag_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, fn + ": needs H2O among the active species");
+    if (!ntrop) return fail(s, RCM_ERR_ARG, fn + ": ntrop is NULL");
+    for (int c = 0; c < ncol; ++c)
+        if (ntrop[c] < 0 || ntrop[c] > FDH_MAXM)
+            return fail(s, RCM_ERR_ARG, fn + ": ntrop[" + std::to_string(c) + "] = " + std::to_string(ntrop[c]) + " outside [0, 19]");
+    if (!std::isfinite(tol) || !(tol > 0.0)) return fail(s, RCM_ERR_ARG, fn + ": tol must be finite and > 0");
+    if (max_iter < 1) return fail(s, RCM_ERR_ARG, fn + ": max_iter must be >= 1");
+    CU(cudaSetDevice(s->device));
+    st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
+    const int nwvl = s->dc.nwvl, na = s->nactive, nsm = nsm_of(s);
+    const bool first = (s->step_index == 0);
+    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
+    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], T_tau, T + dT, dT [ch][20], E_down, E_up [ch][21] and
+    // dE [ch][20] of the base and of the current iterate, F [ch][4], the output E_down, E_up [ch][21], J [ch][2][21][41],
+    // dE_jac [ch][20][41], spectral [2][ch][nwvl][21]; ntrop, iters [ch] and the active count; then the tile blocks
+    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 3 * NLAY + 2 * (2 * NLEV + NLAY) + 4 + 2 * NLEV + FJAC_NJ + FJAC_NH) +
+                         2 * ch * nwvl * NLEV;
+    const size_t n_int = 2 * ch + 1;
+    const size_t tile_off = (n_dbl * D + n_int * sizeof(int) + 255) / 256 * 256,
+                 set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
+    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
+    struct Slot {
+        cudaStream_t q;
+        int c0 = 0, n = 0, iter = 0;
+        bool live = false;
+        double *T, *Tprev, *vmr, *stat, *Ttau, *Tp, *dT, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *spec_dn, *spec_up;
+        int *ntrop, *iters, *count;
+        unsigned char* tile;
+        SplitArgs a;
+    } slot[2];
+    for (int k = 0; k < 2; ++k) {
+        Slot& z = slot[k];
+        z.q = s->dg_stream[k];
+        double* p = reinterpret_cast<double*>(s->d_diagnose + k * set_bytes);
+        z.T = p; p += ch * NLAY;
+        z.Tprev = p; p += ch * NLAY;
+        z.vmr = p; p += ch * na * NLAY;
+        z.stat = p; p += ch;
+        z.Ttau = p; p += ch * NLAY;
+        z.Tp = p; p += ch * NLAY;
+        z.dT = p; p += ch * NLAY;
+        z.Ed0 = p; p += ch * NLEV;
+        z.Eu0 = p; p += ch * NLEV;
+        z.dE0 = p; p += ch * NLAY;
+        z.Ed = p; p += ch * NLEV;
+        z.Eu = p; p += ch * NLEV;
+        z.dE = p; p += ch * NLAY;
+        z.F = p; p += ch * 4;
+        z.Edo = p; p += ch * NLEV;
+        z.Euo = p; p += ch * NLEV;
+        z.J = p; p += ch * FJAC_NJ;
+        z.H = p; p += ch * FJAC_NH;
+        z.spec_dn = p; p += ch * nwvl * NLEV;
+        z.spec_up = p; p += ch * nwvl * NLEV;
+        int* ip = reinterpret_cast<int*>(p);
+        z.ntrop = ip; ip += ch;
+        z.iters = ip; ip += ch;
+        z.count = ip;
+        z.tile = s->d_diagnose + k * set_bytes + tile_off;
+    }
+    // broadband fluxes of the chunk's tile blocks into Ed, Eu, dE (rcm_diagnose_fluxes' kernels)
+    auto evaluate = [&](Slot& z, double* Ed, double* Eu, double* dE) -> int {
+        DiagArgs g{};
+        g.ncol = z.n;
+        g.ntiles = z.a.ntiles;
+        g.nsplit = z.a.nsplit;
+        g.ipu = z.a.ipu;
+        g.nitem = z.a.nitem;
+        g.nunits = z.a.nunits;
+        g.clampk = s->clampk;
+        g.tau_clamp = s->tau_clamp;
+        g.coef = s->d_coef3;
+        g.planck_c = s->d_planck_c;
+        g.planck_k = s->d_planck_k;
+        g.exp_tab = s->d_exp_tab;
+        g.tile = z.tile;
+        g.spec_dn = z.spec_dn;
+        g.spec_up = z.spec_up;
+        g.E_down = Ed;
+        g.E_up = Eu;
+        g.dE = dE;
+        g.solar_col = z.a.solar_col;
+        CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm), z.q));
+        CU(rcm_launch_diag_sum(g, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    auto fdh_args = [&](const Slot& z) {
+        FdhArgs f{};
+        f.ncol = z.n;
+        f.iter = z.iter;
+        f.max_iter = max_iter;
+        f.tol = tol;
+        f.T_floor = s->T_floor;
+        f.tile = z.tile;
+        f.Tb = z.T;
+        f.Ttau = first ? z.Ttau : z.T;
+        f.Tp = z.Tp;
+        f.dT = z.dT;
+        f.ntrop = z.ntrop;
+        f.Ed0 = z.Ed0;
+        f.Eu0 = z.Eu0;
+        f.dE0 = z.dE0;
+        f.Ed = z.Ed;
+        f.Eu = z.Eu;
+        f.dE = z.dE;
+        f.dE_jac = z.H;
+        f.iters = z.iters;
+        f.F = z.F;
+        f.Ed_out = z.Edo;
+        f.Eu_out = z.Euo;
+        f.nactive = z.count;
+        return f;
+    };
+    // iterate z.iter: the tile blocks at T + dT, their fluxes, the check, the active count into h_fdh_count[k]
+    auto check = [&](Slot& z, int k) -> int {
+        const FdhArgs f = fdh_args(z);
+        CU(rcm_launch_fdh_retemper(f, z.q));
+        if ((st = evaluate(z, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
+        CU(rcm_launch_fdh_check(f, z.q));
+        CU(cudaMemcpyAsync(s->h_fdh_count + k, z.count, sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    auto newton = [&](Slot& z) -> int {
+        FjacArgs g{};
+        g.ncol = z.n;
+        g.clampk = s->clampk;
+        g.tau_clamp = s->tau_clamp;
+        g.T_floor = s->T_floor;
+        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+        g.coef = s->d_coef3;
+        g.planck_c = s->d_planck_c;
+        g.planck_k = s->d_planck_k;
+        g.exp_tab = s->d_exp_tab;
+        g.tile = z.tile;
+        g.T = z.Tp;
+        g.Ts = s->d_Ts + z.c0;
+        g.J = z.J;
+        g.dE_jac = z.H;
+        CU(rcm_launch_fjac(g, z.q));
+        CU(rcm_launch_fdh_newton(fdh_args(z), z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the chunk [c0, c0 + n): T_tau, prep, base evaluation, scaling, iterate 0
+    auto start = [&](Slot& z, int k, int c0) -> int {
+        z.c0 = c0;
+        z.n = std::min((int)ch, col0 + ncol - c0);
+        z.iter = 0;
+        z.live = true;
+        if (first) CU(cudaMemcpyAsync(z.Ttau, s->d_T + (size_t)c0 * NLAY, z.n * NLAY * D, cudaMemcpyDeviceToDevice, z.q));
+        CU(cudaMemcpyAsync(z.ntrop, ntrop + (c0 - col0), z.n * sizeof(int), cudaMemcpyHostToDevice, z.q));
+        if ((st = diag_prep(s, z.q, c0, z.n, z.T, z.Tprev, z.vmr, z.stat, z.tile, nullptr, z.a)) != RCM_OK) return st;
+        if ((st = evaluate(z, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
+        if (vmr_scale) {
+            CU(rcm_launch_diag_scale(z.tile, z.a.ntiles, sc, z.q));
+            s->launches += 1;
+        }
+        return check(z, k);
+    };
+    auto download = [&](const Slot& z) -> int {
+        const size_t r = (size_t)(z.c0 - col0);
+        if (F) CU(cudaMemcpyAsync(F + r * 4, z.F, z.n * 4 * D, cudaMemcpyDeviceToHost, z.q));
+        if (dT_adj) CU(cudaMemcpyAsync(dT_adj + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        return RCM_OK;
+    };
+    int next = col0;
+    for (int k = 0; k < 2 && next < col0 + ncol; ++k, next += (int)ch)
+        if ((st = start(slot[k], k, next)) != RCM_OK) return st;
+    for (int k = 0; slot[0].live || slot[1].live; k ^= 1) {
+        Slot& z = slot[k];
+        if (!z.live) continue;
+        CU(cudaStreamSynchronize(z.q));
+        if (s->h_fdh_count[k] > 0) {  // (none is left after iterate max_iter)
+            if ((st = newton(z)) != RCM_OK) return st;
+            ++z.iter;
+            if ((st = check(z, k)) != RCM_OK) return st;
+            continue;
+        }
+        if ((st = download(z)) != RCM_OK) return st;
+        z.live = false;
+        if (next < col0 + ncol) {
+            if ((st = start(z, k, next)) != RCM_OK) return st;
+            next += (int)ch;
+        }
+    }
     return diag_end(s);
 }
 

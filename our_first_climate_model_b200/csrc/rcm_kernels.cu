@@ -24,6 +24,7 @@
 #include "rcm_diag.cuh"
 #include "rcm_jac.cuh"
 #include "rcm_fjac.cuh"
+#include "rcm_fdh.cuh"
 
 __constant__ DevConst cst;
 
@@ -197,6 +198,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_diag_kernels.cuh"
 #include "rcm_jac_kernels.cuh"
 #include "rcm_fjac_kernels.cuh"
+#include "rcm_fdh_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -432,5 +434,20 @@ cudaError_t rcm_launch_fjac(const FjacArgs& a, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FJAC_SMEM);
     if (e != cudaSuccess) return e;
     kern<<<(a.ncol + FJAC_WARPS - 1) / FJAC_WARPS, FJAC_NT, FJAC_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_fdh_retemper(const FdhArgs& a, cudaStream_t st) {
+    rcm_fdh_retemper_kernel<<<(a.ncol * NLAY + 255) / 256, 256, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_fdh_check(const FdhArgs& a, cudaStream_t st) {
+    rcm_fdh_check_kernel<<<(a.ncol + FDH_CHECK_NT - 1) / FDH_CHECK_NT, FDH_CHECK_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_fdh_newton(const FdhArgs& a, cudaStream_t st) {
+    rcm_fdh_newton_kernel<<<(a.ncol + FDH_NEWTON_WARPS - 1) / FDH_NEWTON_WARPS, FDH_NEWTON_NT, 0, st>>>(a);
     return cudaGetLastError();
 }
