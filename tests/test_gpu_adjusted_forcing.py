@@ -31,19 +31,15 @@ def ens21(rcm):
 
 
 # ---- the port's fixed-dynamical-heating solve -----------------------------------------------------------------------------
-class PortColumn:
-    """One column of the port: fluxes of the base state and of the perturbed state at T + dT (dT on layers 0 .. m - 1)."""
+class FdhColumn:
+    """The fixed-dynamical-heating problem of one column: fluxes(v9, dT) -> E_down [21], E_up [21], dE [20] of the next
+    step with the VMRs v9 and dT added to layers 0 .. len(dT) - 1 of both the profile tau is interpolated at and the radiated
+    profile; v0 the base VMRs, v1 the perturbed ones.  fluxes is given, or a subclass's method."""
 
-    def __init__(self, port, tab, st, T, vmr9, rel_hum, Tsurf, first, co2_scale, tau_s):
-        self.port, self.tab, self.pl, self.Tsurf, self.tau_s = port, tab, st["plevel"], Tsurf, tau_s
-        self.tau_T, self.Trad, self.v0 = radiated_inputs(port, st, T, vmr9, rel_hum, first)
-        self.v1 = radiated_inputs(port, st, T, vmr9, rel_hum, first, co2_scale=co2_scale)[2]
-
-    def fluxes(self, v9, dT=()):
-        d = np.zeros(NLAY)
-        d[:len(dT)] = dT
-        tau, _, _ = self.port.read_tau(self.tab, self.pl, self.tau_T + d, v9, tau_s=self.tau_s)
-        return self.port.radiative_transfer(tau, self.tab["wvl"], self.tab["weight"], self.Trad + d, self.Tsurf, 0.0)
+    def __init__(self, v0, v1, fluxes=None):
+        self.v0, self.v1 = v0, v1
+        if fluxes is not None:
+            self.fluxes = fluxes
 
     def solve(self, m):
         """-> dT [20], F [4] of the port's own solution (tight hybr tolerance, from dT = 0)."""
@@ -65,6 +61,21 @@ class PortColumn:
         if m == 0:
             return 0.0
         return np.abs(self.fluxes(self.v1, dT[:m])[2][:m] - self.fluxes(self.v0)[2][:m]).max()
+
+
+class PortColumn(FdhColumn):
+    """One column of the port at 30 angles with the cloud in layer 17 (optical depth tau_s), perturbed by co2_scale."""
+
+    def __init__(self, port, tab, st, T, vmr9, rel_hum, Tsurf, first, co2_scale, tau_s):
+        self.port, self.tab, self.pl, self.Tsurf, self.tau_s = port, tab, st["plevel"], Tsurf, tau_s
+        self.tau_T, self.Trad, v0 = radiated_inputs(port, st, T, vmr9, rel_hum, first)
+        super().__init__(v0, radiated_inputs(port, st, T, vmr9, rel_hum, first, co2_scale=co2_scale)[2])
+
+    def fluxes(self, v9, dT=()):
+        d = np.zeros(NLAY)
+        d[:len(dT)] = dT
+        tau, _, _ = self.port.read_tau(self.tab, self.pl, self.tau_T + d, v9, tau_s=self.tau_s)
+        return self.port.radiative_transfer(tau, self.tab["wvl"], self.tab["weight"], self.Trad + d, self.Tsurf, 0.0)
 
 
 def check_against_port(port, s, st, tab, nsteps_done, vmr_scale, tau_s=None):
