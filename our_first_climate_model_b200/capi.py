@@ -394,16 +394,21 @@ class Solver:
         _check(_lib.rcm_radiative_transfer(self._h, _p(t), _p(Ed), _p(Eu), _p(dE)), self._h)
         return Ed, Eu, dE
 
+    def _vmr_scale(self, vmr_scale):
+        """vmr_scale of the diagnostic calls as contiguous float64 with one factor per active species (None stays None)."""
+        if vmr_scale is None:
+            return None
+        sc = _f64(vmr_scale).ravel()
+        if sc.size != self.nactive:
+            raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        return sc
+
     def diagnose_fluxes(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, spectral: bool = True) -> dict:
         """rcm_diagnose_fluxes: the fluxes the next step would compute for columns [col0, col0 + ncol), without changing
         anything.  vmr_scale [nactive]: factors on the active species' VMRs (ascending species index; None = unscaled).
         -> E_down, E_up [ncol, 21], dE [ncol, 20] and, with spectral, E_down_spec / E_up_spec [ncol, nwvl, 21]."""
         n = self.ncol - col0 if ncol is None else int(ncol)
-        sc = None
-        if vmr_scale is not None:
-            sc = _f64(vmr_scale).ravel()
-            if sc.size != self.nactive:
-                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        sc = self._vmr_scale(vmr_scale)
         m = max(n, 0)
         out = dict(E_down=np.zeros((m, NLEV)), E_up=np.zeros((m, NLEV)), dE=np.zeros((m, NLAY)))
         if spectral:
@@ -421,11 +426,7 @@ class Solver:
         views dOLR_dT [ncol, 20], dOLR_dTs [ncol], dOLR_dlnq [ncol, 20], dSFC_dT, dSFC_dlnq, and with spectral
         K_spec [ncol, nwvl, 2, 41] (each wavelength's contribution; K is its sum over the wavelengths in index order)."""
         n = self.ncol - col0 if ncol is None else int(ncol)
-        sc = None
-        if vmr_scale is not None:
-            sc = _f64(vmr_scale).ravel()
-            if sc.size != self.nactive:
-                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        sc = self._vmr_scale(vmr_scale)
         m = max(n, 0)
         K = np.zeros((m, 2, 2 * NLAY + 1))
         Ks = np.zeros((m, self.nwvl, 2, 2 * NLAY + 1)) if spectral else None
@@ -442,11 +443,7 @@ class Solver:
         radiative_kernels (dT_l for the 20 layers top-down, dT_surf, dln q_l for the 20 layers).
         -> J [ncol, 2, 21, 41] (J[:, 0, k] = dE_down[k], J[:, 1, k] = dE_up[k]) and dE_jac [ncol, 20, 41]."""
         n = self.ncol - col0 if ncol is None else int(ncol)
-        sc = None
-        if vmr_scale is not None:
-            sc = _f64(vmr_scale).ravel()
-            if sc.size != self.nactive:
-                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        sc = self._vmr_scale(vmr_scale)
         m = max(n, 0)
         J = np.zeros((m, 2, NLAY + 1, 2 * NLAY + 1))
         H = np.zeros((m, NLAY, 2 * NLAY + 1))
@@ -464,11 +461,7 @@ class Solver:
         converged [ncol] (iters >= 0)."""
         n = self.ncol - col0 if ncol is None else int(ncol)
         m = max(n, 0)
-        sc = None
-        if vmr_scale is not None:
-            sc = _f64(vmr_scale).ravel()
-            if sc.size != self.nactive:
-                raise ValueError(f"vmr_scale needs {self.nactive} factors (one per active species), got {sc.size}")
+        sc = self._vmr_scale(vmr_scale)
         nt = np.asarray(ntrop)
         if nt.ndim == 0:
             nt = np.full(m, int(nt), dtype=np.int32)

@@ -1443,19 +1443,23 @@ int rcm_get_state(rcm_solver* s, double* Tlayer, double* Tsurf, double* h2o, flo
 }
 
 // ------------------------------------------------------------------------------------------
-// Diagnostic calls (rcm_diagnose_fluxes, rcm_radiative_kernels, rcm_flux_jacobian).  The split path's prep kernel - the
-// sort, the water-vapour feedback and the table indices of the next step - runs on COPIES of a chunk's T, previous profile
-// and VMRs and writes its tile blocks into a scratch buffer; the solver's state, its tile blocks and every flag stay as they
-// are.  Chunks of at most 8,192 columns alternate between two streams with a scratch set each (about 0.6 GB with 100
-// wavelengths for the fluxes, 1.1 GB for the radiative kernels, 0.4 GB for the flux Jacobians, whatever the wavelengths):
-// the memory-bound sum kernel and the copies of one chunk overlap the radiative transfer of the next, and the last round of
-// one chunk's units the first of the next.
+// Diagnostic calls (rcm_diagnose_fluxes, rcm_radiative_kernels, rcm_flux_jacobian, rcm_adjusted_forcing).  The split path's
+// prep kernel - the sort, the water-vapour feedback and the table indices of the next step - runs on COPIES of a chunk's T,
+// previous profile and VMRs and writes its tile blocks into a scratch buffer; the solver's state, its tile blocks and every
+// flag stay as they are.  Chunks of at most 8,192 columns alternate between two streams with a scratch set each (about 0.6 GB
+// with 100 wavelengths for the fluxes, 1.1 GB for the radiative kernels, 0.4 GB for the flux Jacobians, whatever the
+// wavelengths): the memory-bound sum kernel and the copies of one chunk overlap the radiative transfer of the next, and the
+// last round of one chunk's units the first of the next.
 // ------------------------------------------------------------------------------------------
+extern "C++" {  // (templates)
 namespace {
 
 constexpr int kDiagMaxChunk = 8192;
 
-// the checks both calls make; the factors of vmr_scale (NULL = all 1) into sc
+// columns per chunk: whole tiles of 16, at most kDiagMaxChunk
+size_t diag_chunk(int ncol) { return (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16); }
+
+// the checks every call makes; the factors of vmr_scale (NULL = all 1) into sc
 int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
     if (s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": the line-by-line path is not supported");
     if (!s->has_table) return fail(s, RCM_ERR_STATE, fn + ": no lookup table loaded");
@@ -1473,12 +1477,52 @@ int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const d
     return RCM_OK;
 }
 
-// two scratch sets of set_bytes each, the two streams; work queued on the solver's stream comes first
-int diag_begin(rcm_solver* s, size_t set_bytes) {
+// A chunk's copies of what the prep reads - T, Tprev [ch][20], VMRs [ch][5][20] - its stationarity diagnostic stat [ch]
+// (unused), and the tile blocks it writes: the front and the end of every scratch set.
+struct DiagState {
+    double *T, *Tprev, *vmr, *stat;
+    unsigned char* tile;
+};
+
+// Hands out a scratch set front to back (doubles first, then ints).  On a null base it only counts.
+struct DiagCarve {
+    unsigned char* base;
+    size_t off = 0;
+    template <class T>
+    T* take(size_t n) {
+        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+        off += n * sizeof(T);
+        return p;
+    }
+};
+
+// The device, its constants, two scratch sets for chunks of ch columns and the two streams; work queued on the solver's stream
+// comes first.  A set is the state copies, what layout(m, ch, z) takes for the call's own arrays, then the tile blocks at a
+// 256-byte boundary.  The description runs once on a null base for the size of a set, then once on each set: the size and
+// the pointers cannot disagree.
+template <class Set, class Layout>
+int diag_begin(rcm_solver* s, size_t ch, Set (&set)[2], Layout layout) {
+    CU(cudaSetDevice(s->device));
+    const int st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    auto carve = [&](unsigned char* base, Set& z) {
+        DiagCarve m{base};
+        z.state.T = m.take<double>(ch * NLAY);
+        z.state.Tprev = m.take<double>(ch * NLAY);
+        z.state.vmr = m.take<double>(ch * s->nactive * NLAY);
+        z.state.stat = m.take<double>(ch);
+        layout(m, ch, z);
+        m.off = (m.off + 255) / 256 * 256;
+        z.state.tile = m.take<unsigned char>(ch / 16 * rcm_split_tile_bytes());
+        return (m.off + 255) / 256 * 256;
+    };
+    Set sized{};
+    const size_t set_bytes = carve(nullptr, sized);
     if (2 * set_bytes > s->diagnose_bytes) {
         CU(dalloc(s->d_diagnose, 2 * set_bytes));
         s->diagnose_bytes = 2 * set_bytes;
     }
+    for (int k = 0; k < 2; ++k) carve(s->d_diagnose + k * set_bytes, set[k]);
     if (!s->dg_fork) {
         for (int i = 0; i < 2; ++i) {
             CU(cudaStreamCreateWithFlags(&s->dg_stream[i], cudaStreamNonBlocking));
@@ -1491,23 +1535,21 @@ int diag_begin(rcm_solver* s, size_t set_bytes) {
     return RCM_OK;
 }
 
-// Copies of columns [c0, c0 + n) - T and Tprev into dT, dTprev [ch][20], VMRs into dvmr [ch][5][20] - and the prep of the
-// next step on them (dstat [ch]: its stationarity diagnostic, unused), tile blocks into dtile, then the VMR factors (sc:
-// NULL = unscaled).  On return dT holds the sorted profile the step radiates with; a carries the chunk's unit plan.
-int diag_prep(rcm_solver* s, cudaStream_t q, int c0, int n, double* dT, double* dTprev, double* dvmr, double* dstat,
-              unsigned char* dtile, const DiagScale* sc, SplitArgs& a) {
+// Copies of columns [c0, c0 + n) into d and the prep of the next step on them, tile blocks into d.tile, then the VMR factors
+// (sc: NULL = unscaled).  On return d.T holds the sorted profile the step radiates with; a carries the chunk's unit plan.
+int diag_prep(rcm_solver* s, cudaStream_t q, int c0, int n, const DiagState& d, const DiagScale* sc, SplitArgs& a) {
     constexpr size_t D = sizeof(double);
     const size_t o = (size_t)c0;
     const int na = s->nactive;
-    CU(cudaMemcpyAsync(dT, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-    CU(cudaMemcpyAsync(dTprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-    CU(cudaMemcpyAsync(dvmr, s->d_vmr + o * na * NLAY, (size_t)n * na * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(d.T, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(d.Tprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(d.vmr, s->d_vmr + o * na * NLAY, (size_t)n * na * NLAY * D, cudaMemcpyDeviceToDevice, q));
     a = split_args(s, c0, n, 0);
-    a.Tlayer = dT;
-    a.Tprev = dTprev;
-    a.vmr = dvmr;
-    a.dTstat = dstat;
-    a.tile = dtile;
+    a.Tlayer = d.T;
+    a.Tprev = d.Tprev;
+    a.vmr = d.vmr;
+    a.dTstat = d.stat;
+    a.tile = d.tile;
     a.counter = nullptr;
     a.part = nullptr;
     a.diag = nullptr;
@@ -1518,7 +1560,7 @@ int diag_prep(rcm_solver* s, cudaStream_t q, int c0, int n, double* dT, double* 
     f.first = (s->step_index == 0);
     f.write_all_vmr = 1;
     CU(rcm_launch_split_col(a, f, q));
-    if (sc) CU(rcm_launch_diag_scale(dtile, a.ntiles, *sc, q));
+    if (sc) CU(rcm_launch_diag_scale(d.tile, a.ntiles, *sc, q));
     s->launches += sc ? 2 : 1;
     return RCM_OK;
 }
@@ -1533,218 +1575,194 @@ int diag_end(rcm_solver* s) {
     return RCM_OK;
 }
 
+// what DiagArgs, JacArgs and FjacArgs take from the prep's arguments a: the chunk, the table, the clamp, the tile blocks
+template <class A>
+A diag_args(const SplitArgs& a) {
+    A g{};
+    g.ncol = a.ncol;
+    g.clampk = a.clampk;
+    g.tau_clamp = a.tau_clamp;
+    g.coef = a.coef;
+    g.planck_c = a.planck_c;
+    g.planck_k = a.planck_k;
+    g.exp_tab = a.exp_tab;
+    g.tile = a.tile;
+    return g;
+}
+
+// and the (tile, split) units of DiagArgs and JacArgs
+template <class A>
+A unit_args(const SplitArgs& a) {
+    A g = diag_args<A>(a);
+    g.ntiles = a.ntiles;
+    g.nsplit = a.nsplit;
+    g.ipu = a.ipu;
+    g.nitem = a.nitem;
+    g.nunits = a.nunits;
+    return g;
+}
+
+// rcm_diag_rt_kernel + rcm_diag_sum_kernel on the tile blocks of the prep a: the spectra dn, up and the broadband Ed, Eu, dE
+int diag_fluxes(rcm_solver* s, const SplitArgs& a, cudaStream_t q, double* dn, double* up, double* Ed, double* Eu, double* dE) {
+    DiagArgs g = unit_args<DiagArgs>(a);
+    g.spec_dn = dn;
+    g.spec_up = up;
+    g.E_down = Ed;
+    g.E_up = Eu;
+    g.dE = dE;
+    g.solar_col = a.solar_col;
+    CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm_of(s)), q));
+    CU(rcm_launch_diag_sum(g, q));
+    s->launches += 2;
+    return RCM_OK;
+}
+
+// rcm_fjac_kernel on the tile blocks of the prep a, the Planck source at T: J and dE_jac into J, H
+int flux_jacobian(rcm_solver* s, const SplitArgs& a, cudaStream_t q, const double* T, double* J, double* H) {
+    FjacArgs g = diag_args<FjacArgs>(a);
+    g.T_floor = a.T_floor;
+    g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    g.T = T;
+    g.Ts = a.Tsurf;
+    g.J = J;
+    g.dE_jac = H;
+    CU(rcm_launch_fjac(g, q));
+    s->launches += 1;
+    return RCM_OK;
+}
+
+// The chunks of a single-pass call.  Chunk k runs on stream k % 2 with scratch set k % 2 (chunk k + 2 reuses the set of chunk
+// k after it on the same stream): the prep (sc: VMR factors or NULL), then enqueue(z, a, q).  Its downloads, download(z, r,
+// n, q) for the output rows [r, r + n), are issued after the kernels of chunk k + 1: into pageable memory they block the host.
+template <class Set, class Layout, class Enqueue, class Download>
+int diag_chunks(rcm_solver* s, int col0, int ncol, const DiagScale* sc, Layout layout, Enqueue enqueue, Download download) {
+    const size_t ch = diag_chunk(ncol);
+    Set set[2];
+    int st = diag_begin(s, ch, set, layout);
+    if (st != RCM_OK) return st;
+    struct { const Set* z; size_t r; int n; cudaStream_t q; } pend{};
+    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
+        const int n = std::min((int)ch, col0 + ncol - c0);
+        const Set& z = set[k % 2];
+        cudaStream_t q = s->dg_stream[k % 2];
+        SplitArgs a;
+        if ((st = diag_prep(s, q, c0, n, z.state, sc, a)) != RCM_OK) return st;
+        if ((st = enqueue(z, a, q)) != RCM_OK) return st;
+        if (k > 0 && (st = download(*pend.z, pend.r, pend.n, pend.q)) != RCM_OK) return st;
+        pend = {&z, (size_t)(c0 - col0), n, q};
+    }
+    if ((st = download(*pend.z, pend.r, pend.n, pend.q)) != RCM_OK) return st;
+    return diag_end(s);
+}
+
 }  // namespace
+}  // extern "C++"
 
 int rcm_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* E_down_spec, double* E_up_spec,
                         double* E_down, double* E_up, double* dE) {
     if (!s) return RCM_ERR_ARG;
     DiagScale sc{};
-    int st = diag_check(s, "rcm_diagnose_fluxes", col0, ncol, vmr_scale, sc);
+    const int st = diag_check(s, "rcm_diagnose_fluxes", col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
-    CU(cudaSetDevice(s->device));
-    st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    const int nwvl = s->dc.nwvl, na = s->nactive;
-    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
-    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], E_down, E_up [ch][21], dE [ch][20], spectral [2][ch][nwvl][21],
-    // then the tile blocks
-    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 2 * NLEV + NLAY) + 2 * ch * nwvl * NLEV;
-    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
-    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
-    const bool scaled = vmr_scale != nullptr;
-    const int nsm = nsm_of(s);
-    // the downloads of chunk k are issued after the kernels of chunk k + 1: into pageable memory they block the host
-    struct Pending { cudaStream_t q; size_t r; int n; const double *dn, *up, *Ed, *Eu, *dE; } pend{};
-    auto download = [&](const Pending& c) -> int {
-        const size_t nspec = (size_t)c.n * nwvl * NLEV;
-        if (E_down_spec) CU(cudaMemcpyAsync(E_down_spec + c.r * nwvl * NLEV, c.dn, nspec * D, cudaMemcpyDeviceToHost, c.q));
-        if (E_up_spec) CU(cudaMemcpyAsync(E_up_spec + c.r * nwvl * NLEV, c.up, nspec * D, cudaMemcpyDeviceToHost, c.q));
-        if (E_down) CU(cudaMemcpyAsync(E_down + c.r * NLEV, c.Ed, c.n * NLEV * D, cudaMemcpyDeviceToHost, c.q));
-        if (E_up) CU(cudaMemcpyAsync(E_up + c.r * NLEV, c.Eu, c.n * NLEV * D, cudaMemcpyDeviceToHost, c.q));
-        if (dE) CU(cudaMemcpyAsync(dE + c.r * NLAY, c.dE, c.n * NLAY * D, cudaMemcpyDeviceToHost, c.q));
-        return RCM_OK;
+    const int nwvl = s->dc.nwvl;
+    constexpr size_t D = sizeof(double);
+    struct Set {
+        DiagState state;
+        double *Ed, *Eu, *dE, *spec_dn, *spec_up;
     };
-    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
-        const int n = std::min((int)ch, col0 + ncol - c0);
-        const size_t r = (size_t)(c0 - col0);
-        cudaStream_t q = s->dg_stream[k % 2];  // chunk k + 2 reuses the set of chunk k after it on the same stream
-        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
-        double* dT = p; p += ch * NLAY;
-        double* dTprev = p; p += ch * NLAY;
-        double* dvmr = p; p += ch * na * NLAY;
-        double* dstat = p; p += ch;
-        double* dEd = p; p += ch * NLEV;
-        double* dEu = p; p += ch * NLEV;
-        double* ddE = p; p += ch * NLAY;
-        double* dspec_dn = p; p += ch * nwvl * NLEV;
-        double* dspec_up = p;
-        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
-        SplitArgs a;
-        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, scaled ? &sc : nullptr, a)) != RCM_OK) return st;
-        DiagArgs g{};
-        g.ncol = n;
-        g.ntiles = a.ntiles;
-        g.nsplit = a.nsplit;
-        g.ipu = a.ipu;
-        g.nitem = a.nitem;
-        g.nunits = a.nunits;
-        g.clampk = s->clampk;
-        g.tau_clamp = s->tau_clamp;
-        g.coef = s->d_coef3;
-        g.planck_c = s->d_planck_c;
-        g.planck_k = s->d_planck_k;
-        g.exp_tab = s->d_exp_tab;
-        g.tile = dtile;
-        g.spec_dn = dspec_dn;
-        g.spec_up = dspec_up;
-        g.E_down = dEd;
-        g.E_up = dEu;
-        g.dE = ddE;
-        g.solar_col = a.solar_col;
-        CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm), q));
-        CU(rcm_launch_diag_sum(g, q));
-        s->launches += 2;
-        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
-        pend = {q, r, n, dspec_dn, dspec_up, dEd, dEu, ddE};
-    }
-    if ((st = download(pend)) != RCM_OK) return st;
-    return diag_end(s);
+    return diag_chunks<Set>(
+        s, col0, ncol, vmr_scale ? &sc : nullptr,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // E_down, E_up [ch][21], dE [ch][20], spectral [2][ch][nwvl][21]
+            z.Ed = m.take<double>(ch * NLEV);
+            z.Eu = m.take<double>(ch * NLEV);
+            z.dE = m.take<double>(ch * NLAY);
+            z.spec_dn = m.take<double>(ch * nwvl * NLEV);
+            z.spec_up = m.take<double>(ch * nwvl * NLEV);
+        },
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) {
+            return diag_fluxes(s, a, q, z.spec_dn, z.spec_up, z.Ed, z.Eu, z.dE);
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            const size_t nspec = (size_t)n * nwvl * NLEV;
+            if (E_down_spec) CU(cudaMemcpyAsync(E_down_spec + r * nwvl * NLEV, z.spec_dn, nspec * D, cudaMemcpyDeviceToHost, q));
+            if (E_up_spec) CU(cudaMemcpyAsync(E_up_spec + r * nwvl * NLEV, z.spec_up, nspec * D, cudaMemcpyDeviceToHost, q));
+            if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Ed, n * NLEV * D, cudaMemcpyDeviceToHost, q));
+            if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Eu, n * NLEV * D, cudaMemcpyDeviceToHost, q));
+            if (dE) CU(cudaMemcpyAsync(dE + r * NLAY, z.dE, n * NLAY * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
 }
 
-// Radiative kernels: the same chunks, streams and prep as rcm_diagnose_fluxes; rcm_jac_rt_kernel per (column, wavelength),
-// rcm_jac_sum_kernel for the sum over the wavelengths.
+// Radiative kernels: rcm_jac_rt_kernel per (column, wavelength), rcm_jac_sum_kernel for the sum over the wavelengths.
 int rcm_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* K_spec, double* K) {
     if (!s) return RCM_ERR_ARG;
     DiagScale sc{};
-    int st = diag_check(s, "rcm_radiative_kernels", col0, ncol, vmr_scale, sc);
+    const int st = diag_check(s, "rcm_radiative_kernels", col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, "rcm_radiative_kernels: needs H2O among the active species");
-    CU(cudaSetDevice(s->device));
-    st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    const int nwvl = s->dc.nwvl, na = s->nactive;
-    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
-    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], K [ch][82], K_spec [ch][nwvl][82], then the tile blocks
-    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + JAC_NK) + ch * nwvl * JAC_NK;
-    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
-    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
-    const int grid_max = rcm_jac_ctas_per_sm() * nsm_of(s);
-    struct Pending { cudaStream_t q; size_t r; int n; const double *Ks, *K; } pend{};
-    auto download = [&](const Pending& c) -> int {
-        if (K_spec) CU(cudaMemcpyAsync(K_spec + c.r * nwvl * JAC_NK, c.Ks, (size_t)c.n * nwvl * JAC_NK * D, cudaMemcpyDeviceToHost, c.q));
-        if (K) CU(cudaMemcpyAsync(K + c.r * JAC_NK, c.K, (size_t)c.n * JAC_NK * D, cudaMemcpyDeviceToHost, c.q));
-        return RCM_OK;
+    const int nwvl = s->dc.nwvl;
+    constexpr size_t D = sizeof(double);
+    struct Set {
+        DiagState state;
+        double *K, *K_spec;
     };
-    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
-        const int n = std::min((int)ch, col0 + ncol - c0);
-        const size_t r = (size_t)(c0 - col0);
-        cudaStream_t q = s->dg_stream[k % 2];
-        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
-        double* dT = p; p += ch * NLAY;
-        double* dTprev = p; p += ch * NLAY;
-        double* dvmr = p; p += ch * na * NLAY;
-        double* dstat = p; p += ch;
-        double* dK = p; p += ch * JAC_NK;
-        double* dKs = p;
-        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
-        SplitArgs a;
-        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, vmr_scale ? &sc : nullptr, a)) != RCM_OK) return st;
-        JacArgs g{};
-        g.ncol = n;
-        g.ntiles = a.ntiles;
-        g.nsplit = a.nsplit;
-        g.ipu = a.ipu;
-        g.nitem = a.nitem;
-        g.nunits = a.nunits;
-        g.clampk = s->clampk;
-        g.tau_clamp = s->tau_clamp;
-        g.T_floor = s->T_floor;
-        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
-        g.coef = s->d_coef3;
-        g.planck_c = s->d_planck_c;
-        g.planck_k = s->d_planck_k;
-        g.exp_tab = s->d_exp_tab;
-        g.tile = dtile;
-        g.T = dT;
-        g.Ts = s->d_Ts + c0;
-        g.K_spec = dKs;
-        g.K = dK;
-        CU(rcm_launch_jac_rt(g, std::min(g.nunits, grid_max), q));
-        CU(rcm_launch_jac_sum(g, q));
-        s->launches += 2;
-        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
-        pend = {q, r, n, dKs, dK};
-    }
-    if ((st = download(pend)) != RCM_OK) return st;
-    return diag_end(s);
+    return diag_chunks<Set>(
+        s, col0, ncol, vmr_scale ? &sc : nullptr,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // K [ch][82], K_spec [ch][nwvl][82]
+            z.K = m.take<double>(ch * JAC_NK);
+            z.K_spec = m.take<double>(ch * nwvl * JAC_NK);
+        },
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) -> int {
+            JacArgs g = unit_args<JacArgs>(a);
+            g.T_floor = a.T_floor;
+            g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+            g.T = a.Tlayer;
+            g.Ts = a.Tsurf;
+            g.K_spec = z.K_spec;
+            g.K = z.K;
+            CU(rcm_launch_jac_rt(g, std::min(g.nunits, rcm_jac_ctas_per_sm() * nsm_of(s)), q));
+            CU(rcm_launch_jac_sum(g, q));
+            s->launches += 2;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (K_spec) CU(cudaMemcpyAsync(K_spec + r * nwvl * JAC_NK, z.K_spec, (size_t)n * nwvl * JAC_NK * D, cudaMemcpyDeviceToHost, q));
+            if (K) CU(cudaMemcpyAsync(K + r * JAC_NK, z.K, (size_t)n * JAC_NK * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
 }
 
-// Flux Jacobians: the same chunks, streams and prep as rcm_diagnose_fluxes; rcm_fjac_kernel sums over the wavelengths
-// itself, one warp per column.
+// Flux Jacobians: rcm_fjac_kernel sums over the wavelengths itself, one warp per column.
 int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac) {
     if (!s) return RCM_ERR_ARG;
     DiagScale sc{};
-    int st = diag_check(s, "rcm_flux_jacobian", col0, ncol, vmr_scale, sc);
+    const int st = diag_check(s, "rcm_flux_jacobian", col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, "rcm_flux_jacobian: needs H2O among the active species");
-    CU(cudaSetDevice(s->device));
-    st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    const int na = s->nactive;
-    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
-    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], J [ch][2][21][41], dE_jac [ch][20][41], then the tile blocks
-    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + FJAC_NJ + FJAC_NH);
-    const size_t tile_off = (n_dbl * D + 255) / 256 * 256, set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
-    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
-    struct Pending { cudaStream_t q; size_t r; int n; const double *J, *H; } pend{};
-    auto download = [&](const Pending& c) -> int {
-        if (J) CU(cudaMemcpyAsync(J + c.r * FJAC_NJ, c.J, (size_t)c.n * FJAC_NJ * D, cudaMemcpyDeviceToHost, c.q));
-        if (dE_jac) CU(cudaMemcpyAsync(dE_jac + c.r * FJAC_NH, c.H, (size_t)c.n * FJAC_NH * D, cudaMemcpyDeviceToHost, c.q));
-        return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    struct Set {
+        DiagState state;
+        double *J, *H;
     };
-    for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
-        const int n = std::min((int)ch, col0 + ncol - c0);
-        const size_t r = (size_t)(c0 - col0);
-        cudaStream_t q = s->dg_stream[k % 2];
-        double* p = reinterpret_cast<double*>(s->d_diagnose + (k % 2) * set_bytes);
-        double* dT = p; p += ch * NLAY;
-        double* dTprev = p; p += ch * NLAY;
-        double* dvmr = p; p += ch * na * NLAY;
-        double* dstat = p; p += ch;
-        double* dJ = p; p += ch * FJAC_NJ;
-        double* dH = p;
-        unsigned char* dtile = s->d_diagnose + (k % 2) * set_bytes + tile_off;
-        SplitArgs a;
-        if ((st = diag_prep(s, q, c0, n, dT, dTprev, dvmr, dstat, dtile, vmr_scale ? &sc : nullptr, a)) != RCM_OK) return st;
-        FjacArgs g{};
-        g.ncol = n;
-        g.clampk = s->clampk;
-        g.tau_clamp = s->tau_clamp;
-        g.T_floor = s->T_floor;
-        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
-        g.coef = s->d_coef3;
-        g.planck_c = s->d_planck_c;
-        g.planck_k = s->d_planck_k;
-        g.exp_tab = s->d_exp_tab;
-        g.tile = dtile;
-        g.T = dT;
-        g.Ts = s->d_Ts + c0;
-        g.J = dJ;
-        g.dE_jac = dH;
-        CU(rcm_launch_fjac(g, q));
-        s->launches += 1;
-        if (k > 0 && (st = download(pend)) != RCM_OK) return st;
-        pend = {q, r, n, dJ, dH};
-    }
-    if ((st = download(pend)) != RCM_OK) return st;
-    return diag_end(s);
+    return diag_chunks<Set>(
+        s, col0, ncol, vmr_scale ? &sc : nullptr,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // J [ch][2][21][41], dE_jac [ch][20][41]
+            z.J = m.take<double>(ch * FJAC_NJ);
+            z.H = m.take<double>(ch * FJAC_NH);
+        },
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) { return flux_jacobian(s, a, q, a.Tlayer, z.J, z.H); },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (J) CU(cudaMemcpyAsync(J + r * FJAC_NJ, z.J, (size_t)n * FJAC_NJ * D, cudaMemcpyDeviceToHost, q));
+            if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * FJAC_NH, z.H, (size_t)n * FJAC_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
 }
 
-// Stratosphere-adjusted forcing: the chunks, streams, state copies and prep of the calls above.  Per chunk a base evaluation
-// (unscaled), the VMR scaling, then Newton iterations: retemper, evaluation (rcm_diag_rt_kernel + rcm_diag_sum_kernel),
-// check; while columns are active, the flux Jacobian (rcm_fjac_kernel) and the Newton step.  The host reads a chunk's active
-// count after every check.  The chunks of the two streams take turns: one chunk's kernels run while the host waits for the
-// other's count.
+// Stratosphere-adjusted forcing: the scratch sets, streams, state copies and prep of the calls above.  Per chunk a base
+// evaluation (unscaled), the VMR scaling, then Newton iterations: retemper, evaluation (rcm_diag_rt_kernel +
+// rcm_diag_sum_kernel), check; while columns are active, the flux Jacobian (rcm_fjac_kernel) and the Newton step.  The host
+// reads a chunk's active count after every check.  The chunks of the two streams take turns: one chunk's kernels run while
+// the host waits for the other's count.
 int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol, int max_iter,
                          double* F, double* dT_adj, double* E_down, double* E_up, int* iters) {
     if (!s) return RCM_ERR_ARG;
@@ -1759,88 +1777,45 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
             return fail(s, RCM_ERR_ARG, fn + ": ntrop[" + std::to_string(c) + "] = " + std::to_string(ntrop[c]) + " outside [0, 19]");
     if (!std::isfinite(tol) || !(tol > 0.0)) return fail(s, RCM_ERR_ARG, fn + ": tol must be finite and > 0");
     if (max_iter < 1) return fail(s, RCM_ERR_ARG, fn + ": max_iter must be >= 1");
-    CU(cudaSetDevice(s->device));
-    st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
-    const int nwvl = s->dc.nwvl, na = s->nactive, nsm = nsm_of(s);
+    const int nwvl = s->dc.nwvl;
     const bool first = (s->step_index == 0);
-    const size_t ch = (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16), D = sizeof(double);
-    // scratch: T, Tprev [ch][20], VMRs [ch][5][20], dTstat [ch], T_tau, T + dT, dT [ch][20], E_down, E_up [ch][21] and
-    // dE [ch][20] of the base and of the current iterate, F [ch][4], the output E_down, E_up [ch][21], J [ch][2][21][41],
-    // dE_jac [ch][20][41], spectral [2][ch][nwvl][21]; ntrop, iters [ch] and the active count; then the tile blocks
-    const size_t n_dbl = ch * (2 * NLAY + (size_t)na * NLAY + 1 + 3 * NLAY + 2 * (2 * NLEV + NLAY) + 4 + 2 * NLEV + FJAC_NJ + FJAC_NH) +
-                         2 * ch * nwvl * NLEV;
-    const size_t n_int = 2 * ch + 1;
-    const size_t tile_off = (n_dbl * D + n_int * sizeof(int) + 255) / 256 * 256,
-                 set_bytes = (tile_off + ch / 16 * rcm_split_tile_bytes() + 255) / 256 * 256;
-    if ((st = diag_begin(s, set_bytes)) != RCM_OK) return st;
+    const size_t ch = diag_chunk(ncol), D = sizeof(double);
     struct Slot {
         cudaStream_t q;
         int c0 = 0, n = 0, iter = 0;
         bool live = false;
-        double *T, *Tprev, *vmr, *stat, *Ttau, *Tp, *dT, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *spec_dn, *spec_up;
+        DiagState state;
+        double *Ttau, *Tp, *dT, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *spec_dn, *spec_up;
         int *ntrop, *iters, *count;
-        unsigned char* tile;
         SplitArgs a;
     } slot[2];
-    for (int k = 0; k < 2; ++k) {
-        Slot& z = slot[k];
-        z.q = s->dg_stream[k];
-        double* p = reinterpret_cast<double*>(s->d_diagnose + k * set_bytes);
-        z.T = p; p += ch * NLAY;
-        z.Tprev = p; p += ch * NLAY;
-        z.vmr = p; p += ch * na * NLAY;
-        z.stat = p; p += ch;
-        z.Ttau = p; p += ch * NLAY;
-        z.Tp = p; p += ch * NLAY;
-        z.dT = p; p += ch * NLAY;
-        z.Ed0 = p; p += ch * NLEV;
-        z.Eu0 = p; p += ch * NLEV;
-        z.dE0 = p; p += ch * NLAY;
-        z.Ed = p; p += ch * NLEV;
-        z.Eu = p; p += ch * NLEV;
-        z.dE = p; p += ch * NLAY;
-        z.F = p; p += ch * 4;
-        z.Edo = p; p += ch * NLEV;
-        z.Euo = p; p += ch * NLEV;
-        z.J = p; p += ch * FJAC_NJ;
-        z.H = p; p += ch * FJAC_NH;
-        z.spec_dn = p; p += ch * nwvl * NLEV;
-        z.spec_up = p; p += ch * nwvl * NLEV;
-        int* ip = reinterpret_cast<int*>(p);
-        z.ntrop = ip; ip += ch;
-        z.iters = ip; ip += ch;
-        z.count = ip;
-        z.tile = s->d_diagnose + k * set_bytes + tile_off;
-    }
-    // broadband fluxes of the chunk's tile blocks into Ed, Eu, dE (rcm_diagnose_fluxes' kernels)
-    auto evaluate = [&](Slot& z, double* Ed, double* Eu, double* dE) -> int {
-        DiagArgs g{};
-        g.ncol = z.n;
-        g.ntiles = z.a.ntiles;
-        g.nsplit = z.a.nsplit;
-        g.ipu = z.a.ipu;
-        g.nitem = z.a.nitem;
-        g.nunits = z.a.nunits;
-        g.clampk = s->clampk;
-        g.tau_clamp = s->tau_clamp;
-        g.coef = s->d_coef3;
-        g.planck_c = s->d_planck_c;
-        g.planck_k = s->d_planck_k;
-        g.exp_tab = s->d_exp_tab;
-        g.tile = z.tile;
-        g.spec_dn = z.spec_dn;
-        g.spec_up = z.spec_up;
-        g.E_down = Ed;
-        g.E_up = Eu;
-        g.dE = dE;
-        g.solar_col = z.a.solar_col;
-        CU(rcm_launch_diag_rt(g, std::min(g.nunits, 3 * nsm), z.q));
-        CU(rcm_launch_diag_sum(g, z.q));
-        s->launches += 2;
-        return RCM_OK;
-    };
+    // T_tau, T + dT, dT [ch][20], E_down, E_up [ch][21] and dE [ch][20] of the base and of the current iterate, F [ch][4], the
+    // output E_down, E_up [ch][21], J [ch][2][21][41], dE_jac [ch][20][41], spectral [2][ch][nwvl][21]; ntrop, iters [ch] and
+    // the active count
+    st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
+        z.Ttau = m.take<double>(ch * NLAY);
+        z.Tp = m.take<double>(ch * NLAY);
+        z.dT = m.take<double>(ch * NLAY);
+        z.Ed0 = m.take<double>(ch * NLEV);
+        z.Eu0 = m.take<double>(ch * NLEV);
+        z.dE0 = m.take<double>(ch * NLAY);
+        z.Ed = m.take<double>(ch * NLEV);
+        z.Eu = m.take<double>(ch * NLEV);
+        z.dE = m.take<double>(ch * NLAY);
+        z.F = m.take<double>(ch * 4);
+        z.Edo = m.take<double>(ch * NLEV);
+        z.Euo = m.take<double>(ch * NLEV);
+        z.J = m.take<double>(ch * FJAC_NJ);
+        z.H = m.take<double>(ch * FJAC_NH);
+        z.spec_dn = m.take<double>(ch * nwvl * NLEV);
+        z.spec_up = m.take<double>(ch * nwvl * NLEV);
+        z.ntrop = m.take<int>(ch);
+        z.iters = m.take<int>(ch);
+        z.count = m.take<int>(1);
+    });
+    if (st != RCM_OK) return st;
+    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
+    for (int k = 0; k < 2; ++k) slot[k].q = s->dg_stream[k];
     auto fdh_args = [&](const Slot& z) {
         FdhArgs f{};
         f.ncol = z.n;
@@ -1848,9 +1823,9 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
         f.max_iter = max_iter;
         f.tol = tol;
         f.T_floor = s->T_floor;
-        f.tile = z.tile;
-        f.Tb = z.T;
-        f.Ttau = first ? z.Ttau : z.T;
+        f.tile = z.state.tile;
+        f.Tb = z.state.T;
+        f.Ttau = first ? z.Ttau : z.state.T;
         f.Tp = z.Tp;
         f.dT = z.dT;
         f.ntrop = z.ntrop;
@@ -1872,31 +1847,17 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
     auto check = [&](Slot& z, int k) -> int {
         const FdhArgs f = fdh_args(z);
         CU(rcm_launch_fdh_retemper(f, z.q));
-        if ((st = evaluate(z, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
+        if ((st = diag_fluxes(s, z.a, z.q, z.spec_dn, z.spec_up, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
         CU(rcm_launch_fdh_check(f, z.q));
         CU(cudaMemcpyAsync(s->h_fdh_count + k, z.count, sizeof(int), cudaMemcpyDeviceToHost, z.q));
         s->launches += 2;
         return RCM_OK;
     };
+    // the flux Jacobian at T + dT and the Newton step
     auto newton = [&](Slot& z) -> int {
-        FjacArgs g{};
-        g.ncol = z.n;
-        g.clampk = s->clampk;
-        g.tau_clamp = s->tau_clamp;
-        g.T_floor = s->T_floor;
-        g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
-        g.coef = s->d_coef3;
-        g.planck_c = s->d_planck_c;
-        g.planck_k = s->d_planck_k;
-        g.exp_tab = s->d_exp_tab;
-        g.tile = z.tile;
-        g.T = z.Tp;
-        g.Ts = s->d_Ts + z.c0;
-        g.J = z.J;
-        g.dE_jac = z.H;
-        CU(rcm_launch_fjac(g, z.q));
+        if ((st = flux_jacobian(s, z.a, z.q, z.Tp, z.J, z.H)) != RCM_OK) return st;
         CU(rcm_launch_fdh_newton(fdh_args(z), z.q));
-        s->launches += 2;
+        s->launches += 1;
         return RCM_OK;
     };
     // the chunk [c0, c0 + n): T_tau, prep, base evaluation, scaling, iterate 0
@@ -1907,10 +1868,10 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
         z.live = true;
         if (first) CU(cudaMemcpyAsync(z.Ttau, s->d_T + (size_t)c0 * NLAY, z.n * NLAY * D, cudaMemcpyDeviceToDevice, z.q));
         CU(cudaMemcpyAsync(z.ntrop, ntrop + (c0 - col0), z.n * sizeof(int), cudaMemcpyHostToDevice, z.q));
-        if ((st = diag_prep(s, z.q, c0, z.n, z.T, z.Tprev, z.vmr, z.stat, z.tile, nullptr, z.a)) != RCM_OK) return st;
-        if ((st = evaluate(z, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
+        if ((st = diag_prep(s, z.q, c0, z.n, z.state, nullptr, z.a)) != RCM_OK) return st;
+        if ((st = diag_fluxes(s, z.a, z.q, z.spec_dn, z.spec_up, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
         if (vmr_scale) {
-            CU(rcm_launch_diag_scale(z.tile, z.a.ntiles, sc, z.q));
+            CU(rcm_launch_diag_scale(z.state.tile, z.a.ntiles, sc, z.q));
             s->launches += 1;
         }
         return check(z, k);

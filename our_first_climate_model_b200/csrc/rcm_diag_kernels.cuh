@@ -28,7 +28,7 @@ __global__ void __launch_bounds__(256) rcm_diag_scale_kernel(unsigned char* tile
 
 template <bool CLAMPK>
 __global__ void __launch_bounds__(DIAG_NT, 3) rcm_diag_rt_kernel(const DiagArgs a) {
-    constexpr int C = SPLIT_C, NT = DIAG_NT, G = SPLIT_G, NACT = 5;
+    constexpr int C = SPLIT_C, NT = DIAG_NT, G = SPLIT_G;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* const s_exp = reinterpret_cast<double*>(smem_raw);
     double* const tb = reinterpret_cast<double*>(smem_raw + (size_t)EXP_TAB * EXP_REP * 8);
@@ -39,42 +39,15 @@ __global__ void __launch_bounds__(DIAG_NT, 3) rcm_diag_rt_kernel(const DiagArgs 
     const int h = tid & 1, q = tid >> 1, c = q % C, g = q / C;  // as the unit kernel: one warp per wavelength group
     const int sb = tbd(h * HALF, c), sbi = tbix(h * HALF, c);
     const int nwvl = cst.nwvl;
-    for (int i = tid; i < EXP_TAB * EXP_REP; i += NT) s_exp[i] = a.exp_tab[i / EXP_REP];
+    load_exp_tab(s_exp, a.exp_tab, tid, NT);
     const unsigned tab_lane = (unsigned)__cvta_generic_to_shared(s_exp + (lane & (EXP_REP - 1)));
     const int tau_clamp_hi = __double2hiint(a.tau_clamp);
-
-    // K1 from the table in global memory: the expression of the unit kernel's tau_from (rcm_split_unit_loop.inc, "K1 for
-    // owned layer j"), evaluated on the same numbers - three FMAs per species on {c0 + cP*dP, cT, cPT} and dT, dT*dP
-    auto tau_from = [&](int j, const double2* cf, double cl) -> double {
-        const int r = h * HALF + j;
-        const double dT = tb[TB_DELT + sb + j * C], dTdP = tb[TB_DTDP + sb + j * C];
-        double cc[16];
-#pragma unroll
-        for (int q2 = 0; q2 < 8; ++q2) {
-            const double2 v = cf[q2];
-            cc[2 * q2] = v.x;
-            cc[2 * q2 + 1] = v.y;
-        }
-        double acc = 0.0;
-#pragma unroll
-        for (int k = 0; k < NACT; ++k) {
-            double v = fma(cc[3 * k + 1], dT, cc[3 * k]);
-            v = fma(cc[3 * k + 2], dTdP, v);
-            acc = fma(v, tb[TB_VMR + k * TBD_LEN + sb + j * C], acc);
-        }
-        acc = acc * cst.numDens[r];
-        return fma(cst.cloud_w[r], cl, acc);
-    };
 
     for (int unit = blockIdx.x; unit < a.nunits; unit += gridDim.x) {
         const int tile = unit / a.nsplit, split = unit - tile * a.nsplit;
         const int col0 = tile * C, ncl = min(C, a.ncol - col0);
         __syncthreads();  // the previous unit is done with the tile block
-        {
-            const uint4* src = reinterpret_cast<const uint4*>(a.tile + (size_t)tile * TILE_BYTES);
-            uint4* dst = reinterpret_cast<uint4*>(tb);
-            for (int i = tid; i < TILE_BYTES / 16; i += NT) dst[i] = src[i];
-        }
+        load_tile(tb, a.tile + (size_t)tile * TILE_BYTES, tid, NT);
         __syncthreads();
         const int item0 = split * a.ipu, item1 = min(item0 + a.ipu, a.nitem);
 #pragma unroll 1
@@ -89,15 +62,16 @@ __global__ void __launch_bounds__(DIAG_NT, 3) rcm_diag_rt_kernel(const DiagArgs 
 #pragma unroll
             for (int j = 0; j < HALF; ++j) {
                 const int cell = cst.ipcell[h * HALF + j] + tbi[TBI_IT + sbi + j * C];
-                const double v = tau_from(j, reinterpret_cast<const double2*>(a.coef) + (size_t)(cell * nwvl + w) * 8, cl);
+                const double v = tau_k1(tb, sb + j * C, h * HALF + j,
+                                        reinterpret_cast<const double2*>(a.coef) + (size_t)(cell * nwvl + w) * 8, cl);
                 tau[j] = fmax(CLAMPK ? v : clamp_hi(v, tau_clamp_hi), TAU_FLOOR);
             }
             // K2 (main.cpp:188-191)
             const double pc = __ldg(a.planck_c + w);
             const double pk = real ? __ldg(a.planck_k + w) : 0.0;
 #pragma unroll
-            for (int j = 0; j < HALF; ++j) Bo[j] = div_fast(pk, exp_scaled<false>(pc, tb[TB_INVT + sb + j * C], tab_lane) - 1.0);
-            const double Bs = div_fast(pk, exp_scaled<false>(pc, tb[TB_INVTS + c], tab_lane) - 1.0);
+            for (int j = 0; j < HALF; ++j) Bo[j] = planck_b(pc, pk, tb[TB_INVT + sb + j * C], tab_lane);
+            const double Bs = planck_b(pc, pk, tb[TB_INVTS + c], tab_lane);
             sweep_item<CLAMPK>(tau, Bo, Bs, h, tab_lane, E1, E2, Eu20);
             // the pair's 42 values in level order: E_down[0..20], then E_up[0..20] (rows of the unit kernel's K4)
             double* o = s_out + (size_t)(g * C + c) * 2 * NLEV;

@@ -43,7 +43,7 @@ __global__ void __launch_bounds__(FJAC_NT, FJAC_CTAS) rcm_fjac_kernel(const Fjac
     double* const s_exp = reinterpret_cast<double*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
     FjacWarp& s = reinterpret_cast<FjacWarp*>(smem_raw + (size_t)EXP_TAB * EXP_REP * 8)[tid >> 5];
-    for (int i = tid; i < EXP_TAB * EXP_REP; i += FJAC_NT) s_exp[i] = a.exp_tab[i / EXP_REP];
+    load_exp_tab(s_exp, a.exp_tab, tid, FJAC_NT);
     __syncthreads();
     const int col = blockIdx.x * FJAC_WARPS + (tid >> 5);
     if (col >= a.ncol) return;  // (whole warps)
@@ -75,7 +75,7 @@ __global__ void __launch_bounds__(FJAC_NT, FJAC_CTAS) rcm_fjac_kernel(const Fjac
 
 #pragma unroll 1
     for (int w = 0; w < nwvl; ++w) {
-        // K1 as rcm_jac_rt_kernel's tau_from, and the chain-rule factors of its layer
+        // K1: tau_k1's expression (a copy: the call changes this kernel's SASS), and the chain-rule factors of its layer
         double c[16];
 #pragma unroll
         for (int q2 = 0; q2 < 8; ++q2) {
@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(FJAC_NT, FJAC_CTAS) rcm_fjac_kernel(const Fjac
         const double nd = (tau == tv) ? cst.numDens[r] : 0.0;
         // K2 (main.cpp:188-191) and dB/dT = B (1 + B/k) (c/T) / T for B = k / (exp(c/T) - 1)
         const double pc = __ldg(a.planck_c + w), pk = __ldg(a.planck_k + w);
-        const double B = div_fast(pk, exp_scaled<false>(pc, invT, tab_lane) - 1.0);
+        const double B = planck_b(pc, pk, invT, tab_lane);
         const double dB = (Tsrc > a.T_floor) ? B * (1.0 + B / pk) * (pc / Tsrc) / Tsrc : 0.0;
         if (lane < NLAY) {
             s.B[lane] = B;

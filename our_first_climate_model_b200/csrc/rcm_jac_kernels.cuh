@@ -129,7 +129,7 @@ __global__ void __launch_bounds__(JAC_NT, JAC_CTAS) rcm_jac_rt_kernel(const JacA
     const int h = tid & 1, q = tid >> 1, c = q % C, g = q / C;  // as the unit kernel: one warp per wavelength group
     const int sb = tbd(h * HALF, c), sbi = tbix(h * HALF, c);
     const int nwvl = cst.nwvl;
-    for (int i = tid; i < EXP_TAB * EXP_REP; i += NT) s_exp[i] = a.exp_tab[i / EXP_REP];
+    load_exp_tab(s_exp, a.exp_tab, tid, NT);
     const unsigned tab_lane = (unsigned)__cvta_generic_to_shared(s_exp + (lane & (EXP_REP - 1)));
     const int tau_clamp_hi = __double2hiint(a.tau_clamp);
 
@@ -145,33 +145,13 @@ __global__ void __launch_bounds__(JAC_NT, JAC_CTAS) rcm_jac_rt_kernel(const JacA
             cc[2 * q2 + 1] = v.y;
         }
     };
-    // K1 as rcm_diag_rt_kernel's tau_from (the unit kernel's expression on the same numbers)
-    auto tau_from = [&](int j, const double2* cf, double cl) -> double {
-        const int r = h * HALF + j;
-        const double dT = tb[TB_DELT + sb + j * C], dTdP = tb[TB_DTDP + sb + j * C];
-        double cc[16];
-        load_row(cf, cc);
-        double acc = 0.0;
-#pragma unroll
-        for (int k = 0; k < NACT; ++k) {
-            double v = fma(cc[3 * k + 1], dT, cc[3 * k]);
-            v = fma(cc[3 * k + 2], dTdP, v);
-            acc = fma(v, tb[TB_VMR + k * TBD_LEN + sb + j * C], acc);
-        }
-        acc = acc * cst.numDens[r];
-        return fma(cst.cloud_w[r], cl, acc);
-    };
 
     for (int unit = blockIdx.x; unit < a.nunits; unit += gridDim.x) {
         const int tile = unit / a.nsplit, split = unit - tile * a.nsplit;
         const int col0 = tile * C, ncl = min(C, a.ncol - col0);
         const int col = col0 + (c < ncl ? c : 0);  // padding columns of the last tile repeat its first column (prep)
         __syncthreads();  // the previous unit is done with the tile block
-        {
-            const uint4* src = reinterpret_cast<const uint4*>(a.tile + (size_t)tile * TILE_BYTES);
-            uint4* dst = reinterpret_cast<uint4*>(tb);
-            for (int i = tid; i < TILE_BYTES / 16; i += NT) dst[i] = src[i];
-        }
+        load_tile(tb, a.tile + (size_t)tile * TILE_BYTES, tid, NT);
         __syncthreads();
         const int item0 = split * a.ipu, item1 = min(item0 + a.ipu, a.nitem);
 #pragma unroll 1
@@ -184,7 +164,7 @@ __global__ void __launch_bounds__(JAC_NT, JAC_CTAS) rcm_jac_rt_kernel(const JacA
             const double cl = tb[TB_CLOUD + c];
 #pragma unroll
             for (int j = 0; j < HALF; ++j) {
-                const double v = tau_from(j, row_of(j, w), cl);
+                const double v = tau_k1(tb, sb + j * C, h * HALF + j, row_of(j, w), cl);
                 tau[j] = fmax(CLAMPK ? v : clamp_hi(v, tau_clamp_hi), TAU_FLOOR);
                 live |= (tau[j] == v ? 1u : 0u) << j;
             }
@@ -192,8 +172,8 @@ __global__ void __launch_bounds__(JAC_NT, JAC_CTAS) rcm_jac_rt_kernel(const JacA
             const double pc = __ldg(a.planck_c + w);
             const double pk = real ? __ldg(a.planck_k + w) : 0.0;
 #pragma unroll
-            for (int j = 0; j < HALF; ++j) Bo[j] = div_fast(pk, exp_scaled<false>(pc, tb[TB_INVT + sb + j * C], tab_lane) - 1.0);
-            const double Bs = div_fast(pk, exp_scaled<false>(pc, tb[TB_INVTS + c], tab_lane) - 1.0);
+            for (int j = 0; j < HALF; ++j) Bo[j] = planck_b(pc, pk, tb[TB_INVT + sb + j * C], tab_lane);
+            const double Bs = planck_b(pc, pk, tb[TB_INVTS + c], tab_lane);
             double aB[HALF], aT[HALF], bB[HALF], bT[HALF], aS = 0.0;
 #pragma unroll
             for (int j = 0; j < HALF; ++j) aB[j] = aT[j] = bB[j] = bT[j] = 0.0;

@@ -331,6 +331,53 @@ __device__ __forceinline__ void mbar_wait(unsigned mbar, unsigned phase) {
 }
 
 // ------------------------------------------------------------------------------------------
+// K1, K2 and the shared-memory fills of the unit kernels, also used by the diagnostic kernels (rcm_diag_kernels.cuh,
+// rcm_jac_kernels.cuh): one definition, so that every kernel evaluates the same expression on the same numbers, bit for bit.
+// ------------------------------------------------------------------------------------------
+// K1 for the layer of tile-block row r whose doubles start at offset s (tbd(r, column)), from the row at cf: the bilinear
+// (p, T) interpolation of repwvl_thermal.cpp:235-246,
+//   x = c0 + cT*dT + cP*dP + cPT*dT*dP,   tau = numDens * sum_k x_k * vmr_k,
+// contracted to three FMAs per species on {c0 + cP*dP, cT, cPT} and dT, dT*dP (17 instead of 42 FP64 instructions per
+// layer and wavelength; within a few ulp of the reference's operation order - the bit-exact form is rcm_build_tau's).
+__device__ __forceinline__ double tau_k1(const double* tb, int s, int r, const double2* cf, double cl) {
+    const double dT = tb[TB_DELT + s], dTdP = tb[TB_DTDP + s];
+    double c[16];
+#pragma unroll
+    for (int q2 = 0; q2 < 8; ++q2) {
+        const double2 v = cf[q2];
+        c[2 * q2] = v.x;
+        c[2 * q2 + 1] = v.y;
+    }
+    double acc = 0.0;
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+        double v = fma(c[3 * k + 1], dT, c[3 * k]);
+        v = fma(c[3 * k + 2], dTdP, v);
+        acc = fma(v, tb[TB_VMR + k * TBD_LEN + s], acc);
+    }
+    acc = acc * cst.numDens[r];
+    return fma(cst.cloud_w[r], cl, acc);  // main.cpp:270: + cl on the cloud layer, + 0 * cl (exact) elsewhere
+}
+
+// K2: Planck source B = k_w / (exp(c_w / T) - 1) (main.cpp:188-191, wavelength-only factors from the host) at
+// invT = EXP_L2E / T
+__device__ __forceinline__ double planck_b(double pc, double pk, double invT, unsigned tab_lane) {
+    return div_fast(pk, exp_scaled<false>(pc, invT, tab_lane) - 1.0);
+}
+
+// the exp table into shared memory, EXP_REP copies of every entry side by side (exp_scaled), by the nt threads of a CTA
+__device__ __forceinline__ void load_exp_tab(double* s_exp, const double* tab, int tid, int nt) {
+    for (int i = tid; i < EXP_TAB * EXP_REP; i += nt) s_exp[i] = tab[i / EXP_REP];
+}
+
+// a tile block into shared memory, 16 bytes per copy, by the nt threads of a CTA
+__device__ __forceinline__ void load_tile(double* tb, const unsigned char* tile, int tid, int nt) {
+    const uint4* src = reinterpret_cast<const uint4*>(tile);
+    uint4* dst = reinterpret_cast<uint4*>(tb);
+    for (int i = tid; i < TILE_BYTES / 16; i += nt) dst[i] = src[i];
+}
+
+// ------------------------------------------------------------------------------------------
 // K1-K4 for (tile, split) units.  Persistent CTAs (3 per SM, 168 registers), units by atomic counter.
 // Shared memory: exp table 8 KB | four row buffers 4 x 7,680 B (after the wavelength loop: the groups' partial fluxes)
 // | tile block 23,552 B | Planck factors 2 KB | mbarrier, next unit.
