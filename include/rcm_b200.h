@@ -293,6 +293,33 @@ int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale
  * tol is not finite or not > 0, or max_iter < 1. */
 int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol,
                          int max_iter, double* F, double* dT_adj, double* E_down, double* E_up, int* iters);
+/* Diagnostic radiation call of the line-by-line path: the thermal fluxes the NEXT LBL step would compute for the columns
+ * [col0, col0 + ncol) - after its theta-sort and water-vapour feedback (none at step 0), with the grey cloud or the per-column
+ * cloud tau and solar_irr of rcm_set_column_solar - optionally with scaled species and resolved into bands of wavelengths.
+ * Changes nothing: T, Tprev, VMRs, model time, dt, fluxes, step counter, checkpoint bytes and every later step stay as they are.
+ * vmr_scale [5] (NULL = all 1): one factor per species in ASCENDING SPECIES INDEX - H2O, CO2, O3, N2O, CH4 (not the table order
+ * of rcm_set_lbl_tables).  The perturbed optical depth, defined so that all factors 1 give the step's tau bit for bit:
+ *   s_H2O = (f_H2O x h2o) / h2o_ref with h2o the VMR after the feedback, one rounded multiplication before the division;
+ *   s_O3  = (f_O3 x o3) / o3_ref, or f_O3 without o3_ref;
+ *   column-independent plane = ((f_CO2 x co2_factor) x tau_CO2 + f_CH4 x tau_CH4) + f_N2O x tau_N2O, left to right, each
+ *   operation rounded (composed only when one of these three factors is not 1; the tables' own plane otherwise).
+ * Broadband outputs (host, any may be NULL): E_down / E_up [ncol][21], dE [ncol][20] (main.cpp:337-341, the column's own
+ * solar_irr in dE[19]).  They come from the step's own kernels on copies of the state: unscaled they equal what the next
+ * rcm_advance(1) computes, bit for bit.
+ * Band outputs (host, either may be NULL): E_down_band / E_up_band [ncol][nband][21]; band b is the sum of each wavelength's own
+ * flux over [band_start[b], band_start[b + 1]) in index order, from 0.0 (a band of one wavelength is that wavelength alone).
+ * band_start [nband + 1] must satisfy 0 = b_0 < b_1 < ... < b_nband = nwvl; it is read only when a band output is wanted.
+ * Every value is a function of its column alone: ranges, chunks and shards give bit-identical rows.  The band pass runs only
+ * for band outputs, the broadband pass only for broadband outputs.  Synchronous.
+ * Device scratch of its own: two sets for chunks of ch columns (whole tiles of 16, at most 8,192; with band outputs also at most
+ * 2e9 / (nwvl x 42 x 8) rounded down to whole tiles, at least 16), each of 8 ch (141 + 42 nchunks_b + 42 nwvl_b + 42 nband_b)
+ * + 4 ch + 4 (nband + 1)_b bytes, nchunks = ceil(nwvl / 128), the _b terms only for broadband (nchunks) or band outputs;
+ * with CO2, CH4 or N2O scaled also 3 x nwvl x 20 doubles.
+ * Errors: RCM_ERR_STATE not on the line-by-line path, without columns, or with another species_mask than the default's five
+ * species; RCM_ERR_ARG for a range outside the loaded columns, a factor that is negative or not finite, and with a band output
+ * for nband < 1, a NULL band_start or one that does not rise strictly from 0 to nwvl.  Each error leaves the solver usable. */
+int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
+                            double* E_down_band, double* E_up_band, double* E_down, double* E_up, double* dE);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

@@ -419,6 +419,27 @@ class Solver:
                self._h)
         return out
 
+    def lbl_diagnose_fluxes(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, bands=None) -> dict:
+        """rcm_lbl_diagnose_fluxes: the fluxes the next line-by-line step would compute for columns [col0, col0 + ncol),
+        without changing anything.  vmr_scale [5]: factors on H2O, CO2, O3, N2O, CH4 (ascending species index; None =
+        unscaled).  bands: band_start [nband + 1], 0 = b_0 < ... < b_nband = nwvl, or None for no band outputs.
+        -> E_down, E_up [ncol, 21], dE [ncol, 20] and, with bands, E_down_band / E_up_band [ncol, nband, 21] (each band the
+        sum of its wavelengths' fluxes in index order)."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = self._vmr_scale(vmr_scale)
+        m = max(n, 0)
+        out = dict(E_down=np.zeros((m, NLEV)), E_up=np.zeros((m, NLEV)), dE=np.zeros((m, NLAY)))
+        bs, nband = None, 0
+        if bands is not None:
+            bs = np.ascontiguousarray(bands, dtype=np.int32).ravel()
+            nband = bs.size - 1
+            out["E_down_band"] = np.zeros((m, max(nband, 0), NLEV))
+            out["E_up_band"] = np.zeros((m, max(nband, 0), NLEV))
+        _check(_lib.rcm_lbl_diagnose_fluxes(self._h, C.c_int(col0), C.c_int(n), _p(sc), C.c_int(nband), _p(bs),
+                                            _p(out.get("E_down_band")), _p(out.get("E_up_band")), _p(out["E_down"]),
+                                            _p(out["E_up"]), _p(out["dE"])), self._h)
+        return out
+
     def radiative_kernels(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, spectral: bool = False) -> dict:
         """rcm_radiative_kernels: derivatives of the next step's OLR (output 0) and surface downward flux (output 1) for
         columns [col0, col0 + ncol), without changing anything.  vmr_scale as in diagnose_fluxes.

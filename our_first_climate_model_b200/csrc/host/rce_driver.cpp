@@ -11,6 +11,7 @@
 //           [--spectral-out spectrum.csv] [--kernels-out kernels.csv] [--jacobian-out jacobian.csv]
 //           [--forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
+//           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]]
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
 // --gpus N (N > 1): one process, one host thread and one solver per GPU, contiguous blocks of columns per GPU (tables
@@ -46,6 +47,13 @@
 // ensemble-mean adjustment (K), then the rows "IRF_toa,,v", "IRF_trop,,v", "SARF_toa,,v", "SARF_trop,,v" with the ensemble
 // means (W/m2) and "unconverged,,n" with the number of columns that did not converge.  Summed in column order: the file is
 // byte-identical for any --gpus N.
+//
+// --lbl-bands-out FILE (line-by-line tables only): after the run, the fluxes the next step would see
+// (rcm_lbl_diagnose_fluxes) in bands of --band-size K consecutive wavelengths (default 100; the last band is shorter),
+// unscaled and with the factors --forcing-scale (H2O, CO2, O3, N2O, CH4; default 1,2,1,1,1) - header
+// "wvl_lo_nm,wvl_hi_nm,olr,surface_down,olr_scaled,surface_down_scaled", then one row per band with its edges (the midpoint
+// bins of rcm_set_lbl_tables) and the ensemble means of its TOA upward and surface downward flux (W/m2), unscaled and scaled.
+// Summed in column order: the file is byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -108,6 +116,9 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     const int* ntrop;         // [ncol]
     double *F_out, *dTadj_out;
     int* iters_out;
+    int lbl_nband;            // > 0: --lbl-bands-out, rows [ncol][nband][4] (olr, sfc, olr scaled, sfc scaled) into B_out
+    const int* lbl_bstart;    // [nband + 1]
+    double* B_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -244,6 +255,61 @@ int write_forcing(const std::string& path, int ncol, const double* player, const
     return 0;
 }
 
+// TOA E_up and surface E_down of every (column, band) of the n columns of s, unscaled and with the factors scale:
+// out [n][nband][4] = olr, sfc, olr scaled, sfc scaled
+int diagnose_lbl_bands(rcm_solver* s, int n, int nband, const int* bstart, const double* scale, double* out) {
+    constexpr int NLEV = RCM_NLEVEL, CHUNK = 1024;
+    std::vector<double> dn((size_t)std::min(n, CHUNK) * nband * NLEV), up(dn.size());
+    for (int pass = 0; pass < 2; ++pass)
+        for (int c0 = 0; c0 < n; c0 += CHUNK) {
+            const int m = std::min(CHUNK, n - c0);
+            const int st = rcm_lbl_diagnose_fluxes(s, c0, m, pass ? scale : nullptr, nband, bstart, dn.data(), up.data(), nullptr,
+                                                   nullptr, nullptr);
+            if (st != RCM_OK) return st;
+            for (size_t c = 0; c < (size_t)m; ++c)
+                for (size_t b = 0; b < (size_t)nband; ++b) {
+                    double* o = out + (((size_t)c0 + c) * nband + b) * 4 + 2 * pass;
+                    o[0] = up[(c * nband + b) * NLEV];
+                    o[1] = dn[(c * nband + b) * NLEV + NLEV - 1];
+                }
+        }
+    return RCM_OK;
+}
+
+// band starts of K consecutive wavelengths: [nband + 1]
+std::vector<int> lbl_band_starts(int nwvl, int K) {
+    std::vector<int> b;
+    for (int w = 0; w < nwvl; w += K) b.push_back(w);
+    b.push_back(nwvl);
+    return b;
+}
+
+// ensemble means per band, summed in column order; edges as rcm_set_lbl_tables' bins
+int write_lbl_bands(const std::string& path, int ncol, const std::vector<double>& wvl, const std::vector<int>& bstart, const double* B) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    const int nwvl = (int)wvl.size(), nband = (int)bstart.size() - 1;
+    std::fprintf(f, "wvl_lo_nm,wvl_hi_nm,olr,surface_down,olr_scaled,surface_down_scaled\n");
+    for (int b = 0; b < nband; ++b) {
+        const int i = bstart[b], k = bstart[b + 1] - 1;
+        const double dl = (i > 0) ? (wvl[i] - wvl[i - 1]) : (wvl[1] - wvl[0]);
+        const double dh = (k < nwvl - 1) ? (wvl[k + 1] - wvl[k]) : (wvl[k] - wvl[k - 1]);
+        double sum[4] = {0.0, 0.0, 0.0, 0.0};
+        for (size_t c = 0; c < (size_t)ncol; ++c)
+            for (int q = 0; q < 4; ++q) sum[q] += B[(c * nband + b) * 4 + q];
+        std::fprintf(f, "%.17g,%.17g,%.17g,%.17g,%.17g,%.17g\n", wvl[i] - dl / 2.0, wvl[k] + dh / 2.0, sum[0] / ncol, sum[1] / ncol,
+                     sum[2] / ncol, sum[3] / ncol);
+    }
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
+
 void run_shard(Shard* sh, const Job* j) {
     auto fail = [&](const char* what, int st) {
         sh->err = std::string(what) + ": " + rcm_status_string(st) + (sh->s ? std::string(" - ") + rcm_last_error(sh->s) : "");
@@ -327,13 +393,17 @@ void run_shard(Shard* sh, const Job* j) {
                                   j->dTadj_out + lo * NLAY, nullptr, nullptr, j->iters_out + lo);
         if (st != RCM_OK) return fail("rcm_adjusted_forcing", st);
     }
+    if (j->lbl_nband > 0) {
+        st = diagnose_lbl_bands(sh->s, (int)n, j->lbl_nband, j->lbl_bstart, j->forcing_scale, j->B_out + lo * j->lbl_nband * 4);
+        if (st != RCM_OK) return fail("rcm_lbl_diagnose_fluxes", st);
+    }
 }
 
 }  // namespace
 
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
-        jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4";
+        jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100";
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -363,6 +433,8 @@ int main(int argc, char** argv) {
         else if (a == "--forcing-out") forcing_path = val();
         else if (a == "--forcing-scale") forcing_scale_arg = val();
         else if (a == "--trop-layers") trop_layers_arg = val();
+        else if (a == "--lbl-bands-out") bands_path = val();
+        else if (a == "--band-size") band_size_arg = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -373,7 +445,8 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "usage: rcm_rce --atm FILE (--table FILE | --lbl DIR [--co2-factor F]) [--ncol N] [--seed S] [--max-steps M] [--check-every K] "
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
                              "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE] "
-                             "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]\n");
+                             "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
+                             "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -392,8 +465,27 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rcm_rce: --forcing-out needs a repwvl table (--table): the line-by-line path has no adjusted forcing\n");
         return 1;
     }
+    if (lbl_dir.empty() && !bands_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-bands-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
     double forcing_scale[5];
-    int trop_layers = 0;
+    int trop_layers = 0, band_size = 0;
+    if (!bands_path.empty()) {  // --forcing-scale: exactly five numbers; --band-size: an integer >= 1
+        int k = 0;
+        const char* q = forcing_scale_arg.c_str();
+        for (char* e = nullptr; k < 5; ++k, q = e + 1) {
+            forcing_scale[k] = std::strtod(q, &e);
+            if (e == q || (k < 4 && *e != ',') || (k == 4 && *e != '\0')) break;
+        }
+        char* e = nullptr;
+        const long bs = std::strtol(band_size_arg.c_str(), &e, 10);
+        if (k < 5 || e == band_size_arg.c_str() || *e != '\0' || bs < 1 || bs > 1000000000L) {
+            std::fprintf(stderr, "rcm_rce: --forcing-scale needs five comma-separated factors and --band-size an integer >= 1\n");
+            return 1;
+        }
+        band_size = (int)bs;
+    }
     if (!forcing_path.empty()) {  // --forcing-scale: exactly five numbers; --trop-layers: one integer in [0, 19]
         int k = 0;
         const char* q = forcing_scale_arg.c_str();
@@ -496,10 +588,13 @@ int main(int argc, char** argv) {
         const bool forcing = !forcing_path.empty();
         std::vector<double> Ff(forcing ? n * 4 : 0), dTf(forcing ? n * NLAY : 0);
         std::vector<int> itf(forcing ? n : 0), ntrop(n, trop_layers);
+        const std::vector<int> bstart = bands_path.empty() ? std::vector<int>() : lbl_band_starts(nwvl, band_size);
+        const int nband = bands_path.empty() ? 0 : (int)bstart.size() - 1;
+        std::vector<double> B(n * nband * 4);
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
                 dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data(),
-                forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data()};
+                forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data(), nband, bstart.data(), B.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -549,6 +644,7 @@ int main(int argc, char** argv) {
             rcm_table_free(table);
             return 1;
         }
+        if (nband > 0 && write_lbl_bands(bands_path, ncol, wvl, bstart, B.data())) return 1;
         if (table) rcm_table_free(table);
         st = rcm_write_profiles(out_path.c_str(), 0, 1, ncol, plevel, T.data(), time_h.data(), ncol > 1);
         if (st != RCM_OK) return die(out_path.c_str(), st, nullptr);
@@ -565,6 +661,7 @@ int main(int argc, char** argv) {
         return 0;
     }
     std::vector<double> spec_wvl, spec_weight;  // --spectral-out: the table's wavelengths and weights
+    std::vector<double> lbl_wvl;                // --lbl-bands-out: the LBL wavelengths
     rcm_solver* s = nullptr;
     st = rcm_create(device, &p, &s);
     if (st != RCM_OK) return die("rcm_create", st, nullptr);
@@ -598,6 +695,7 @@ int main(int argc, char** argv) {
         // reference profiles of the tables = the .atm file's own column = member 0 (layer VMRs, species 0 and 2 of vmr9)
         st = rcm_set_lbl_tables(s, wvl.data(), tau5.data(), nwvl, &vmr9[0 * NLAY], &vmr9[2 * NLAY], co2_factor);
         if (st != RCM_OK) return die("rcm_set_lbl_tables", st, s);
+        lbl_wvl = wvl;
     } else {
         rcm_table* t = nullptr;
         st = rcm_table_load(table_path.c_str(), &t);
@@ -679,6 +777,14 @@ int main(int argc, char** argv) {
                                   nullptr, itf.data());
         if (st != RCM_OK) return die("rcm_adjusted_forcing", st, s);
         if (write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) return 1;
+    }
+    if (!bands_path.empty()) {
+        const std::vector<int> bstart = lbl_band_starts((int)lbl_wvl.size(), band_size);
+        const int nband = (int)bstart.size() - 1;
+        std::vector<double> B(m * nband * 4);
+        st = diagnose_lbl_bands(s, ncol, nband, bstart.data(), forcing_scale, B.data());
+        if (st != RCM_OK) return die("rcm_lbl_diagnose_fluxes", st, s);
+        if (write_lbl_bands(bands_path, ncol, lbl_wvl, bstart, B.data())) return 1;
     }
     double ts_mean = 0.0;
     for (size_t c = 0; c < m; ++c) ts_mean += Ts[c];

@@ -13,6 +13,7 @@
 
 #include "rcm_jac.cuh"
 #include "rcm_fdh.cuh"
+#include "rcm_lbl_diag.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -65,6 +66,9 @@ struct rcm_solver {
     double *d_lbl_lo = nullptr, *d_lbl_hi = nullptr, *d_lbl_tau5 = nullptr, *d_lbl_h2o_ref = nullptr,
            *d_lbl_o3_ref = nullptr, *d_sH = nullptr, *d_sO = nullptr, *d_dTstat = nullptr, *d_part = nullptr;
     size_t part_cap = 0;
+    // d_lbl_tau5 holds the step's three planes, then the raw CO2, CH4 and N2O planes (rcm_lbl_diagnose_fluxes scales them)
+    double* d_lbl_tau3s = nullptr;  // [3][nwvl][20] the step's planes with scaled species (rcm_lbl_diagnose_fluxes)
+    size_t tau3s_cap = 0;
     // split path (rcm_split_kernels.cuh)
     unsigned char* d_tile = nullptr;    // [tiles][TILE_BYTES]
     double* d_spart = nullptr;          // [tiles][nsplit][42][16]
@@ -907,7 +911,7 @@ int rcm_destroy(rcm_solver* s) {
     cudaStreamSynchronize(s->stream);
     if (g_const_owner[s->device & 63] == s) g_const_owner[s->device & 63] = nullptr;
     void* ptrs[] = {s->d_coef3, s->d_xsec_file, s->d_coef, s->d_species, s->d_planck_c, s->d_planck_k, s->d_exp_tab, s->d_T, s->d_Ts, s->d_vmr, s->d_rh,
-                    s->d_Tprev, s->d_time, s->d_lbl_lo, s->d_lbl_hi, s->d_lbl_tau5, s->d_lbl_h2o_ref, s->d_lbl_o3_ref, s->d_sH, s->d_sO,
+                    s->d_Tprev, s->d_time, s->d_lbl_lo, s->d_lbl_hi, s->d_lbl_tau5, s->d_lbl_h2o_ref, s->d_lbl_o3_ref, s->d_lbl_tau3s, s->d_sH, s->d_sO,
                     s->d_dTstat, s->d_part, s->d_Ed, s->d_Eu, s->d_dE, s->d_dt, s->d_diag, s->d_scalars, s->d_red, s->d_tau,
                     s->d_lowpos, s->d_solar_col, s->d_cloud_col, s->d_ticket, s->d_tile, s->d_spart, s->d_counter, s->d_multi, s->d_diagnose};
     for (void* q : ptrs)
@@ -1099,7 +1103,7 @@ int rcm_set_lbl_tables(rcm_solver* s, const double* wvl, const double* tau5, int
     const size_t n = (size_t)nwvl;
     CU(dalloc(s->d_lbl_lo, 4 * n));  // planes: lo, (hi in d_lbl_hi), whi, wlo, and the narrow-band flags as ints
     CU(dalloc(s->d_lbl_hi, n));
-    CU(dalloc(s->d_lbl_tau5, 3 * n * NLAY));
+    CU(dalloc(s->d_lbl_tau5, 6 * n * NLAY));
     CU(dalloc(s->d_lbl_h2o_ref, (size_t)NLAY));
     CU(dalloc(s->d_lbl_o3_ref, (size_t)NLAY));
     CU(cudaMemcpy(s->d_lbl_lo, lo.data(), n * sizeof(double), cudaMemcpyHostToDevice));
@@ -1116,12 +1120,15 @@ int rcm_set_lbl_tables(rcm_solver* s, const double* wvl, const double* tau5, int
         CU(cudaMemcpy(s->d_lbl_lo + 3 * n, ok.data(), n * sizeof(int), cudaMemcpyHostToDevice));
     }
     CU(cudaMemcpy(s->d_lbl_hi, hi.data(), n * sizeof(double), cudaMemcpyHostToDevice));
-    {   // device planes: tau_H2O, tau_O3, and the column-independent part f_CO2 * tau_CO2 + tau_CH4 + tau_N2O
+    {   // device planes: tau_H2O, tau_O3, and the column-independent part f_CO2 * tau_CO2 + tau_CH4 + tau_N2O; behind them the
+        // raw CO2, CH4, N2O planes, from which rcm_lbl_diagnose_fluxes composes that part with scaled species
         const size_t plane = n * NLAY;
-        std::vector<double> t3(3 * plane);
+        std::vector<double> t3(6 * plane);
         std::memcpy(&t3[0], tau5, plane * sizeof(double));
         std::memcpy(&t3[plane], tau5 + 2 * plane, plane * sizeof(double));
         for (size_t i = 0; i < plane; ++i) t3[2 * plane + i] = co2_factor * tau5[plane + i] + tau5[3 * plane + i] + tau5[4 * plane + i];
+        std::memcpy(&t3[3 * plane], tau5 + plane, plane * sizeof(double));
+        std::memcpy(&t3[4 * plane], tau5 + 3 * plane, 2 * plane * sizeof(double));
         CU(cudaMemcpy(s->d_lbl_tau5, t3.data(), t3.size() * sizeof(double), cudaMemcpyHostToDevice));
     }
     CU(cudaMemcpy(s->d_lbl_h2o_ref, h2o_ref, NLAY * sizeof(double), cudaMemcpyHostToDevice));
@@ -1297,19 +1304,11 @@ int rcm_radiative_transfer(rcm_solver* s, const double* tau, double* E_down, dou
     return RCM_OK;
 }
 
-static int lbl_advance(rcm_solver* s, int nsteps) {
-    if (s->h2o_slot < 0) return fail(s, RCM_ERR_STATE, "the LBL path needs H2O in species_mask");
-    int st = refresh_const(s);
-    if (st != RCM_OK) return st;
-    const size_t n = (size_t)s->ncol;
-    if (!s->d_sH || s->part_cap == 0) {
-        CU(dalloc(s->d_sH, (size_t)s->cap * NLAY));
-        CU(dalloc(s->d_sO, (size_t)s->cap * NLAY));
-        CU(dalloc(s->d_dTstat, (size_t)s->cap));
-    }
+// The LBL kernels' arguments for ncol columns: sizes, species slots and tables; the state pointers are the caller's.
+static LblArgs lbl_args(const rcm_solver* s, int ncol) {
     LblArgs a{};
-    a.ncol = s->ncol;
-    a.ntiles = (s->ncol + RCM_LBL_C - 1) / RCM_LBL_C;
+    a.ncol = ncol;
+    a.ntiles = (ncol + RCM_LBL_C - 1) / RCM_LBL_C;
     a.nwvl = s->lbl_nwvl;
     // (tile, wavelength chunk) CTAs with a FIXED chunk of 128 wavelengths (32 rounds of the 4 wavelength groups): the
     // order of the spectral sum - registers over a chunk's rounds, groups, chunks - does not depend on how many columns
@@ -1317,11 +1316,6 @@ static int lbl_advance(rcm_solver* s, int nsteps) {
     // 20,000 wavelengths are 40,192 units for the hardware scheduler to balance instead of 1,792 (4.04 rounds of 444)
     a.chunk_len = 128;
     a.nchunks = (a.nwvl + a.chunk_len - 1) / a.chunk_len;
-    const size_t need = (size_t)a.nchunks * n * 42;
-    if (need > s->part_cap) {
-        CU(dalloc(s->d_part, need));
-        s->part_cap = need;
-    }
     a.nact = s->nactive;
     a.h2o_slot = s->h2o_slot;
     a.o3_slot = -1;
@@ -1339,6 +1333,25 @@ static int lbl_advance(rcm_solver* s, int nsteps) {
     a.h2o_ref = s->d_lbl_h2o_ref;
     a.o3_ref = s->lbl_has_o3_ref ? s->d_lbl_o3_ref : nullptr;
     a.exp_tab = s->d_exp_tab;
+    return a;
+}
+
+static int lbl_advance(rcm_solver* s, int nsteps) {
+    if (s->h2o_slot < 0) return fail(s, RCM_ERR_STATE, "the LBL path needs H2O in species_mask");
+    int st = refresh_const(s);
+    if (st != RCM_OK) return st;
+    const size_t n = (size_t)s->ncol;
+    if (!s->d_sH || s->part_cap == 0) {
+        CU(dalloc(s->d_sH, (size_t)s->cap * NLAY));
+        CU(dalloc(s->d_sO, (size_t)s->cap * NLAY));
+        CU(dalloc(s->d_dTstat, (size_t)s->cap));
+    }
+    LblArgs a = lbl_args(s, s->ncol);
+    const size_t need = (size_t)a.nchunks * n * 42;
+    if (need > s->part_cap) {
+        CU(dalloc(s->d_part, need));
+        s->part_cap = need;
+    }
     a.Tlayer = s->d_T; a.Tsurf = s->d_Ts; a.vmr = s->d_vmr; a.rel_hum = s->d_rh; a.Tprev = s->d_Tprev;
     a.time_h = s->d_time; a.sH = s->d_sH; a.sO = s->d_sO; a.dTstat = s->d_dTstat; a.part = s->d_part;
     a.E_down = s->d_Ed; a.E_up = s->d_Eu; a.dE = s->d_dE; a.dt = s->d_dt;
@@ -1459,13 +1472,8 @@ constexpr int kDiagMaxChunk = 8192;
 // columns per chunk: whole tiles of 16, at most kDiagMaxChunk
 size_t diag_chunk(int ncol) { return (size_t)std::min(kDiagMaxChunk, (ncol + 15) / 16 * 16); }
 
-// the checks every call makes; the factors of vmr_scale (NULL = all 1) into sc
-int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
-    if (s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": the line-by-line path is not supported");
-    if (!s->has_table) return fail(s, RCM_ERR_STATE, fn + ": no lookup table loaded");
-    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
-    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
-    if (!use_split(s)) return fail(s, RCM_ERR_STATE, fn + ": needs the split path (RCM_OPT_PATH 0, no forced tile shape)");
+// the range [col0, col0 + ncol) inside the loaded columns; the factors of vmr_scale (NULL = all 1) into sc
+int diag_range(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
     if (col0 < 0 || ncol <= 0 || (long long)col0 + ncol > s->ncol)
         return fail(s, RCM_ERR_ARG, fn + ": columns [" + std::to_string(col0) + ", " + std::to_string((long long)col0 + ncol) +
                                         ") outside the " + std::to_string(s->ncol) + " loaded");
@@ -1475,6 +1483,16 @@ int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const d
             return fail(s, RCM_ERR_ARG, fn + ": vmr_scale[" + std::to_string(k) + "] must be finite and >= 0");
     }
     return RCM_OK;
+}
+
+// the checks every repwvl call makes, then diag_range
+int diag_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
+    if (s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": the line-by-line path is not supported");
+    if (!s->has_table) return fail(s, RCM_ERR_STATE, fn + ": no lookup table loaded");
+    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
+    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
+    if (!use_split(s)) return fail(s, RCM_ERR_STATE, fn + ": needs the split path (RCM_OPT_PATH 0, no forced tile shape)");
+    return diag_range(s, fn, col0, ncol, vmr_scale, sc);
 }
 
 // A chunk's copies of what the prep reads - T, Tprev [ch][20], VMRs [ch][5][20] - its stationarity diagnostic stat [ch]
@@ -1498,10 +1516,10 @@ struct DiagCarve {
 
 // The device, its constants, two scratch sets for chunks of ch columns and the two streams; work queued on the solver's stream
 // comes first.  A set is the state copies, what layout(m, ch, z) takes for the call's own arrays, then the tile blocks at a
-// 256-byte boundary.  The description runs once on a null base for the size of a set, then once on each set: the size and
-// the pointers cannot disagree.
+// 256-byte boundary (none without tiles: the line-by-line path has none).  The description runs once on a null base for the
+// size of a set, then once on each set: the size and the pointers cannot disagree.
 template <class Set, class Layout>
-int diag_begin(rcm_solver* s, size_t ch, Set (&set)[2], Layout layout) {
+int diag_begin(rcm_solver* s, size_t ch, Set (&set)[2], Layout layout, bool tiles = true) {
     CU(cudaSetDevice(s->device));
     const int st = refresh_const(s);
     if (st != RCM_OK) return st;
@@ -1513,7 +1531,7 @@ int diag_begin(rcm_solver* s, size_t ch, Set (&set)[2], Layout layout) {
         z.state.stat = m.take<double>(ch);
         layout(m, ch, z);
         m.off = (m.off + 255) / 256 * 256;
-        z.state.tile = m.take<unsigned char>(ch / 16 * rcm_split_tile_bytes());
+        z.state.tile = m.take<unsigned char>(tiles ? ch / 16 * rcm_split_tile_bytes() : 0);
         return (m.off + 255) / 256 * 256;
     };
     Set sized{};
@@ -1631,28 +1649,36 @@ int flux_jacobian(rcm_solver* s, const SplitArgs& a, cudaStream_t q, const doubl
     return RCM_OK;
 }
 
-// The chunks of a single-pass call.  Chunk k runs on stream k % 2 with scratch set k % 2 (chunk k + 2 reuses the set of chunk
-// k after it on the same stream): the prep (sc: VMR factors or NULL), then enqueue(z, a, q).  Its downloads, download(z, r,
-// n, q) for the output rows [r, r + n), are issued after the kernels of chunk k + 1: into pageable memory they block the host.
-template <class Set, class Layout, class Enqueue, class Download>
-int diag_chunks(rcm_solver* s, int col0, int ncol, const DiagScale* sc, Layout layout, Enqueue enqueue, Download download) {
-    const size_t ch = diag_chunk(ncol);
+// The chunks of a single-pass call, ch columns each.  Chunk k runs on stream k % 2 with scratch set k % 2 (chunk k + 2 reuses
+// the set of chunk k after it on the same stream): prep(z, c0, n, q, a) for its columns [c0, c0 + n), then enqueue(z, a, q).
+// Its downloads, download(z, r, n, q) for the output rows [r, r + n), are issued after the kernels of chunk k + 1: into
+// pageable memory they block the host.
+template <class Set, class Args, class Layout, class Prep, class Enqueue, class Download>
+int chunk_loop(rcm_solver* s, int col0, int ncol, size_t ch, bool tiles, Layout layout, Prep prep, Enqueue enqueue,
+               Download download) {
     Set set[2];
-    int st = diag_begin(s, ch, set, layout);
+    int st = diag_begin(s, ch, set, layout, tiles);
     if (st != RCM_OK) return st;
     struct { const Set* z; size_t r; int n; cudaStream_t q; } pend{};
     for (int c0 = col0, k = 0; c0 < col0 + ncol; c0 += (int)ch, ++k) {
         const int n = std::min((int)ch, col0 + ncol - c0);
         const Set& z = set[k % 2];
         cudaStream_t q = s->dg_stream[k % 2];
-        SplitArgs a;
-        if ((st = diag_prep(s, q, c0, n, z.state, sc, a)) != RCM_OK) return st;
+        Args a;
+        if ((st = prep(z, c0, n, q, a)) != RCM_OK) return st;
         if ((st = enqueue(z, a, q)) != RCM_OK) return st;
         if (k > 0 && (st = download(*pend.z, pend.r, pend.n, pend.q)) != RCM_OK) return st;
         pend = {&z, (size_t)(c0 - col0), n, q};
     }
     if ((st = download(*pend.z, pend.r, pend.n, pend.q)) != RCM_OK) return st;
     return diag_end(s);
+}
+
+// the repwvl calls: chunks of diag_chunk(ncol) columns, diag_prep (sc: VMR factors or NULL) in front of enqueue
+template <class Set, class Layout, class Enqueue, class Download>
+int diag_chunks(rcm_solver* s, int col0, int ncol, const DiagScale* sc, Layout layout, Enqueue enqueue, Download download) {
+    auto prep = [&](const Set& z, int c0, int n, cudaStream_t q, SplitArgs& a) { return diag_prep(s, q, c0, n, z.state, sc, a); };
+    return chunk_loop<Set, SplitArgs>(s, col0, ncol, diag_chunk(ncol), true, layout, prep, enqueue, download);
 }
 
 }  // namespace
@@ -1754,6 +1780,117 @@ int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale
         [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
             if (J) CU(cudaMemcpyAsync(J + r * FJAC_NJ, z.J, (size_t)n * FJAC_NJ * D, cudaMemcpyDeviceToHost, q));
             if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * FJAC_NH, z.H, (size_t)n * FJAC_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+// Line-by-line fluxes: the step's three kernels on copies of a chunk (prep, the species factors, rt, finish into scratch), and
+// for bands rcm_lbl_band_kernel + rcm_lbl_band_sum_kernel on the same prepared copies, in front of the finish (which moves T).
+constexpr double kLblStageBytes = 2e9;  // per scratch set: the band pass's staging, ch x nwvl x 42 doubles
+
+int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
+                            double* E_down_band, double* E_up_band, double* E_down, double* E_up, double* dE) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_diagnose_fluxes";
+    if (!s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": needs the line-by-line path (rcm_set_lbl_tables)");
+    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
+    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
+    DiagScale sc{};
+    int st = diag_range(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    const int nwvl = s->lbl_nwvl;
+    const bool bands = E_down_band || E_up_band, broad = E_down || E_up || dE;
+    if (bands) {
+        if (nband < 1 || !band_start) return fail(s, RCM_ERR_ARG, fn + ": band outputs need nband >= 1 and band_start");
+        for (int b = 0; b < nband; ++b)
+            if (!(band_start[b] < band_start[b + 1]))
+                return fail(s, RCM_ERR_ARG, fn + ": band_start must be strictly increasing (entry " + std::to_string(b + 1) + ")");
+        if (band_start[0] != 0 || band_start[nband] != nwvl)
+            return fail(s, RCM_ERR_ARG, fn + ": band_start must run from 0 to nwvl = " + std::to_string(nwvl));
+    }
+    if (!bands && !broad) return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    CU(cudaSetDevice(s->device));
+    // CO2, CH4 or N2O scaled: the column-independent plane composed anew, the H2O and O3 planes copied next to it
+    const bool plane3 = sc.f[1] != 1.0 || sc.f[3] != 1.0 || sc.f[4] != 1.0;
+    const size_t plane = (size_t)nwvl * NLAY;
+    if (plane3) {
+        if (s->tau3s_cap < 3 * plane) {
+            CU(dalloc(s->d_lbl_tau3s, 3 * plane));
+            s->tau3s_cap = 3 * plane;
+        }
+        CU(cudaMemcpyAsync(s->d_lbl_tau3s, s->d_lbl_tau5, 2 * plane * D, cudaMemcpyDeviceToDevice, s->stream));
+        CU(rcm_launch_lbl_plane(s->d_lbl_tau5 + 3 * plane, plane, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3],
+                                s->d_lbl_tau3s + 2 * plane, s->stream));
+        s->launches += 1;
+    }
+    size_t ch = diag_chunk(ncol);
+    if (bands) ch = std::min(ch, std::max<size_t>(16, (size_t)(kLblStageBytes / ((double)nwvl * 2 * NLEV * D)) / 16 * 16));
+    const size_t nchunks = (size_t)lbl_args(s, 0).nchunks;
+    struct Set {
+        DiagState state;
+        double *Ts, *sH, *sO, *dt, *part, *Ed, *Eu, *dE, *spec_dn, *spec_up, *band_dn, *band_up;
+        float* time;
+        int* bstart;
+    };
+    return chunk_loop<Set, LblArgs>(
+        s, col0, ncol, ch, false,
+        [&](DiagCarve& m, size_t ch, Set& z) {
+            z.Ts = m.take<double>(ch);
+            z.sH = m.take<double>(ch * NLAY);
+            z.sO = m.take<double>(ch * NLAY);
+            z.dt = m.take<double>(ch);
+            z.part = m.take<double>(broad ? nchunks * ch * 2 * NLEV : 0);
+            z.Ed = m.take<double>(ch * NLEV);
+            z.Eu = m.take<double>(ch * NLEV);
+            z.dE = m.take<double>(ch * NLAY);
+            z.spec_dn = m.take<double>(bands ? ch * nwvl * NLEV : 0);
+            z.spec_up = m.take<double>(bands ? ch * nwvl * NLEV : 0);
+            z.band_dn = m.take<double>(bands ? ch * nband * NLEV : 0);
+            z.band_up = m.take<double>(bands ? ch * nband * NLEV : 0);
+            z.time = m.take<float>(ch);
+            z.bstart = m.take<int>(bands ? nband + 1 : 0);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
+            const size_t o = (size_t)c0;
+            CU(cudaMemcpyAsync(z.state.T, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+            CU(cudaMemcpyAsync(z.state.Tprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+            CU(cudaMemcpyAsync(z.state.vmr, s->d_vmr + o * 5 * NLAY, (size_t)n * 5 * NLAY * D, cudaMemcpyDeviceToDevice, q));
+            CU(cudaMemcpyAsync(z.Ts, s->d_Ts + o, n * D, cudaMemcpyDeviceToDevice, q));
+            if (bands) CU(cudaMemcpyAsync(z.bstart, band_start, (nband + 1) * sizeof(int), cudaMemcpyHostToDevice, q));
+            a = lbl_args(s, n);
+            a.step_index = s->step_index;
+            if (plane3) a.tau3 = s->d_lbl_tau3s;
+            a.Tlayer = z.state.T; a.Tprev = z.state.Tprev; a.vmr = z.state.vmr; a.rel_hum = s->d_rh + o * NLAY;
+            a.Tsurf = z.Ts; a.time_h = z.time; a.sH = z.sH; a.sO = z.sO; a.dTstat = z.state.stat; a.part = z.part;
+            a.E_down = z.Ed; a.E_up = z.Eu; a.dE = z.dE; a.dt = z.dt; a.diag = nullptr;
+            a.solar_col = s->has_col_solar ? s->d_solar_col + o : nullptr;
+            a.cloud_col = s->has_col_cloud ? s->d_cloud_col + o : nullptr;
+            CU(rcm_launch_lbl_prep(a, q));
+            if (vmr_scale) CU(rcm_launch_lbl_scale(a, sc.f[0], sc.f[2], q));
+            s->launches += vmr_scale ? 2 : 1;
+            return RCM_OK;
+        },
+        [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
+            if (bands) {
+                CU(rcm_launch_lbl_band(a, z.spec_dn, z.spec_up, q));
+                CU(rcm_launch_lbl_band_sum(a.ncol, nwvl, nband, z.bstart, z.spec_dn, z.spec_up, z.band_dn, z.band_up, q));
+                s->launches += 2;
+            }
+            if (broad) {
+                CU(rcm_launch_lbl_rt(a, q, nullptr, nullptr));
+                CU(rcm_launch_lbl_finish(a, q));
+                s->launches += 2;
+            }
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            const size_t nb = (size_t)n * nband * NLEV;
+            if (E_down_band) CU(cudaMemcpyAsync(E_down_band + r * nband * NLEV, z.band_dn, nb * D, cudaMemcpyDeviceToHost, q));
+            if (E_up_band) CU(cudaMemcpyAsync(E_up_band + r * nband * NLEV, z.band_up, nb * D, cudaMemcpyDeviceToHost, q));
+            if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Ed, n * NLEV * D, cudaMemcpyDeviceToHost, q));
+            if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Eu, n * NLEV * D, cudaMemcpyDeviceToHost, q));
+            if (dE) CU(cudaMemcpyAsync(dE + r * NLAY, z.dE, n * NLAY * D, cudaMemcpyDeviceToHost, q));
             return RCM_OK;
         });
 }

@@ -25,6 +25,7 @@
 #include "rcm_jac.cuh"
 #include "rcm_fjac.cuh"
 #include "rcm_fdh.cuh"
+#include "rcm_lbl_diag.cuh"
 
 __constant__ DevConst cst;
 
@@ -194,6 +195,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 }
 
 #include "rcm_lbl_kernels.cuh"
+#include "rcm_lbl_diag_kernels.cuh"
 #include "rcm_split_kernels.cuh"
 #include "rcm_diag_kernels.cuh"
 #include "rcm_jac_kernels.cuh"
@@ -378,9 +380,13 @@ size_t rcm_lbl_smem_bytes(int C, int nthreads) {
             (size_t)NLEV * (nthreads / 2)) * sizeof(double);
 }
 
-cudaError_t rcm_launch_lbl_step(const LblArgs& a, cudaStream_t st, cudaEvent_t ev0, cudaEvent_t ev1) {
-    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
+cudaError_t rcm_launch_lbl_prep(const LblArgs& a, cudaStream_t st) {
     rcm_lbl_prep_kernel<<<(a.ncol + 127) / 128, 128, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_rt(const LblArgs& a, cudaStream_t st, cudaEvent_t ev0, cudaEvent_t ev1) {
+    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
     const size_t smem = rcm_lbl_smem_bytes(C, NT);
     auto kern = a.clampk ? rcm_lbl_rt_kernel<C, NT, true> : rcm_lbl_rt_kernel<C, NT, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -388,7 +394,50 @@ cudaError_t rcm_launch_lbl_step(const LblArgs& a, cudaStream_t st, cudaEvent_t e
     if (ev0) cudaEventRecord(ev0, st);
     kern<<<a.ntiles * a.nchunks, NT, smem, st>>>(a);
     if (ev1) cudaEventRecord(ev1, st);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_finish(const LblArgs& a, cudaStream_t st) {
     rcm_lbl_finish_kernel<<<a.ncol, LBL_FIN_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_step(const LblArgs& a, cudaStream_t st, cudaEvent_t ev0, cudaEvent_t ev1) {
+    cudaError_t e = rcm_launch_lbl_prep(a, st);
+    if (e == cudaSuccess) e = rcm_launch_lbl_rt(a, st, ev0, ev1);
+    if (e == cudaSuccess) e = rcm_launch_lbl_finish(a, st);
+    return e;
+}
+
+cudaError_t rcm_launch_lbl_scale(const LblArgs& a, double f_h2o, double f_o3, cudaStream_t st) {
+    rcm_lbl_scale_kernel<<<(a.ncol * NLAY + 127) / 128, 128, 0, st>>>(a, f_h2o, f_o3);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_plane(const double* raw, size_t n, double f_co2x, double f_ch4, double f_n2o, double* out, cudaStream_t st) {
+    rcm_lbl_plane_kernel<<<296, 256, 0, st>>>(raw, n, f_co2x, f_ch4, f_n2o, out);
+    return cudaGetLastError();
+}
+
+size_t rcm_lbl_band_smem_bytes() {
+    return rcm_lbl_smem_bytes(RCM_LBL_C, RCM_LBL_NT) + (size_t)NLEV * (RCM_LBL_NT / 2) * sizeof(double);
+}
+
+cudaError_t rcm_launch_lbl_band(const LblArgs& a, double* spec_dn, double* spec_up, cudaStream_t st) {
+    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
+    const size_t smem = rcm_lbl_band_smem_bytes();
+    auto kern = a.clampk ? rcm_lbl_band_kernel<C, NT, true> : rcm_lbl_band_kernel<C, NT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<a.ntiles * a.nchunks, NT, smem, st>>>(a, spec_dn, spec_up);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_band_sum(int ncol, int nwvl, int nband, const int* band_start, const double* spec_dn,
+                                    const double* spec_up, double* band_dn, double* band_up, cudaStream_t st) {
+    const size_t blocks = ((size_t)ncol * nband * NLEV + 255) / 256;
+    rcm_lbl_band_sum_kernel<<<blocks < 4096 ? (int)blocks : 4096, 256, 0, st>>>(ncol, nwvl, nband, band_start, spec_dn, spec_up,
+                                                                                band_dn, band_up);
     return cudaGetLastError();
 }
 
