@@ -320,6 +320,31 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
  * for nband < 1, a NULL band_start or one that does not rise strictly from 0 to nwvl.  Each error leaves the solver usable. */
 int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
                             double* E_down_band, double* E_up_band, double* E_down, double* E_up, double* dE);
+/* Radiative kernels of the line-by-line path: analytic derivatives of the OLR (output 0, E_up[0]) and the surface downward
+ * flux (output 1, E_down[20]) of the NEXT LBL step for the columns [col0, col0 + ncol), at exactly the state
+ * rcm_lbl_diagnose_fluxes radiates for the same arguments (theta-sorted profile, H2O after the feedback - none at step 0 -,
+ * grey or per-column cloud, vmr_scale applied as there).  Entries and outputs as rcm_radiative_kernels, 41 per output:
+ * 0..19 dF/dT_l (layers top-down), 20 dF/dT_surf, 21..40 dF/dln q_l (q_l the layer's H2O VMR as the step uses it).
+ * LBL tau does not depend on T, so:
+ *   d/dT_l moves layer l's Planck source only (fixed q, no re-sort, no feedback); d/dT_surf the surface source (exactly 0.0
+ *   for output 1); d/dln q_l = dF/dtau_l x (tau_H2O,l x s_H2O,l) at fixed T, 0 where the tau clamp acts (tau_clamp, on angle
+ *   schedules that clamp tau in front of the exp).
+ *   dB/dT of the band Planck source, K = sigma/pi x 15/pi^4, f(x) = x^3 / (e^x - 1): on the Simpson branch K T^3 S_n[g],
+ *   g(x) = x^4 e^x / (e^x - 1)^2, Simpson's rule on the abscissae, exponentials and order n of B itself (the exact derivative
+ *   of the Simpson value); on every other branch 4 B / T - K T^3 (v1 f(v1) - v0 f(v0)) (an overflowing exp: a term of 0);
+ *   0 for T < 1e-4.
+ * Outputs (host, either may be NULL; both NULL: RCM_OK without work): K [ncol][2][41] the sum over all wavelengths in index
+ * order from 0.0; K_band [ncol][nband][2][41], band b the sum over [band_start[b], band_start[b + 1]) in index order from 0.0
+ * (K equals K_band of the one band {0, nwvl} bit for bit; a band of one wavelength is that wavelength's contribution).
+ * band_start as rcm_lbl_diagnose_fluxes, read only for K_band.  Every value is a function of its column alone: ranges,
+ * chunks and shards give bit-identical rows.  Synchronous; changes nothing.
+ * Device scratch of its own: two sets for chunks of ch columns (whole tiles of 16, at most 8,192 and at most
+ * 2e9 / (nwvl x 82 x 8) rounded down to whole tiles, at least 16), each of 8 ch (182 + 82 nwvl + 82_K + 82 nband_b) + 4 (2 +
+ * (nband + 1)_b) bytes rounded up to 256, the _K term only for K, the _b terms only for K_band; with CO2, CH4 or N2O scaled
+ * also the 3 x nwvl x 20 doubles of rcm_lbl_diagnose_fluxes.  About 3.8 GB at 20,000 wavelengths.
+ * Errors as rcm_lbl_diagnose_fluxes (the band checks for K_band); each leaves the solver usable. */
+int rcm_lbl_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
+                              double* K_band, double* K);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

@@ -440,6 +440,30 @@ class Solver:
                                             _p(out["E_up"]), _p(out["dE"])), self._h)
         return out
 
+    def lbl_radiative_kernels(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, bands=None) -> dict:
+        """rcm_lbl_radiative_kernels: derivatives of the next line-by-line step's OLR (output 0) and surface downward flux
+        (output 1) for columns [col0, col0 + ncol), at the state lbl_diagnose_fluxes radiates, without changing anything.
+        vmr_scale and bands as in lbl_diagnose_fluxes.
+        -> K [ncol, 2, 41] (entries as radiative_kernels; the sum over the wavelengths in index order) with the views
+        dOLR_dT, dOLR_dTs, dOLR_dlnq, dSFC_dT, dSFC_dlnq, and with bands K_band [ncol, nband, 2, 41] (each band the sum of
+        its wavelengths' contributions in index order)."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = self._vmr_scale(vmr_scale)
+        m = max(n, 0)
+        K = np.zeros((m, 2, 2 * NLAY + 1))
+        bs, nband, Kb = None, 0, None
+        if bands is not None:
+            bs = np.ascontiguousarray(bands, dtype=np.int32).ravel()
+            nband = bs.size - 1
+            Kb = np.zeros((m, max(nband, 0), 2, 2 * NLAY + 1))
+        _check(_lib.rcm_lbl_radiative_kernels(self._h, C.c_int(col0), C.c_int(n), _p(sc), C.c_int(nband), _p(bs), _p(Kb),
+                                              _p(K)), self._h)
+        out = dict(K=K, dOLR_dT=K[:, 0, :NLAY], dOLR_dTs=K[:, 0, NLAY], dOLR_dlnq=K[:, 0, NLAY + 1:],
+                   dSFC_dT=K[:, 1, :NLAY], dSFC_dlnq=K[:, 1, NLAY + 1:])
+        if Kb is not None:
+            out["K_band"] = Kb
+        return out
+
     def radiative_kernels(self, col0: int = 0, ncol: int | None = None, vmr_scale=None, spectral: bool = False) -> dict:
         """rcm_radiative_kernels: derivatives of the next step's OLR (output 0) and surface downward flux (output 1) for
         columns [col0, col0 + ncol), without changing anything.  vmr_scale as in diagnose_fluxes.

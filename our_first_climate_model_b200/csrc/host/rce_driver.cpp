@@ -11,7 +11,7 @@
 //           [--spectral-out spectrum.csv] [--kernels-out kernels.csv] [--jacobian-out jacobian.csv]
 //           [--forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
-//           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]]
+//           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out kernels.csv]
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
 // --gpus N (N > 1): one process, one host thread and one solver per GPU, contiguous blocks of columns per GPU (tables
@@ -54,6 +54,10 @@
 // "wvl_lo_nm,wvl_hi_nm,olr,surface_down,olr_scaled,surface_down_scaled", then one row per band with its edges (the midpoint
 // bins of rcm_set_lbl_tables) and the ensemble means of its TOA upward and surface downward flux (W/m2), unscaled and scaled.
 // Summed in column order: the file is byte-identical for any --gpus N.
+//
+// --lbl-kernels-out FILE (line-by-line tables only): after the run, the radiative kernels of the next LBL step
+// (rcm_lbl_radiative_kernels, summed over all wavelengths) in the format of --kernels-out.  Summed in column order: the file
+// is byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -107,7 +111,8 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     float* time_out;
     int spec_nwvl;            // > 0: --spectral-out, rows [ncol][spec_nwvl] of olr / sfc
     double *olr_out, *sfc_out;
-    int kernels;              // --kernels-out: rows [ncol][2][41] of rcm_radiative_kernels into K_out
+    int kernels;              // --kernels-out / --lbl-kernels-out: rows [ncol][2][41] of rcm_radiative_kernels (repwvl) or
+                              // rcm_lbl_radiative_kernels (line-by-line) into K_out
     double* K_out;
     int jacobian;             // --jacobian-out: rows [ncol][20][41] of rcm_flux_jacobian's dE_jac into H_out
     double* H_out;
@@ -381,8 +386,9 @@ void run_shard(Shard* sh, const Job* j) {
         if (st != RCM_OK) return fail("rcm_diagnose_fluxes", st);
     }
     if (j->kernels) {
-        st = rcm_radiative_kernels(sh->s, 0, (int)n, nullptr, nullptr, j->K_out + lo * KERN_NK);
-        if (st != RCM_OK) return fail("rcm_radiative_kernels", st);
+        st = j->table ? rcm_radiative_kernels(sh->s, 0, (int)n, nullptr, nullptr, j->K_out + lo * KERN_NK)
+                      : rcm_lbl_radiative_kernels(sh->s, 0, (int)n, nullptr, 0, nullptr, nullptr, j->K_out + lo * KERN_NK);
+        if (st != RCM_OK) return fail(j->table ? "rcm_radiative_kernels" : "rcm_lbl_radiative_kernels", st);
     }
     if (j->jacobian) {
         st = rcm_flux_jacobian(sh->s, 0, (int)n, nullptr, nullptr, j->H_out + lo * JAC_NH);
@@ -403,7 +409,8 @@ void run_shard(Shard* sh, const Job* j) {
 
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
-        jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100";
+        jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100",
+        lbl_kernels_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -435,6 +442,7 @@ int main(int argc, char** argv) {
         else if (a == "--trop-layers") trop_layers_arg = val();
         else if (a == "--lbl-bands-out") bands_path = val();
         else if (a == "--band-size") band_size_arg = val();
+        else if (a == "--lbl-kernels-out") lbl_kernels_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -446,7 +454,7 @@ int main(int argc, char** argv) {
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
                              "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE] "
                              "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
-                             "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]]\n");
+                             "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out FILE]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -454,7 +462,7 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (!lbl_dir.empty() && !kernels_path.empty()) {
-        std::fprintf(stderr, "rcm_rce: --kernels-out needs a repwvl table (--table): the line-by-line path has no radiative kernels\n");
+        std::fprintf(stderr, "rcm_rce: --kernels-out needs a repwvl table (--table): with --lbl use --lbl-kernels-out\n");
         return 1;
     }
     if (!lbl_dir.empty() && !jacobian_path.empty()) {
@@ -465,6 +473,11 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rcm_rce: --forcing-out needs a repwvl table (--table): the line-by-line path has no adjusted forcing\n");
         return 1;
     }
+    if (lbl_dir.empty() && !lbl_kernels_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-kernels-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
+    if (!lbl_kernels_path.empty()) kernels_path = lbl_kernels_path;  // the same kernels file, from the LBL call
     if (lbl_dir.empty() && !bands_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --lbl-bands-out needs line-by-line tables (--lbl)\n");
         return 1;
@@ -760,8 +773,9 @@ int main(int argc, char** argv) {
     }
     if (!kernels_path.empty()) {
         std::vector<double> K(m * KERN_NK);
-        st = rcm_radiative_kernels(s, 0, ncol, nullptr, nullptr, K.data());
-        if (st != RCM_OK) return die("rcm_radiative_kernels", st, s);
+        st = lbl ? rcm_lbl_radiative_kernels(s, 0, ncol, nullptr, 0, nullptr, nullptr, K.data())
+                 : rcm_radiative_kernels(s, 0, ncol, nullptr, nullptr, K.data());
+        if (st != RCM_OK) return die(lbl ? "rcm_lbl_radiative_kernels" : "rcm_radiative_kernels", st, s);
         if (write_kernels(kernels_path, ncol, player.data(), plevel[NLAY], K.data())) return 1;
     }
     if (!jacobian_path.empty()) {

@@ -14,6 +14,7 @@
 #include "rcm_jac.cuh"
 #include "rcm_fdh.cuh"
 #include "rcm_lbl_diag.cuh"
+#include "rcm_lbl_jac.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -1784,61 +1785,128 @@ int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale
         });
 }
 
+// ------------------------------------------------------------------------------------------
+// Line-by-line calls (rcm_lbl_diagnose_fluxes, rcm_lbl_radiative_kernels): the step's prep kernel on copies of a chunk's T,
+// previous profile, VMRs and T_surf, then the species factors; the state stays as it is.
+// ------------------------------------------------------------------------------------------
+constexpr double kLblStageBytes = 2e9;  // per scratch set: a chunk's per-wavelength staging (band fluxes, kernels)
+
+extern "C++" {
+namespace {
+
+// the checks every LBL call makes, then diag_range
+int lbl_check(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, DiagScale& sc) {
+    if (!s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": needs the line-by-line path (rcm_set_lbl_tables)");
+    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
+    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
+    return diag_range(s, fn, col0, ncol, vmr_scale, sc);
+}
+
+// band_start [nband + 1]: 0 = b_0 < b_1 < ... < b_nband = nwvl
+int lbl_band_check(rcm_solver* s, const std::string& fn, int nband, const int* band_start) {
+    if (nband < 1 || !band_start) return fail(s, RCM_ERR_ARG, fn + ": band outputs need nband >= 1 and band_start");
+    for (int b = 0; b < nband; ++b)
+        if (!(band_start[b] < band_start[b + 1]))
+            return fail(s, RCM_ERR_ARG, fn + ": band_start must be strictly increasing (entry " + std::to_string(b + 1) + ")");
+    if (band_start[0] != 0 || band_start[nband] != s->lbl_nwvl)
+        return fail(s, RCM_ERR_ARG, fn + ": band_start must run from 0 to nwvl = " + std::to_string(s->lbl_nwvl));
+    return RCM_OK;
+}
+
+// The planes the chunks radiate with into tau3: NULL (the tables' own) unless CO2, CH4 or N2O is scaled; then the
+// column-independent plane composed anew on the solver's stream, the H2O and O3 planes copied next to it.
+int lbl_planes(rcm_solver* s, const DiagScale& sc, const double*& tau3) {
+    constexpr size_t D = sizeof(double);
+    tau3 = nullptr;
+    CU(cudaSetDevice(s->device));
+    if (sc.f[1] == 1.0 && sc.f[3] == 1.0 && sc.f[4] == 1.0) return RCM_OK;
+    const size_t plane = (size_t)s->lbl_nwvl * NLAY;
+    if (s->tau3s_cap < 3 * plane) {
+        CU(dalloc(s->d_lbl_tau3s, 3 * plane));
+        s->tau3s_cap = 3 * plane;
+    }
+    CU(cudaMemcpyAsync(s->d_lbl_tau3s, s->d_lbl_tau5, 2 * plane * D, cudaMemcpyDeviceToDevice, s->stream));
+    CU(rcm_launch_lbl_plane(s->d_lbl_tau5 + 3 * plane, plane, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3],
+                            s->d_lbl_tau3s + 2 * plane, s->stream));
+    s->launches += 1;
+    tau3 = s->d_lbl_tau3s;
+    return RCM_OK;
+}
+
+// What the LBL prep reads and writes besides DiagState: T_surf [ch], sH, sO [ch][20].
+struct LblState {
+    double *Ts, *sH, *sO;
+};
+
+void lbl_take(DiagCarve& m, size_t ch, LblState& l) {
+    l.Ts = m.take<double>(ch);
+    l.sH = m.take<double>(ch * NLAY);
+    l.sO = m.take<double>(ch * NLAY);
+}
+
+// Copies of columns [c0, c0 + n) into d and l, the prep of the next step on them, then the H2O and O3 factors (sc: NULL =
+// unscaled).  On return l.sH / l.sO and d.T hold what the step radiates with; a carries the chunk's sizes, tables (tau3:
+// NULL = the tables' own planes) and the prepared copies.
+int lbl_prep(rcm_solver* s, cudaStream_t q, int c0, int n, const DiagState& d, const LblState& l, const double* tau3,
+             const DiagScale* sc, LblArgs& a) {
+    constexpr size_t D = sizeof(double);
+    const size_t o = (size_t)c0;
+    CU(cudaMemcpyAsync(d.T, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(d.Tprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(d.vmr, s->d_vmr + o * 5 * NLAY, (size_t)n * 5 * NLAY * D, cudaMemcpyDeviceToDevice, q));
+    CU(cudaMemcpyAsync(l.Ts, s->d_Ts + o, n * D, cudaMemcpyDeviceToDevice, q));
+    a = lbl_args(s, n);
+    a.step_index = s->step_index;
+    if (tau3) a.tau3 = tau3;
+    a.Tlayer = d.T; a.Tprev = d.Tprev; a.vmr = d.vmr; a.rel_hum = s->d_rh + o * NLAY;
+    a.Tsurf = l.Ts; a.sH = l.sH; a.sO = l.sO; a.dTstat = d.stat; a.diag = nullptr;
+    a.solar_col = s->has_col_solar ? s->d_solar_col + o : nullptr;
+    a.cloud_col = s->has_col_cloud ? s->d_cloud_col + o : nullptr;
+    CU(rcm_launch_lbl_prep(a, q));
+    if (sc) CU(rcm_launch_lbl_scale(a, sc->f[0], sc->f[2], q));
+    s->launches += sc ? 2 : 1;
+    return RCM_OK;
+}
+
+// columns per chunk of a call that stages row_doubles per (column, wavelength): diag_chunk(ncol), and at most kLblStageBytes of
+// staging rounded down to whole tiles, at least one tile
+size_t lbl_stage_chunk(const rcm_solver* s, int ncol, size_t row_doubles) {
+    const size_t fit = (size_t)(kLblStageBytes / ((double)s->lbl_nwvl * row_doubles * sizeof(double))) / 16 * 16;
+    return std::min(diag_chunk(ncol), std::max<size_t>(16, fit));
+}
+
+}  // namespace
+}  // extern "C++"
+
 // Line-by-line fluxes: the step's three kernels on copies of a chunk (prep, the species factors, rt, finish into scratch), and
 // for bands rcm_lbl_band_kernel + rcm_lbl_band_sum_kernel on the same prepared copies, in front of the finish (which moves T).
-constexpr double kLblStageBytes = 2e9;  // per scratch set: the band pass's staging, ch x nwvl x 42 doubles
-
 int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
                             double* E_down_band, double* E_up_band, double* E_down, double* E_up, double* dE) {
     if (!s) return RCM_ERR_ARG;
     const std::string fn = "rcm_lbl_diagnose_fluxes";
-    if (!s->lbl_mode) return fail(s, RCM_ERR_STATE, fn + ": needs the line-by-line path (rcm_set_lbl_tables)");
-    if (s->ncol <= 0) return fail(s, RCM_ERR_STATE, fn + ": no columns loaded");
-    if (s->nactive != 5) return fail(s, RCM_ERR_STATE, fn + ": needs the five active species of the default species_mask");
     DiagScale sc{};
-    int st = diag_range(s, fn, col0, ncol, vmr_scale, sc);
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     const int nwvl = s->lbl_nwvl;
     const bool bands = E_down_band || E_up_band, broad = E_down || E_up || dE;
-    if (bands) {
-        if (nband < 1 || !band_start) return fail(s, RCM_ERR_ARG, fn + ": band outputs need nband >= 1 and band_start");
-        for (int b = 0; b < nband; ++b)
-            if (!(band_start[b] < band_start[b + 1]))
-                return fail(s, RCM_ERR_ARG, fn + ": band_start must be strictly increasing (entry " + std::to_string(b + 1) + ")");
-        if (band_start[0] != 0 || band_start[nband] != nwvl)
-            return fail(s, RCM_ERR_ARG, fn + ": band_start must run from 0 to nwvl = " + std::to_string(nwvl));
-    }
+    if (bands && (st = lbl_band_check(s, fn, nband, band_start)) != RCM_OK) return st;
     if (!bands && !broad) return RCM_OK;
     constexpr size_t D = sizeof(double);
-    CU(cudaSetDevice(s->device));
-    // CO2, CH4 or N2O scaled: the column-independent plane composed anew, the H2O and O3 planes copied next to it
-    const bool plane3 = sc.f[1] != 1.0 || sc.f[3] != 1.0 || sc.f[4] != 1.0;
-    const size_t plane = (size_t)nwvl * NLAY;
-    if (plane3) {
-        if (s->tau3s_cap < 3 * plane) {
-            CU(dalloc(s->d_lbl_tau3s, 3 * plane));
-            s->tau3s_cap = 3 * plane;
-        }
-        CU(cudaMemcpyAsync(s->d_lbl_tau3s, s->d_lbl_tau5, 2 * plane * D, cudaMemcpyDeviceToDevice, s->stream));
-        CU(rcm_launch_lbl_plane(s->d_lbl_tau5 + 3 * plane, plane, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3],
-                                s->d_lbl_tau3s + 2 * plane, s->stream));
-        s->launches += 1;
-    }
-    size_t ch = diag_chunk(ncol);
-    if (bands) ch = std::min(ch, std::max<size_t>(16, (size_t)(kLblStageBytes / ((double)nwvl * 2 * NLEV * D)) / 16 * 16));
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const size_t ch = bands ? lbl_stage_chunk(s, ncol, 2 * NLEV) : diag_chunk(ncol);
     const size_t nchunks = (size_t)lbl_args(s, 0).nchunks;
     struct Set {
         DiagState state;
-        double *Ts, *sH, *sO, *dt, *part, *Ed, *Eu, *dE, *spec_dn, *spec_up, *band_dn, *band_up;
+        LblState lbl;
+        double *dt, *part, *Ed, *Eu, *dE, *spec_dn, *spec_up, *band_dn, *band_up;
         float* time;
         int* bstart;
     };
     return chunk_loop<Set, LblArgs>(
         s, col0, ncol, ch, false,
         [&](DiagCarve& m, size_t ch, Set& z) {
-            z.Ts = m.take<double>(ch);
-            z.sH = m.take<double>(ch * NLAY);
-            z.sO = m.take<double>(ch * NLAY);
+            lbl_take(m, ch, z.lbl);
             z.dt = m.take<double>(ch);
             z.part = m.take<double>(broad ? nchunks * ch * 2 * NLEV : 0);
             z.Ed = m.take<double>(ch * NLEV);
@@ -1852,24 +1920,10 @@ int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr
             z.bstart = m.take<int>(bands ? nband + 1 : 0);
         },
         [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
-            const size_t o = (size_t)c0;
-            CU(cudaMemcpyAsync(z.state.T, s->d_T + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-            CU(cudaMemcpyAsync(z.state.Tprev, s->d_Tprev + o * NLAY, n * NLAY * D, cudaMemcpyDeviceToDevice, q));
-            CU(cudaMemcpyAsync(z.state.vmr, s->d_vmr + o * 5 * NLAY, (size_t)n * 5 * NLAY * D, cudaMemcpyDeviceToDevice, q));
-            CU(cudaMemcpyAsync(z.Ts, s->d_Ts + o, n * D, cudaMemcpyDeviceToDevice, q));
             if (bands) CU(cudaMemcpyAsync(z.bstart, band_start, (nband + 1) * sizeof(int), cudaMemcpyHostToDevice, q));
-            a = lbl_args(s, n);
-            a.step_index = s->step_index;
-            if (plane3) a.tau3 = s->d_lbl_tau3s;
-            a.Tlayer = z.state.T; a.Tprev = z.state.Tprev; a.vmr = z.state.vmr; a.rel_hum = s->d_rh + o * NLAY;
-            a.Tsurf = z.Ts; a.time_h = z.time; a.sH = z.sH; a.sO = z.sO; a.dTstat = z.state.stat; a.part = z.part;
-            a.E_down = z.Ed; a.E_up = z.Eu; a.dE = z.dE; a.dt = z.dt; a.diag = nullptr;
-            a.solar_col = s->has_col_solar ? s->d_solar_col + o : nullptr;
-            a.cloud_col = s->has_col_cloud ? s->d_cloud_col + o : nullptr;
-            CU(rcm_launch_lbl_prep(a, q));
-            if (vmr_scale) CU(rcm_launch_lbl_scale(a, sc.f[0], sc.f[2], q));
-            s->launches += vmr_scale ? 2 : 1;
-            return RCM_OK;
+            const int r = lbl_prep(s, q, c0, n, z.state, z.lbl, tau3, vmr_scale ? &sc : nullptr, a);
+            a.time_h = z.time; a.part = z.part; a.E_down = z.Ed; a.E_up = z.Eu; a.dE = z.dE; a.dt = z.dt;
+            return r;
         },
         [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
             if (bands) {
@@ -1891,6 +1945,65 @@ int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr
             if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Ed, n * NLEV * D, cudaMemcpyDeviceToHost, q));
             if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Eu, n * NLEV * D, cudaMemcpyDeviceToHost, q));
             if (dE) CU(cudaMemcpyAsync(dE + r * NLAY, z.dE, n * NLAY * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+// Line-by-line radiative kernels: per chunk the prep of the fluxes call, then rcm_lbl_jac_kernel into the staging K_spec and
+// rcm_lbl_jac_band_sum_kernel for the bands and for the one band {0, nwvl} of K.  No finish kernel: nothing here moves T.
+int rcm_lbl_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
+                              double* K_band, double* K) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_radiative_kernels";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    const int nwvl = s->lbl_nwvl;
+    if (K_band && (st = lbl_band_check(s, fn, nband, band_start)) != RCM_OK) return st;
+    if (!K_band && !K) return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const int nb = K_band ? nband : 0;
+    const int whole[2] = {0, nwvl};
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    struct Set {
+        DiagState state;
+        LblState lbl;
+        double *K_spec, *K, *K_band;
+        int *whole, *bstart;
+    };
+    return chunk_loop<Set, LblArgs>(
+        s, col0, ncol, lbl_stage_chunk(s, ncol, JAC_NK), false,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // K_spec [ch][nwvl][82], K [ch][82], K_band [ch][nband][82]
+            lbl_take(m, ch, z.lbl);
+            z.K_spec = m.take<double>(ch * nwvl * JAC_NK);
+            z.K = m.take<double>(K ? ch * JAC_NK : 0);
+            z.K_band = m.take<double>(ch * nb * JAC_NK);
+            z.whole = m.take<int>(2);
+            z.bstart = m.take<int>(K_band ? nb + 1 : 0);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
+            if (K) CU(cudaMemcpyAsync(z.whole, whole, sizeof(whole), cudaMemcpyHostToDevice, q));
+            if (K_band) CU(cudaMemcpyAsync(z.bstart, band_start, (nb + 1) * sizeof(int), cudaMemcpyHostToDevice, q));
+            return lbl_prep(s, q, c0, n, z.state, z.lbl, tau3, vmr_scale ? &sc : nullptr, a);
+        },
+        [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
+            CU(rcm_launch_lbl_jac(a, wtau, z.K_spec, q));
+            s->launches += 1;
+            if (K_band) {
+                CU(rcm_launch_lbl_jac_band_sum(a.ncol, nwvl, nb, z.bstart, z.K_spec, z.K_band, q));
+                s->launches += 1;
+            }
+            if (K) {
+                CU(rcm_launch_lbl_jac_band_sum(a.ncol, nwvl, 1, z.whole, z.K_spec, z.K, q));
+                s->launches += 1;
+            }
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (K_band) CU(cudaMemcpyAsync(K_band + r * nb * JAC_NK, z.K_band, (size_t)n * nb * JAC_NK * D, cudaMemcpyDeviceToHost, q));
+            if (K) CU(cudaMemcpyAsync(K + r * JAC_NK, z.K, (size_t)n * JAC_NK * D, cudaMemcpyDeviceToHost, q));
             return RCM_OK;
         });
 }

@@ -26,6 +26,7 @@
 #include "rcm_fjac.cuh"
 #include "rcm_fdh.cuh"
 #include "rcm_lbl_diag.cuh"
+#include "rcm_lbl_jac.cuh"
 
 __constant__ DevConst cst;
 
@@ -201,6 +202,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_jac_kernels.cuh"
 #include "rcm_fjac_kernels.cuh"
 #include "rcm_fdh_kernels.cuh"
+#include "rcm_lbl_jac_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -483,6 +485,29 @@ cudaError_t rcm_launch_fjac(const FjacArgs& a, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FJAC_SMEM);
     if (e != cudaSuccess) return e;
     kern<<<(a.ncol + FJAC_WARPS - 1) / FJAC_WARPS, FJAC_NT, FJAC_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+size_t rcm_lbl_jac_smem_bytes() {
+    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
+    return ((size_t)EXP_TAB * EXP_REP + 3 * TBD_LEN + 2 * C + 2 * (HALF + 1) * NT + (size_t)(NT / (2 * C)) * C * JAC_NK) *
+           sizeof(double);
+}
+
+cudaError_t rcm_launch_lbl_jac(const LblArgs& a, double wtau, double* K_spec, cudaStream_t st) {
+    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
+    const size_t smem = rcm_lbl_jac_smem_bytes();
+    auto kern = a.clampk ? rcm_lbl_jac_kernel<C, NT, true> : rcm_lbl_jac_kernel<C, NT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<a.ntiles * a.nchunks, NT, smem, st>>>(a, wtau, K_spec);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_jac_band_sum(int ncol, int nwvl, int nband, const int* band_start, const double* K_spec, double* K_band,
+                                        cudaStream_t st) {
+    const size_t blocks = ((size_t)ncol * nband * JAC_NK + 255) / 256;
+    rcm_lbl_jac_band_sum_kernel<<<blocks < 4096 ? (int)blocks : 4096, 256, 0, st>>>(ncol, nwvl, nband, band_start, K_spec, K_band);
     return cudaGetLastError();
 }
 
