@@ -345,6 +345,30 @@ int rcm_lbl_diagnose_fluxes(rcm_solver* s, int col0, int ncol, const double* vmr
  * Errors as rcm_lbl_diagnose_fluxes (the band checks for K_band); each leaves the solver usable. */
 int rcm_lbl_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* vmr_scale, int nband, const int* band_start,
                               double* K_band, double* K);
+/* Flux Jacobians of the line-by-line path: analytic derivatives of every level's broadband E_down and E_up of the NEXT LBL step
+ * (summed over the wavelengths in index order) and of its heating rates, for the columns [col0, col0 + ncol), at exactly the
+ * state rcm_lbl_radiative_kernels differentiates for the same arguments, with its definitions (d/dT_l through layer l's Planck
+ * source alone, d/dln q_l = dF/dtau_l x tau_H2O,l x s_H2O,l, 0 where the tau clamp acts).  Outputs, entries and structural
+ * zeros as rcm_flux_jacobian: J [ncol][2][21][41], dE_jac [ncol][20][41] from J as dE from E (main.cpp:337-341).  Rows
+ * E_up[0] and E_down[20] of J are rcm_lbl_radiative_kernels' K to rounding (the same terms, summed per level instead of per
+ * wavelength).  Both outputs NULL: RCM_OK without work.  Every value is a function of its column alone: ranges, chunks and
+ * shards give bit-identical rows.  Synchronous; changes nothing.  Device scratch of its own: two sets for chunks of at most
+ * 8,192 columns, each of 2,724 doubles per column (about 0.36 GB, independent of the wavelengths); with CO2, CH4 or N2O
+ * scaled also the 3 x nwvl x 20 doubles of rcm_lbl_diagnose_fluxes.  Errors as rcm_lbl_diagnose_fluxes. */
+int rcm_lbl_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
+/* Stratosphere-adjusted forcing of the line-by-line path, as rcm_adjusted_forcing (ntrop, tol, max_iter, convergence, freezing,
+ * iters, the outputs F, dT_adj, E_down, E_up and the argument errors) with these substitutions:
+ * Base state: what rcm_lbl_diagnose_fluxes(..., NULL, ...) radiates; its E_down, E_up and dE equal the next rcm_advance(1) bit
+ * for bit.  Perturbed state: the same with vmr_scale applied exactly as rcm_lbl_diagnose_fluxes applies it, so that the IRF of
+ * iterate 0 is rcm_lbl_diagnose_fluxes(vmr_scale) minus the unscaled call, bit for bit.
+ * Adjustment: dT_l (l < ntrop) moves layer l's Planck source only (LBL tau does not depend on T; no step-0 rule).
+ * Solve: Newton on the ntrop x ntrop block of rcm_lbl_flux_jacobian's dE_jac, re-evaluated at every iterate.
+ * Synchronous; changes nothing.  Device scratch of its own: two sets for chunks of at most 8,192 columns, each of
+ * 2,956 + 42 ceil(nwvl / 128) doubles and 12 bytes per column (about 1.25 GB at 20,000 wavelengths); with CO2, CH4 or N2O
+ * scaled also the 3 x nwvl x 20 doubles of rcm_lbl_diagnose_fluxes.  Errors as rcm_lbl_flux_jacobian, then those of
+ * rcm_adjusted_forcing's arguments. */
+int rcm_lbl_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol,
+                             int max_iter, double* F, double* dT_adj, double* E_down, double* E_up, int* iters);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

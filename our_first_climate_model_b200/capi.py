@@ -504,6 +504,30 @@ class Solver:
         -> F [ncol, 4] with the views IRF_toa, IRF_trop, SARF_toa, SARF_trop (W/m2), dT_adj [ncol, 20] (K), E_down, E_up
         [ncol, 21] at the adjusted perturbed state, iters [ncol] (Newton updates applied, -1: not converged) and
         converged [ncol] (iters >= 0)."""
+        return self._forcing(_lib.rcm_adjusted_forcing, vmr_scale, ntrop, col0, ncol, tol, max_iter)
+
+    def lbl_flux_jacobian(self, col0: int = 0, ncol: int | None = None, vmr_scale=None) -> dict:
+        """rcm_lbl_flux_jacobian: derivatives of the next line-by-line step's broadband fluxes at every level and of its
+        heating rates for columns [col0, col0 + ncol), at the state lbl_radiative_kernels differentiates, without changing
+        anything.  vmr_scale as in lbl_diagnose_fluxes.  Entries as in flux_jacobian.
+        -> J [ncol, 2, 21, 41] (J[:, 0, k] = dE_down[k], J[:, 1, k] = dE_up[k]) and dE_jac [ncol, 20, 41]."""
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = self._vmr_scale(vmr_scale)
+        m = max(n, 0)
+        J = np.zeros((m, 2, NLAY + 1, 2 * NLAY + 1))
+        H = np.zeros((m, NLAY, 2 * NLAY + 1))
+        _check(_lib.rcm_lbl_flux_jacobian(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(J), _p(H)), self._h)
+        return dict(J=J, dE_jac=H)
+
+    def lbl_adjusted_forcing(self, vmr_scale, ntrop, col0: int = 0, ncol: int | None = None, tol: float = 1e-6,
+                             max_iter: int = 20) -> dict:
+        """rcm_lbl_adjusted_forcing: adjusted_forcing on the line-by-line path (base state: what lbl_diagnose_fluxes
+        radiates unscaled; perturbed: with vmr_scale applied as there; dT moves the layers' Planck source only).  Arguments
+        and results as adjusted_forcing."""
+        return self._forcing(_lib.rcm_lbl_adjusted_forcing, vmr_scale, ntrop, col0, ncol, tol, max_iter)
+
+    def _forcing(self, fn, vmr_scale, ntrop, col0, ncol, tol, max_iter) -> dict:
+        """the arguments and results of the two adjusted-forcing calls around fn"""
         n = self.ncol - col0 if ncol is None else int(ncol)
         m = max(n, 0)
         sc = self._vmr_scale(vmr_scale)
@@ -517,8 +541,8 @@ class Solver:
         dT = np.zeros((m, NLAY))
         Ed, Eu = np.zeros((m, NLEV)), np.zeros((m, NLEV))
         it = np.zeros(m, dtype=np.int32)
-        _check(_lib.rcm_adjusted_forcing(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(nt), C.c_double(tol),
-                                         C.c_int(max_iter), _p(F), _p(dT), _p(Ed), _p(Eu), _p(it)), self._h)
+        _check(fn(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(nt), C.c_double(tol), C.c_int(max_iter), _p(F), _p(dT),
+                  _p(Ed), _p(Eu), _p(it)), self._h)
         return dict(F=F, IRF_toa=F[:, 0], IRF_trop=F[:, 1], SARF_toa=F[:, 2], SARF_trop=F[:, 3], dT_adj=dT, E_down=Ed,
                     E_up=Eu, iters=it, converged=it >= 0)
 

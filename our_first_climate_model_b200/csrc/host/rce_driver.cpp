@@ -12,6 +12,7 @@
 //           [--forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out kernels.csv]
+//           [--lbl-jacobian-out jacobian.csv] [--lbl-forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
 // --gpus N (N > 1): one process, one host thread and one solver per GPU, contiguous blocks of columns per GPU (tables
@@ -58,6 +59,15 @@
 // --lbl-kernels-out FILE (line-by-line tables only): after the run, the radiative kernels of the next LBL step
 // (rcm_lbl_radiative_kernels, summed over all wavelengths) in the format of --kernels-out.  Summed in column order: the file
 // is byte-identical for any --gpus N.
+//
+// --lbl-jacobian-out FILE (line-by-line tables only): after the run, the derivatives of the next LBL step's heating rates
+// (rcm_lbl_flux_jacobian's dE_jac) in the format of --jacobian-out.  Summed in column order: the file is byte-identical for any
+// --gpus N.
+//
+// --lbl-forcing-out FILE (line-by-line tables only): after the run, the stratosphere-adjusted forcing of the next LBL step's
+// state (rcm_lbl_adjusted_forcing, tol 1e-6 W/m2, at most 20 Newton updates) for the factors --forcing-scale with the
+// --trop-layers top layers as the stratosphere, in the format of --forcing-out.  Summed in column order: the file is
+// byte-identical for any --gpus N.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -114,9 +124,11 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     int kernels;              // --kernels-out / --lbl-kernels-out: rows [ncol][2][41] of rcm_radiative_kernels (repwvl) or
                               // rcm_lbl_radiative_kernels (line-by-line) into K_out
     double* K_out;
-    int jacobian;             // --jacobian-out: rows [ncol][20][41] of rcm_flux_jacobian's dE_jac into H_out
+    int jacobian;             // --jacobian-out / --lbl-jacobian-out: rows [ncol][20][41] of rcm_flux_jacobian's (repwvl) or
+                              // rcm_lbl_flux_jacobian's (line-by-line) dE_jac into H_out
     double* H_out;
-    int forcing;              // --forcing-out: rcm_adjusted_forcing's F [ncol][4], dT_adj [ncol][20], iters [ncol]
+    int forcing;              // --forcing-out / --lbl-forcing-out: rcm_adjusted_forcing's (repwvl) or rcm_lbl_adjusted_forcing's
+                              // (line-by-line) F [ncol][4], dT_adj [ncol][20], iters [ncol]
     const double* forcing_scale;
     const int* ntrop;         // [ncol]
     double *F_out, *dTadj_out;
@@ -391,13 +403,14 @@ void run_shard(Shard* sh, const Job* j) {
         if (st != RCM_OK) return fail(j->table ? "rcm_radiative_kernels" : "rcm_lbl_radiative_kernels", st);
     }
     if (j->jacobian) {
-        st = rcm_flux_jacobian(sh->s, 0, (int)n, nullptr, nullptr, j->H_out + lo * JAC_NH);
-        if (st != RCM_OK) return fail("rcm_flux_jacobian", st);
+        st = (j->table ? rcm_flux_jacobian : rcm_lbl_flux_jacobian)(sh->s, 0, (int)n, nullptr, nullptr, j->H_out + lo * JAC_NH);
+        if (st != RCM_OK) return fail(j->table ? "rcm_flux_jacobian" : "rcm_lbl_flux_jacobian", st);
     }
     if (j->forcing) {
-        st = rcm_adjusted_forcing(sh->s, 0, (int)n, j->forcing_scale, j->ntrop + lo, FORCING_TOL, FORCING_MAX_ITER, j->F_out + lo * 4,
-                                  j->dTadj_out + lo * NLAY, nullptr, nullptr, j->iters_out + lo);
-        if (st != RCM_OK) return fail("rcm_adjusted_forcing", st);
+        st = (j->table ? rcm_adjusted_forcing : rcm_lbl_adjusted_forcing)(sh->s, 0, (int)n, j->forcing_scale, j->ntrop + lo, FORCING_TOL,
+                                                                         FORCING_MAX_ITER, j->F_out + lo * 4, j->dTadj_out + lo * NLAY,
+                                                                         nullptr, nullptr, j->iters_out + lo);
+        if (st != RCM_OK) return fail(j->table ? "rcm_adjusted_forcing" : "rcm_lbl_adjusted_forcing", st);
     }
     if (j->lbl_nband > 0) {
         st = diagnose_lbl_bands(sh->s, (int)n, j->lbl_nband, j->lbl_bstart, j->forcing_scale, j->B_out + lo * j->lbl_nband * 4);
@@ -410,7 +423,7 @@ void run_shard(Shard* sh, const Job* j) {
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
         jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100",
-        lbl_kernels_path;
+        lbl_kernels_path, lbl_jacobian_path, lbl_forcing_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
     long max_steps = 6000;
@@ -443,6 +456,8 @@ int main(int argc, char** argv) {
         else if (a == "--lbl-bands-out") bands_path = val();
         else if (a == "--band-size") band_size_arg = val();
         else if (a == "--lbl-kernels-out") lbl_kernels_path = val();
+        else if (a == "--lbl-jacobian-out") lbl_jacobian_path = val();
+        else if (a == "--lbl-forcing-out") lbl_forcing_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -454,7 +469,8 @@ int main(int argc, char** argv) {
                              "[--dT K/step] [--device D] [--out FILE] [--checkpoint FILE] [--resume FILE] [--steps-exact] [--gpus N] "
                              "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE] "
                              "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
-                             "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out FILE]\n");
+                             "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out FILE] "
+                             "[--lbl-jacobian-out FILE] [--lbl-forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -466,11 +482,11 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (!lbl_dir.empty() && !jacobian_path.empty()) {
-        std::fprintf(stderr, "rcm_rce: --jacobian-out needs a repwvl table (--table): the line-by-line path has no flux Jacobians\n");
+        std::fprintf(stderr, "rcm_rce: --jacobian-out needs a repwvl table (--table): with --lbl use --lbl-jacobian-out\n");
         return 1;
     }
     if (!lbl_dir.empty() && !forcing_path.empty()) {
-        std::fprintf(stderr, "rcm_rce: --forcing-out needs a repwvl table (--table): the line-by-line path has no adjusted forcing\n");
+        std::fprintf(stderr, "rcm_rce: --forcing-out needs a repwvl table (--table): with --lbl use --lbl-forcing-out\n");
         return 1;
     }
     if (lbl_dir.empty() && !lbl_kernels_path.empty()) {
@@ -478,6 +494,16 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (!lbl_kernels_path.empty()) kernels_path = lbl_kernels_path;  // the same kernels file, from the LBL call
+    if (lbl_dir.empty() && !lbl_jacobian_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-jacobian-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
+    if (!lbl_jacobian_path.empty()) jacobian_path = lbl_jacobian_path;  // the same Jacobian file, from the LBL call
+    if (lbl_dir.empty() && !lbl_forcing_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-forcing-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
+    if (!lbl_forcing_path.empty()) forcing_path = lbl_forcing_path;  // the same forcing file, from the LBL call
     if (lbl_dir.empty() && !bands_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --lbl-bands-out needs line-by-line tables (--lbl)\n");
         return 1;
@@ -780,16 +806,16 @@ int main(int argc, char** argv) {
     }
     if (!jacobian_path.empty()) {
         std::vector<double> H(m * JAC_NH);
-        st = rcm_flux_jacobian(s, 0, ncol, nullptr, nullptr, H.data());
-        if (st != RCM_OK) return die("rcm_flux_jacobian", st, s);
+        st = (lbl ? rcm_lbl_flux_jacobian : rcm_flux_jacobian)(s, 0, ncol, nullptr, nullptr, H.data());
+        if (st != RCM_OK) return die(lbl ? "rcm_lbl_flux_jacobian" : "rcm_flux_jacobian", st, s);
         if (write_jacobian(jacobian_path, ncol, player.data(), H.data())) return 1;
     }
     if (!forcing_path.empty()) {
         std::vector<double> Ff(m * 4), dTf(m * NLAY);
         std::vector<int> itf(m), ntrop(m, trop_layers);
-        st = rcm_adjusted_forcing(s, 0, ncol, forcing_scale, ntrop.data(), FORCING_TOL, FORCING_MAX_ITER, Ff.data(), dTf.data(), nullptr,
-                                  nullptr, itf.data());
-        if (st != RCM_OK) return die("rcm_adjusted_forcing", st, s);
+        st = (lbl ? rcm_lbl_adjusted_forcing : rcm_adjusted_forcing)(s, 0, ncol, forcing_scale, ntrop.data(), FORCING_TOL,
+                                                                    FORCING_MAX_ITER, Ff.data(), dTf.data(), nullptr, nullptr, itf.data());
+        if (st != RCM_OK) return die(lbl ? "rcm_lbl_adjusted_forcing" : "rcm_adjusted_forcing", st, s);
         if (write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) return 1;
     }
     if (!bands_path.empty()) {

@@ -15,6 +15,7 @@
 #include "rcm_fdh.cuh"
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
+#include "rcm_lbl_fjac.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -2008,6 +2009,95 @@ int rcm_lbl_radiative_kernels(rcm_solver* s, int col0, int ncol, const double* v
         });
 }
 
+// Line-by-line flux Jacobians: per chunk the prep of the fluxes call, then rcm_lbl_fjac_kernel, which sums over the
+// wavelengths itself, one warp per column.  No finish kernel: nothing here moves T.
+int rcm_lbl_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_flux_jacobian";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (!J && !dE_jac) return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    struct Set {
+        DiagState state;
+        LblState lbl;
+        double *J, *H;
+    };
+    return chunk_loop<Set, LblArgs>(
+        s, col0, ncol, diag_chunk(ncol), false,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // J [ch][2][21][41], dE_jac [ch][20][41]
+            lbl_take(m, ch, z.lbl);
+            z.J = m.take<double>(ch * FJAC_NJ);
+            z.H = m.take<double>(ch * FJAC_NH);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
+            return lbl_prep(s, q, c0, n, z.state, z.lbl, tau3, vmr_scale ? &sc : nullptr, a);
+        },
+        [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
+            CU(rcm_launch_lbl_fjac(a, wtau, z.J, z.H, q));
+            s->launches += 1;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (J) CU(cudaMemcpyAsync(J + r * FJAC_NJ, z.J, (size_t)n * FJAC_NJ * D, cudaMemcpyDeviceToHost, q));
+            if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * FJAC_NH, z.H, (size_t)n * FJAC_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+extern "C++" {
+namespace {
+
+// the arguments both adjusted-forcing calls check after the solver's state: ntrop [ncol] in [0, 19], tol, max_iter
+int fdh_check_args(rcm_solver* s, const std::string& fn, int ncol, const int* ntrop, double tol, int max_iter) {
+    if (!ntrop) return fail(s, RCM_ERR_ARG, fn + ": ntrop is NULL");
+    for (int c = 0; c < ncol; ++c)
+        if (ntrop[c] < 0 || ntrop[c] > FDH_MAXM)
+            return fail(s, RCM_ERR_ARG, fn + ": ntrop[" + std::to_string(c) + "] = " + std::to_string(ntrop[c]) + " outside [0, 19]");
+    if (!std::isfinite(tol) || !(tol > 0.0)) return fail(s, RCM_ERR_ARG, fn + ": tol must be finite and > 0");
+    if (max_iter < 1) return fail(s, RCM_ERR_ARG, fn + ": max_iter must be >= 1");
+    return RCM_OK;
+}
+
+// The two-slot Newton schedule of the adjusted-forcing calls over the chunks of ch columns from col0.  Slot k runs on its
+// stream z.q and carries c0, n, iter and live.  start(z, k, c0) enqueues a chunk up to the check of its iterate 0, whose active
+// count lands in h_fdh_count[k]; newton(z) enqueues the Jacobian and the Newton step; check(z, k) the evaluation of iterate
+// z.iter and its check; download(z) the chunk's outputs.  The host reads a chunk's active count after every check, and the two
+// slots take turns: one chunk's kernels run while the host waits for the other's count.
+template <class Slot, class Start, class Check, class Newton, class Download>
+int fdh_schedule(rcm_solver* s, Slot (&slot)[2], int col0, int ncol, size_t ch, Start start, Check check, Newton newton,
+                 Download download) {
+    int st;
+    int next = col0;
+    for (int k = 0; k < 2 && next < col0 + ncol; ++k, next += (int)ch)
+        if ((st = start(slot[k], k, next)) != RCM_OK) return st;
+    for (int k = 0; slot[0].live || slot[1].live; k ^= 1) {
+        Slot& z = slot[k];
+        if (!z.live) continue;
+        CU(cudaStreamSynchronize(z.q));
+        if (s->h_fdh_count[k] > 0) {  // (none is left after iterate max_iter)
+            if ((st = newton(z)) != RCM_OK) return st;
+            ++z.iter;
+            if ((st = check(z, k)) != RCM_OK) return st;
+            continue;
+        }
+        if ((st = download(z)) != RCM_OK) return st;
+        z.live = false;
+        if (next < col0 + ncol) {
+            if ((st = start(z, k, next)) != RCM_OK) return st;
+            next += (int)ch;
+        }
+    }
+    return diag_end(s);
+}
+
+}  // namespace
+}  // extern "C++"
+
 // Stratosphere-adjusted forcing: the scratch sets, streams, state copies and prep of the calls above.  Per chunk a base
 // evaluation (unscaled), the VMR scaling, then Newton iterations: retemper, evaluation (rcm_diag_rt_kernel +
 // rcm_diag_sum_kernel), check; while columns are active, the flux Jacobian (rcm_fjac_kernel) and the Newton step.  The host
@@ -2021,12 +2111,7 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
     int st = diag_check(s, fn, col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, fn + ": needs H2O among the active species");
-    if (!ntrop) return fail(s, RCM_ERR_ARG, fn + ": ntrop is NULL");
-    for (int c = 0; c < ncol; ++c)
-        if (ntrop[c] < 0 || ntrop[c] > FDH_MAXM)
-            return fail(s, RCM_ERR_ARG, fn + ": ntrop[" + std::to_string(c) + "] = " + std::to_string(ntrop[c]) + " outside [0, 19]");
-    if (!std::isfinite(tol) || !(tol > 0.0)) return fail(s, RCM_ERR_ARG, fn + ": tol must be finite and > 0");
-    if (max_iter < 1) return fail(s, RCM_ERR_ARG, fn + ": max_iter must be >= 1");
+    if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
     const int nwvl = s->dc.nwvl;
     const bool first = (s->step_index == 0);
     const size_t ch = diag_chunk(ncol), D = sizeof(double);
@@ -2135,27 +2220,156 @@ int rcm_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_sc
         if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
         return RCM_OK;
     };
-    int next = col0;
-    for (int k = 0; k < 2 && next < col0 + ncol; ++k, next += (int)ch)
-        if ((st = start(slot[k], k, next)) != RCM_OK) return st;
-    for (int k = 0; slot[0].live || slot[1].live; k ^= 1) {
-        Slot& z = slot[k];
-        if (!z.live) continue;
-        CU(cudaStreamSynchronize(z.q));
-        if (s->h_fdh_count[k] > 0) {  // (none is left after iterate max_iter)
-            if ((st = newton(z)) != RCM_OK) return st;
-            ++z.iter;
-            if ((st = check(z, k)) != RCM_OK) return st;
-            continue;
+    return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
+}
+
+// Line-by-line stratosphere-adjusted forcing: rcm_adjusted_forcing's Newton schedule (fdh_schedule), check and Newton kernels
+// on the state rcm_lbl_diagnose_fluxes radiates.  Per chunk: the prep on copies (unscaled, the tables' own planes), the
+// prepared T_B and T_surf saved, the base evaluation (the step's rt and finish kernels; the finish moves the copies' T and
+// T_surf), the H2O and O3 factors and the composed planes, then per iterate: rcm_lbl_fdh_retemper_kernel (every copy back to
+// T_B + dT and the saved T_surf), the evaluation and the check; while columns are active, rcm_lbl_fjac_kernel at T_B + dT and
+// the Newton step.  LBL tau does not depend on T: dT moves the Planck source of its layer alone.
+int rcm_lbl_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol,
+                             int max_iter, double* F, double* dT_adj, double* E_down, double* E_up, int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_adjusted_forcing";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const size_t ch = diag_chunk(ncol), D = sizeof(double);
+    const size_t nchunks = (size_t)lbl_args(s, 0).nchunks;
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    struct Slot {
+        cudaStream_t q;
+        int c0 = 0, n = 0, iter = 0;
+        bool live = false;
+        DiagState state;
+        LblState lbl;
+        double *Tb, *Ts0, *Tp, *dT, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *part, *dt;
+        float* time;
+        int *ntrop, *iters, *count;
+        LblArgs a;
+    } slot[2];
+    // the prep's T_surf, sH, sO; T_B, T_surf as prepared, T_B + dT, dT [ch][20]; E_down, E_up [ch][21] and dE [ch][20] of the
+    // base and of the current iterate, F [ch][4], the output E_down, E_up [ch][21], J [ch][2][21][41], dE_jac [ch][20][41],
+    // the rt kernel's partials [nchunks][ch][42], the finish's dt and time [ch]; ntrop, iters [ch] and the active count
+    st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
+        lbl_take(m, ch, z.lbl);
+        z.Tb = m.take<double>(ch * NLAY);
+        z.Ts0 = m.take<double>(ch);
+        z.Tp = m.take<double>(ch * NLAY);
+        z.dT = m.take<double>(ch * NLAY);
+        z.Ed0 = m.take<double>(ch * NLEV);
+        z.Eu0 = m.take<double>(ch * NLEV);
+        z.dE0 = m.take<double>(ch * NLAY);
+        z.Ed = m.take<double>(ch * NLEV);
+        z.Eu = m.take<double>(ch * NLEV);
+        z.dE = m.take<double>(ch * NLAY);
+        z.F = m.take<double>(ch * 4);
+        z.Edo = m.take<double>(ch * NLEV);
+        z.Euo = m.take<double>(ch * NLEV);
+        z.J = m.take<double>(ch * FJAC_NJ);
+        z.H = m.take<double>(ch * FJAC_NH);
+        z.part = m.take<double>(nchunks * ch * 2 * NLEV);
+        z.dt = m.take<double>(ch);
+        z.time = m.take<float>(ch);
+        z.ntrop = m.take<int>(ch);
+        z.iters = m.take<int>(ch);
+        z.count = m.take<int>(1);
+    }, false);
+    if (st != RCM_OK) return st;
+    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
+    for (int k = 0; k < 2; ++k) slot[k].q = s->dg_stream[k];
+    auto fdh_args = [&](const Slot& z) {
+        FdhArgs f{};
+        f.ncol = z.n;
+        f.iter = z.iter;
+        f.max_iter = max_iter;
+        f.tol = tol;
+        f.T_floor = s->T_floor;
+        f.Tb = z.Tb;
+        f.Tp = z.Tp;
+        f.dT = z.dT;
+        f.ntrop = z.ntrop;
+        f.Ed0 = z.Ed0;
+        f.Eu0 = z.Eu0;
+        f.dE0 = z.dE0;
+        f.Ed = z.Ed;
+        f.Eu = z.Eu;
+        f.dE = z.dE;
+        f.dE_jac = z.H;
+        f.iters = z.iters;
+        f.F = z.F;
+        f.Ed_out = z.Edo;
+        f.Eu_out = z.Euo;
+        f.nactive = z.count;
+        return f;
+    };
+    // the step's rt and finish kernels on the chunk's copies: E_down, E_up, dE into Ed, Eu, dE
+    auto evaluate = [&](const Slot& z, double* Ed, double* Eu, double* dE) -> int {
+        LblArgs a = z.a;
+        a.E_down = Ed;
+        a.E_up = Eu;
+        a.dE = dE;
+        CU(rcm_launch_lbl_rt(a, z.q, nullptr, nullptr));
+        CU(rcm_launch_lbl_finish(a, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // iterate z.iter: the copies at T_B + dT, their fluxes, the check, the active count into h_fdh_count[k]
+    auto check = [&](Slot& z, int k) -> int {
+        const FdhArgs f = fdh_args(z);
+        CU(rcm_launch_lbl_fdh_retemper(f, z.a.Tlayer, z.a.Tsurf, z.Ts0, z.q));
+        if ((st = evaluate(z, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
+        CU(rcm_launch_fdh_check(f, z.q));
+        CU(cudaMemcpyAsync(s->h_fdh_count + k, z.count, sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the flux Jacobian at T_B + dT (Tp, never the copy the finish has moved) and the Newton step
+    auto newton = [&](Slot& z) -> int {
+        LblArgs a = z.a;
+        a.Tlayer = z.Tp;
+        a.Tsurf = z.Ts0;
+        CU(rcm_launch_lbl_fjac(a, wtau, z.J, z.H, z.q));
+        CU(rcm_launch_fdh_newton(fdh_args(z), z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the chunk [c0, c0 + n): prep, T_B and T_surf saved, base evaluation, scaling, iterate 0
+    auto start = [&](Slot& z, int k, int c0) -> int {
+        z.c0 = c0;
+        z.n = std::min((int)ch, col0 + ncol - c0);
+        z.iter = 0;
+        z.live = true;
+        CU(cudaMemcpyAsync(z.ntrop, ntrop + (c0 - col0), z.n * sizeof(int), cudaMemcpyHostToDevice, z.q));
+        if ((st = lbl_prep(s, z.q, c0, z.n, z.state, z.lbl, nullptr, nullptr, z.a)) != RCM_OK) return st;
+        z.a.time_h = z.time;
+        z.a.part = z.part;
+        z.a.dt = z.dt;
+        CU(cudaMemcpyAsync(z.Tb, z.a.Tlayer, z.n * NLAY * D, cudaMemcpyDeviceToDevice, z.q));
+        CU(cudaMemcpyAsync(z.Ts0, z.a.Tsurf, z.n * D, cudaMemcpyDeviceToDevice, z.q));
+        if ((st = evaluate(z, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
+        if (vmr_scale) {
+            CU(rcm_launch_lbl_scale(z.a, sc.f[0], sc.f[2], z.q));
+            s->launches += 1;
         }
-        if ((st = download(z)) != RCM_OK) return st;
-        z.live = false;
-        if (next < col0 + ncol) {
-            if ((st = start(z, k, next)) != RCM_OK) return st;
-            next += (int)ch;
-        }
-    }
-    return diag_end(s);
+        if (tau3) z.a.tau3 = tau3;
+        return check(z, k);
+    };
+    auto download = [&](const Slot& z) -> int {
+        const size_t r = (size_t)(z.c0 - col0);
+        if (F) CU(cudaMemcpyAsync(F + r * 4, z.F, z.n * 4 * D, cudaMemcpyDeviceToHost, z.q));
+        if (dT_adj) CU(cudaMemcpyAsync(dT_adj + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        return RCM_OK;
+    };
+    return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -27,6 +27,7 @@
 #include "rcm_fdh.cuh"
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
+#include "rcm_lbl_fjac.cuh"
 
 __constant__ DevConst cst;
 
@@ -203,6 +204,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_fjac_kernels.cuh"
 #include "rcm_fdh_kernels.cuh"
 #include "rcm_lbl_jac_kernels.cuh"
+#include "rcm_lbl_fjac_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -523,5 +525,18 @@ cudaError_t rcm_launch_fdh_check(const FdhArgs& a, cudaStream_t st) {
 
 cudaError_t rcm_launch_fdh_newton(const FdhArgs& a, cudaStream_t st) {
     rcm_fdh_newton_kernel<<<(a.ncol + FDH_NEWTON_WARPS - 1) / FDH_NEWTON_WARPS, FDH_NEWTON_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_fjac(const LblArgs& a, double wtau, double* J, double* dE_jac, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_lbl_fjac_kernel<true> : rcm_lbl_fjac_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LBL_FJAC_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<(a.ncol + LBL_FJAC_WARPS - 1) / LBL_FJAC_WARPS, LBL_FJAC_NT, LBL_FJAC_SMEM, st>>>(a, wtau, J, dE_jac);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_fdh_retemper(const FdhArgs& f, double* T, double* Ts, const double* Ts0, cudaStream_t st) {
+    rcm_lbl_fdh_retemper_kernel<<<(f.ncol * NLAY + 255) / 256, 256, 0, st>>>(f, T, Ts, Ts0);
     return cudaGetLastError();
 }
