@@ -369,6 +369,47 @@ int rcm_lbl_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_s
  * rcm_adjusted_forcing's arguments. */
 int rcm_lbl_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, double tol,
                              int max_iter, double* F, double* dT_adj, double* E_down, double* E_up, int* iters);
+/* Equilibrium climate response of the columns [col0, col0 + ncol) to a VMR perturbation: the surface warming at fixed lapse
+ * rate and, with fixed_rh, fixed relative humidity (Manabe & Wetherald 1967), solved directly by Newton.
+ * Base and perturbed states: exactly those of rcm_adjusted_forcing for the same vmr_scale; iterate 0 is rcm_diagnose_fluxes
+ * (NULL, resp. vmr_scale) bit for bit.
+ * Unknowns: ntrop[c] in [0, 19] (required, never NULL) as there.  Each stratospheric layer l < ntrop has its own dT_l.  The
+ * troposphere and the surface share one, dTs, a uniform potential-temperature increment: layer l >= ntrop moves by
+ * dT_l = dTs / conv_l, conv_l = (1000 / p_l)^(2/7), and the surface temperature by dTs.  (The model's convective adjustment is
+ * the theta-sort and its surface temperature T_19 conv_19: a uniform increment keeps a sorted profile sorted.)
+ * Where a temperature change enters: as rcm_adjusted_forcing for the layers (Planck source and the temperature tau is
+ * interpolated at; at step 0 both the sorted and the unsorted profile), and the surface's Planck source.
+ * Water vapour: with fixed_rh != 0 every layer's H2O is re-evaluated at T + dT by the step's feedback, rel_hum x
+ * 6.1094 exp(17.625 Tc / (Tc + 243.04)) / p_l, then multiplied by the H2O factor of vmr_scale as rcm_diagnose_fluxes does
+ * (at dT = 0 bit-identical to the step's); fixed_rh needs step_index > 0, since the step applies no feedback at step 0.  With
+ * fixed_rh == 0 every VMR stays fixed (fixed absolute humidity), and step 0 is allowed.
+ * Solved for, m = ntrop + 1 equations: dE_l(perturbed, x) = dE_l(base) for l < ntrop (fixed dynamical heating), and
+ * N_k(perturbed, x) = N_k(base) at the tropopause level k = ntrop, N = E_down - E_up formed as (Ed'[k] - Eu'[k]) -
+ * (Ed[k] - Eu[k]); together the TOA net flux is unchanged (with ntrop = 0 this is the TOA balance itself).
+ * Newton matrix, re-evaluated at every iterate from rcm_flux_jacobian at that iterate: with D_i the 41 entries of row i of
+ * dE_jac (i < ntrop) resp. J_down[ntrop] - J_up[ntrop] (i = ntrop), and gamma_l = 17.625 x 243.04 / (T_l - 273.15 + 243.04)^2
+ * at T_l = T_B,l + dT_l (0 with fixed_rh == 0): A[i][j] = D_i[j] + gamma_j D_i[21 + j] for j < ntrop, and A[i][ntrop] =
+ * D_i[20] + sum_{l = ntrop}^{19} (D_i[l] + gamma_l D_i[21 + l]) / conv_l in index order.  FP64 Gaussian elimination with
+ * partial pivoting (lowest row on ties, NaN refused) as rcm_adjusted_forcing.
+ * Convergence and iters as rcm_adjusted_forcing, over all m residuals: max |residual| <= tol (W m-2); -1 for no convergence,
+ * a zero or non-finite pivot or a non-finite residual (a column with a runaway greenhouse lands there), RCM_OK all the same.
+ * Outputs (host, any may be NULL): F [ncol][2] the IRF at TOA and at the tropopause level (iterate 0; bit for bit
+ * rcm_adjusted_forcing's F[c][0..1]); dT [ncol][20] the response profile (K); dTs [ncol] the surface warming (K; for doubled
+ * CO2 the model's equilibrium climate sensitivity); E_down, E_up [ncol][21] the fluxes at the solution; iters [ncol].
+ * Every value is a function of its column alone: ranges, chunks and shards give bit-identical rows.  Synchronous; changes
+ * nothing.  Device scratch of its own: that of rcm_adjusted_forcing, 2,913 + 42 nwvl doubles and 2 ints per column of a chunk
+ * (8,192 at most) plus the tile blocks, twice.  Errors as rcm_adjusted_forcing; also RCM_ERR_STATE for fixed_rh at step 0 or
+ * without H2O among the active species.  Each error leaves the solver usable. */
+int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh, double tol,
+                         int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up, int* iters);
+/* Equilibrium climate response of the line-by-line path, as rcm_climate_response with rcm_lbl_adjusted_forcing's states: dT and
+ * dTs move the Planck sources only (LBL tau does not depend on T; no step-0 rule), with fixed_rh also s_H2O = (f_H2O x h2o) /
+ * h2o_ref at T + dT, and the Newton matrix comes from rcm_lbl_flux_jacobian.  Device scratch of its own: that of
+ * rcm_lbl_adjusted_forcing, 2,956 + 42 ceil(nwvl / 128) doubles and 12 bytes per column of a chunk, twice.  Errors as
+ * rcm_lbl_adjusted_forcing, then those of fixed_rh. */
+int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
+                             double tol, int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up,
+                             int* iters);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

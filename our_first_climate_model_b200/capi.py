@@ -526,8 +526,39 @@ class Solver:
         and results as adjusted_forcing."""
         return self._forcing(_lib.rcm_lbl_adjusted_forcing, vmr_scale, ntrop, col0, ncol, tol, max_iter)
 
-    def _forcing(self, fn, vmr_scale, ntrop, col0, ncol, tol, max_iter) -> dict:
-        """the arguments and results of the two adjusted-forcing calls around fn"""
+    def climate_response(self, vmr_scale, ntrop, fixed_rh: bool = True, col0: int = 0, ncol: int | None = None,
+                         tol: float = 1e-6, max_iter: int = 20) -> dict:
+        """rcm_climate_response: the equilibrium response to the perturbation vmr_scale for columns [col0, col0 + ncol),
+        without changing anything.  Base and perturbed states, ntrop, tol and max_iter as adjusted_forcing; the unknowns are
+        dT of the stratospheric layers 0 .. ntrop - 1 and dTs, a uniform potential-temperature increment of the troposphere
+        (dT_l = dTs / conv_l) and the surface; the equations fix the stratospheric heating rates and the net flux at the
+        tropopause.  fixed_rh: H2O follows the water-vapour feedback at T + dT (needs a step index > 0); False keeps every
+        VMR fixed.
+        -> F [ncol, 2] with the views IRF_toa, IRF_trop (W/m2), dT [ncol, 20] (K), dTs [ncol] (K, the surface warming),
+        E_down, E_up [ncol, 21] at the solution, iters [ncol] (Newton updates applied, -1: not converged) and converged."""
+        return self._response(_lib.rcm_climate_response, vmr_scale, ntrop, fixed_rh, col0, ncol, tol, max_iter)
+
+    def lbl_climate_response(self, vmr_scale, ntrop, fixed_rh: bool = True, col0: int = 0, ncol: int | None = None,
+                             tol: float = 1e-6, max_iter: int = 20) -> dict:
+        """rcm_lbl_climate_response: climate_response on the line-by-line path (the states of lbl_adjusted_forcing; dT and
+        dTs move the Planck sources, with fixed_rh also s_H2O).  Arguments and results as climate_response."""
+        return self._response(_lib.rcm_lbl_climate_response, vmr_scale, ntrop, fixed_rh, col0, ncol, tol, max_iter)
+
+    def _response(self, fn, vmr_scale, ntrop, fixed_rh, col0, ncol, tol, max_iter) -> dict:
+        """the arguments and results of the two climate-response calls around fn"""
+        n, sc, nt = self._forcing_args(vmr_scale, ntrop, col0, ncol)
+        m = max(n, 0)
+        F = np.zeros((m, 2))
+        dT, dTs = np.zeros((m, NLAY)), np.zeros(m)
+        Ed, Eu = np.zeros((m, NLEV)), np.zeros((m, NLEV))
+        it = np.zeros(m, dtype=np.int32)
+        _check(fn(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(nt), C.c_int(1 if fixed_rh else 0), C.c_double(tol),
+                  C.c_int(max_iter), _p(F), _p(dT), _p(dTs), _p(Ed), _p(Eu), _p(it)), self._h)
+        return dict(F=F, IRF_toa=F[:, 0], IRF_trop=F[:, 1], dT=dT, dTs=dTs, E_down=Ed, E_up=Eu, iters=it,
+                    converged=it >= 0)
+
+    def _forcing_args(self, vmr_scale, ntrop, col0, ncol):
+        """(ncol, vmr_scale, ntrop [ncol] int32) of the adjusted-forcing and climate-response calls"""
         n = self.ncol - col0 if ncol is None else int(ncol)
         m = max(n, 0)
         sc = self._vmr_scale(vmr_scale)
@@ -536,7 +567,12 @@ class Solver:
             nt = np.full(m, int(nt), dtype=np.int32)
         elif nt.shape != (m,):
             raise ValueError(f"ntrop needs one entry per column ({m}), got shape {nt.shape}")
-        nt = np.ascontiguousarray(nt, dtype=np.int32)
+        return n, sc, np.ascontiguousarray(nt, dtype=np.int32)
+
+    def _forcing(self, fn, vmr_scale, ntrop, col0, ncol, tol, max_iter) -> dict:
+        """the arguments and results of the two adjusted-forcing calls around fn"""
+        n, sc, nt = self._forcing_args(vmr_scale, ntrop, col0, ncol)
+        m = max(n, 0)
         F = np.zeros((m, 4))
         dT = np.zeros((m, NLAY))
         Ed, Eu = np.zeros((m, NLEV)), np.zeros((m, NLEV))

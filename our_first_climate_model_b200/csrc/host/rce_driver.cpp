@@ -13,6 +13,8 @@
 //   rcm_rce --atm fpda.lbl.atm --lbl DIR [--co2-factor F] ...     line-by-line: DIR/lbl.{h2o,co2,o3,ch4,n2o}.asc
 //           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out kernels.csv]
 //           [--lbl-jacobian-out jacobian.csv] [--lbl-forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
+//           [--response-out response.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]
+//           [--lbl-response-out response.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
 // --gpus N (N > 1): one process, one host thread and one solver per GPU, contiguous blocks of columns per GPU (tables
@@ -68,6 +70,15 @@
 // state (rcm_lbl_adjusted_forcing, tol 1e-6 W/m2, at most 20 Newton updates) for the factors --forcing-scale with the
 // --trop-layers top layers as the stratosphere, in the format of --forcing-out.  Summed in column order: the file is
 // byte-identical for any --gpus N.
+//
+// --response-out FILE (repwvl tables only): after the run, the equilibrium climate response of the next step's state
+// (rcm_climate_response, tol 1e-6 W/m2, at most 20 Newton updates) to the factors --forcing-scale with the --trop-layers top
+// layers as the stratosphere, at fixed relative humidity (--fixed-q: at fixed absolute humidity) - header "layer,p_layer,dT",
+// then one row per layer (top-down; p_layer in hPa) with the ensemble-mean response (K), then the rows "dTs,,v", "IRF_toa,,v",
+// "IRF_trop,,v" with the ensemble means (K, W/m2) and "unconverged,,n".  Summed in column order: the file is byte-identical for
+// any --gpus N.
+//
+// --lbl-response-out FILE (line-by-line tables only): the same from rcm_lbl_climate_response, in the format of --response-out.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -136,6 +147,11 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     int lbl_nband;            // > 0: --lbl-bands-out, rows [ncol][nband][4] (olr, sfc, olr scaled, sfc scaled) into B_out
     const int* lbl_bstart;    // [nband + 1]
     double* B_out;
+    int response;             // --response-out / --lbl-response-out: rcm_climate_response's (repwvl) or
+                              // rcm_lbl_climate_response's (line-by-line) F [ncol][2], dT [ncol][20], dTs [ncol], iters [ncol]
+    int fixed_rh;
+    double *RF_out, *RdT_out, *RdTs_out;
+    int* Riters_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -241,6 +257,40 @@ int write_jacobian(const std::string& path, int ncol, const double* player, cons
 
 constexpr int FORCING_MAX_ITER = 20;
 constexpr double FORCING_TOL = 1e-6;
+
+// ensemble means of the climate response, summed in column order
+int write_response(const std::string& path, int ncol, const double* player, const double* F, const double* dT, const double* dTs,
+                   const int* iters) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    constexpr int NLAY = RCM_NLAYER;
+    std::fprintf(f, "layer,p_layer,dT\n");
+    for (int l = 0; l < NLAY; ++l) {
+        double sum = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) sum += dT[c * NLAY + l];
+        std::fprintf(f, "%d,%.17g,%.17g\n", l, player[l], sum / ncol);
+    }
+    double sum = 0.0;
+    for (size_t c = 0; c < (size_t)ncol; ++c) sum += dTs[c];
+    std::fprintf(f, "dTs,,%.17g\n", sum / ncol);
+    const char* names[2] = {"IRF_toa", "IRF_trop"};
+    for (int k = 0; k < 2; ++k) {
+        double sk = 0.0;
+        for (size_t c = 0; c < (size_t)ncol; ++c) sk += F[c * 2 + k];
+        std::fprintf(f, "%s,,%.17g\n", names[k], sk / ncol);
+    }
+    int bad = 0;
+    for (size_t c = 0; c < (size_t)ncol; ++c) bad += iters[c] < 0;
+    std::fprintf(f, "unconverged,,%d\n", bad);
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
 
 // ensemble means of the adjusted forcing, summed in column order
 int write_forcing(const std::string& path, int ncol, const double* player, const double* F, const double* dT, const int* iters) {
@@ -412,6 +462,13 @@ void run_shard(Shard* sh, const Job* j) {
                                                                          nullptr, nullptr, j->iters_out + lo);
         if (st != RCM_OK) return fail(j->table ? "rcm_adjusted_forcing" : "rcm_lbl_adjusted_forcing", st);
     }
+    if (j->response) {
+        st = (j->table ? rcm_climate_response : rcm_lbl_climate_response)(sh->s, 0, (int)n, j->forcing_scale, j->ntrop + lo, j->fixed_rh,
+                                                                         FORCING_TOL, FORCING_MAX_ITER, j->RF_out + lo * 2,
+                                                                         j->RdT_out + lo * NLAY, j->RdTs_out + lo, nullptr, nullptr,
+                                                                         j->Riters_out + lo);
+        if (st != RCM_OK) return fail(j->table ? "rcm_climate_response" : "rcm_lbl_climate_response", st);
+    }
     if (j->lbl_nband > 0) {
         st = diagnose_lbl_bands(sh->s, (int)n, j->lbl_nband, j->lbl_bstart, j->forcing_scale, j->B_out + lo * j->lbl_nband * 4);
         if (st != RCM_OK) return fail("rcm_lbl_diagnose_fluxes", st);
@@ -423,9 +480,9 @@ void run_shard(Shard* sh, const Job* j) {
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
         jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100",
-        lbl_kernels_path, lbl_jacobian_path, lbl_forcing_path;
+        lbl_kernels_path, lbl_jacobian_path, lbl_forcing_path, response_path, lbl_response_path;
     double co2_factor = 1.0;
-    int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1;
+    int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1, fixed_rh = 1;
     long max_steps = 6000;
     unsigned long long seed = 12345;
     double dT = 1e-3;
@@ -458,6 +515,9 @@ int main(int argc, char** argv) {
         else if (a == "--lbl-kernels-out") lbl_kernels_path = val();
         else if (a == "--lbl-jacobian-out") lbl_jacobian_path = val();
         else if (a == "--lbl-forcing-out") lbl_forcing_path = val();
+        else if (a == "--response-out") response_path = val();
+        else if (a == "--lbl-response-out") lbl_response_path = val();
+        else if (a == "--fixed-q") fixed_rh = 0;
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -470,7 +530,9 @@ int main(int argc, char** argv) {
                              "[--spectral-out FILE] [--kernels-out FILE] [--jacobian-out FILE] "
                              "[--forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
                              "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out FILE] "
-                             "[--lbl-jacobian-out FILE] [--lbl-forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]\n");
+                             "[--lbl-jacobian-out FILE] [--lbl-forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
+                             "[--response-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]] "
+                             "[--lbl-response-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -504,6 +566,15 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (!lbl_forcing_path.empty()) forcing_path = lbl_forcing_path;  // the same forcing file, from the LBL call
+    if (!lbl_dir.empty() && !response_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --response-out needs a repwvl table (--table): with --lbl use --lbl-response-out\n");
+        return 1;
+    }
+    if (lbl_dir.empty() && !lbl_response_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-response-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
+    if (!lbl_response_path.empty()) response_path = lbl_response_path;  // the same response file, from the LBL call
     if (lbl_dir.empty() && !bands_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --lbl-bands-out needs line-by-line tables (--lbl)\n");
         return 1;
@@ -525,7 +596,7 @@ int main(int argc, char** argv) {
         }
         band_size = (int)bs;
     }
-    if (!forcing_path.empty()) {  // --forcing-scale: exactly five numbers; --trop-layers: one integer in [0, 19]
+    if (!forcing_path.empty() || !response_path.empty()) {  // --forcing-scale: five numbers; --trop-layers: an integer in [0, 19]
         int k = 0;
         const char* q = forcing_scale_arg.c_str();
         for (char* e = nullptr; k < 5; ++k, q = e + 1) {
@@ -627,13 +698,17 @@ int main(int argc, char** argv) {
         const bool forcing = !forcing_path.empty();
         std::vector<double> Ff(forcing ? n * 4 : 0), dTf(forcing ? n * NLAY : 0);
         std::vector<int> itf(forcing ? n : 0), ntrop(n, trop_layers);
+        const bool response = !response_path.empty();
+        std::vector<double> Fr(response ? n * 2 : 0), dTr(response ? n * NLAY : 0), dTsr(response ? n : 0);
+        std::vector<int> itr(response ? n : 0);
         const std::vector<int> bstart = bands_path.empty() ? std::vector<int>() : lbl_band_starts(nwvl, band_size);
         const int nband = bands_path.empty() ? 0 : (int)bstart.size() - 1;
         std::vector<double> B(n * nband * 4);
         Job job{&p, table, &wvl, &tau5, nwvl, co2_factor, plevel, Tlayer.data(), Tsurf.data(), vmr9.data(), rel_hum.data(), ncol,
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
                 dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data(),
-                forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data(), nband, bstart.data(), B.data()};
+                forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data(), nband, bstart.data(), B.data(),
+                response, fixed_rh, Fr.data(), dTr.data(), dTsr.data(), itr.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -680,6 +755,10 @@ int main(int argc, char** argv) {
             return 1;
         }
         if (forcing && write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
+        if (response && write_response(response_path, ncol, player.data(), Fr.data(), dTr.data(), dTsr.data(), itr.data())) {
             rcm_table_free(table);
             return 1;
         }
@@ -817,6 +896,15 @@ int main(int argc, char** argv) {
                                                                     FORCING_MAX_ITER, Ff.data(), dTf.data(), nullptr, nullptr, itf.data());
         if (st != RCM_OK) return die(lbl ? "rcm_lbl_adjusted_forcing" : "rcm_adjusted_forcing", st, s);
         if (write_forcing(forcing_path, ncol, player.data(), Ff.data(), dTf.data(), itf.data())) return 1;
+    }
+    if (!response_path.empty()) {
+        std::vector<double> Fr(m * 2), dTr(m * NLAY), dTsr(m);
+        std::vector<int> itr(m), ntrop(m, trop_layers);
+        st = (lbl ? rcm_lbl_climate_response : rcm_climate_response)(s, 0, ncol, forcing_scale, ntrop.data(), fixed_rh, FORCING_TOL,
+                                                                    FORCING_MAX_ITER, Fr.data(), dTr.data(), dTsr.data(), nullptr,
+                                                                    nullptr, itr.data());
+        if (st != RCM_OK) return die(lbl ? "rcm_lbl_climate_response" : "rcm_climate_response", st, s);
+        if (write_response(response_path, ncol, player.data(), Fr.data(), dTr.data(), dTsr.data(), itr.data())) return 1;
     }
     if (!bands_path.empty()) {
         const std::vector<int> bstart = lbl_band_starts((int)lbl_wvl.size(), band_size);

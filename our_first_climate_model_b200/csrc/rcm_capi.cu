@@ -13,6 +13,7 @@
 
 #include "rcm_jac.cuh"
 #include "rcm_fdh.cuh"
+#include "rcm_ecs.cuh"
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
@@ -2364,6 +2365,322 @@ int rcm_lbl_adjusted_forcing(rcm_solver* s, int col0, int ncol, const double* vm
         const size_t r = (size_t)(z.c0 - col0);
         if (F) CU(cudaMemcpyAsync(F + r * 4, z.F, z.n * 4 * D, cudaMemcpyDeviceToHost, z.q));
         if (dT_adj) CU(cudaMemcpyAsync(dT_adj + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        return RCM_OK;
+    };
+    return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
+}
+
+extern "C++" {
+namespace {
+
+// the checks both climate-response calls make after fdh_check_args
+int ecs_check_args(rcm_solver* s, const std::string& fn, int fixed_rh) {
+    if (fixed_rh && s->h2o_slot < 0) return fail(s, RCM_ERR_STATE, fn + ": fixed relative humidity needs H2O among the active species");
+    if (fixed_rh && s->step_index == 0)
+        return fail(s, RCM_ERR_STATE, fn + ": fixed relative humidity needs a step index > 0 (the step applies no feedback at step 0)");
+    return RCM_OK;
+}
+
+}  // namespace
+}  // extern "C++"
+
+// Equilibrium climate response: rcm_adjusted_forcing's scratch sets, streams, prep, base evaluation, scaling and Newton schedule
+// (fdh_schedule) with one more unknown per column, the uniform potential-temperature increment dTs of the troposphere and the
+// surface.  Per iterate: rcm_ecs_retemper_kernel (tile blocks at T + dT and Ts + dTs, with fixed RH the H2O row), the
+// evaluation and rcm_ecs_check_kernel; while columns are active, the flux Jacobian (rcm_fjac_kernel at T + dT, Ts + dTs) and
+// rcm_ecs_newton_kernel.
+int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh, double tol,
+                         int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up, int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_climate_response";
+    DiagScale sc{};
+    int st = diag_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, fn + ": needs H2O among the active species");
+    if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
+    if ((st = ecs_check_args(s, fn, fixed_rh)) != RCM_OK) return st;
+    const int nwvl = s->dc.nwvl;
+    const bool first = (s->step_index == 0);
+    const size_t ch = diag_chunk(ncol), D = sizeof(double);
+    struct Slot {
+        cudaStream_t q;
+        int c0 = 0, n = 0, iter = 0;
+        bool live = false;
+        DiagState state;
+        double *Ttau, *Tp, *dT, *Tsp, *dTs, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *spec_dn, *spec_up;
+        int *ntrop, *iters, *count;
+        SplitArgs a;
+    } slot[2];
+    // T_tau, T + dT, dT [ch][20], Ts + dTs, dTs [ch], E_down, E_up [ch][21] and dE [ch][20] of the base and of the current
+    // iterate, F [ch][2], the output E_down, E_up [ch][21], J [ch][2][21][41], dE_jac [ch][20][41], spectral [2][ch][nwvl][21];
+    // ntrop, iters [ch] and the active count
+    st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
+        z.Ttau = m.take<double>(ch * NLAY);
+        z.Tp = m.take<double>(ch * NLAY);
+        z.dT = m.take<double>(ch * NLAY);
+        z.Tsp = m.take<double>(ch);
+        z.dTs = m.take<double>(ch);
+        z.Ed0 = m.take<double>(ch * NLEV);
+        z.Eu0 = m.take<double>(ch * NLEV);
+        z.dE0 = m.take<double>(ch * NLAY);
+        z.Ed = m.take<double>(ch * NLEV);
+        z.Eu = m.take<double>(ch * NLEV);
+        z.dE = m.take<double>(ch * NLAY);
+        z.F = m.take<double>(ch * 2);
+        z.Edo = m.take<double>(ch * NLEV);
+        z.Euo = m.take<double>(ch * NLEV);
+        z.J = m.take<double>(ch * FJAC_NJ);
+        z.H = m.take<double>(ch * FJAC_NH);
+        z.spec_dn = m.take<double>(ch * nwvl * NLEV);
+        z.spec_up = m.take<double>(ch * nwvl * NLEV);
+        z.ntrop = m.take<int>(ch);
+        z.iters = m.take<int>(ch);
+        z.count = m.take<int>(1);
+    });
+    if (st != RCM_OK) return st;
+    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
+    for (int k = 0; k < 2; ++k) slot[k].q = s->dg_stream[k];
+    auto ecs_args = [&](const Slot& z) {
+        EcsArgs e{};
+        e.ncol = z.n;
+        e.iter = z.iter;
+        e.max_iter = max_iter;
+        e.fixed_rh = fixed_rh != 0;
+        e.tol = tol;
+        e.T_floor = s->T_floor;
+        e.f_h2o = sc.f[0];
+        e.tile = z.state.tile;
+        e.Tb = z.state.T;
+        e.Ttau = first ? z.Ttau : z.state.T;
+        e.Ts0 = z.a.Tsurf;
+        e.rel_hum = z.a.rel_hum;
+        e.Tp = z.Tp;
+        e.Tsp = z.Tsp;
+        e.dT = z.dT;
+        e.dTs = z.dTs;
+        e.ntrop = z.ntrop;
+        e.Ed0 = z.Ed0;
+        e.Eu0 = z.Eu0;
+        e.dE0 = z.dE0;
+        e.Ed = z.Ed;
+        e.Eu = z.Eu;
+        e.dE = z.dE;
+        e.J = z.J;
+        e.dE_jac = z.H;
+        e.iters = z.iters;
+        e.F = z.F;
+        e.Ed_out = z.Edo;
+        e.Eu_out = z.Euo;
+        e.nactive = z.count;
+        return e;
+    };
+    // iterate z.iter: the tile blocks at T + dT, Ts + dTs, their fluxes, the check, the active count into h_fdh_count[k]
+    auto check = [&](Slot& z, int k) -> int {
+        const EcsArgs e = ecs_args(z);
+        CU(rcm_launch_ecs_retemper(e, z.q));
+        if ((st = diag_fluxes(s, z.a, z.q, z.spec_dn, z.spec_up, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
+        CU(rcm_launch_ecs_check(e, z.q));
+        CU(cudaMemcpyAsync(s->h_fdh_count + k, z.count, sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the flux Jacobian at T + dT, Ts + dTs and the Newton step
+    auto newton = [&](Slot& z) -> int {
+        SplitArgs a = z.a;
+        a.Tsurf = z.Tsp;
+        if ((st = flux_jacobian(s, a, z.q, z.Tp, z.J, z.H)) != RCM_OK) return st;
+        CU(rcm_launch_ecs_newton(ecs_args(z), z.q));
+        s->launches += 1;
+        return RCM_OK;
+    };
+    // the chunk [c0, c0 + n): T_tau, prep, base evaluation, scaling, iterate 0
+    auto start = [&](Slot& z, int k, int c0) -> int {
+        z.c0 = c0;
+        z.n = std::min((int)ch, col0 + ncol - c0);
+        z.iter = 0;
+        z.live = true;
+        if (first) CU(cudaMemcpyAsync(z.Ttau, s->d_T + (size_t)c0 * NLAY, z.n * NLAY * D, cudaMemcpyDeviceToDevice, z.q));
+        CU(cudaMemcpyAsync(z.ntrop, ntrop + (c0 - col0), z.n * sizeof(int), cudaMemcpyHostToDevice, z.q));
+        if ((st = diag_prep(s, z.q, c0, z.n, z.state, nullptr, z.a)) != RCM_OK) return st;
+        if ((st = diag_fluxes(s, z.a, z.q, z.spec_dn, z.spec_up, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
+        if (vmr_scale) {
+            CU(rcm_launch_diag_scale(z.state.tile, z.a.ntiles, sc, z.q));
+            s->launches += 1;
+        }
+        return check(z, k);
+    };
+    auto download = [&](const Slot& z) -> int {
+        const size_t r = (size_t)(z.c0 - col0);
+        if (F) CU(cudaMemcpyAsync(F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
+        if (dT) CU(cudaMemcpyAsync(dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (dTs) CU(cudaMemcpyAsync(dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        return RCM_OK;
+    };
+    return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
+}
+
+// Line-by-line equilibrium climate response: rcm_lbl_adjusted_forcing's chunks, prep, saved T_B and T_surf, base evaluation,
+// scaling and Newton schedule; per iterate rcm_lbl_ecs_retemper_kernel (every copy back to T_B + dT, T_surf + dTs, with fixed
+// RH s_H2O at T_B + dT), the evaluation and rcm_ecs_check_kernel; while columns are active, rcm_lbl_fjac_kernel at
+// T_B + dT, T_surf + dTs and rcm_ecs_newton_kernel.
+int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
+                             double tol, int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up,
+                             int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_climate_response";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
+    if ((st = ecs_check_args(s, fn, fixed_rh)) != RCM_OK) return st;
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const size_t ch = diag_chunk(ncol), D = sizeof(double);
+    const size_t nchunks = (size_t)lbl_args(s, 0).nchunks;
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    struct Slot {
+        cudaStream_t q;
+        int c0 = 0, n = 0, iter = 0;
+        bool live = false;
+        DiagState state;
+        LblState lbl;
+        double *Tb, *Ts0, *Tp, *dT, *Tsp, *dTs, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *part, *dt;
+        float* time;
+        int *ntrop, *iters, *count;
+        LblArgs a;
+    } slot[2];
+    // the prep's T_surf, sH, sO; T_B, T_surf as prepared, T_B + dT, dT [ch][20], T_surf + dTs, dTs [ch]; E_down, E_up [ch][21]
+    // and dE [ch][20] of the base and of the current iterate, F [ch][2], the output E_down, E_up [ch][21], J [ch][2][21][41],
+    // dE_jac [ch][20][41], the rt kernel's partials [nchunks][ch][42], the finish's dt and time [ch]; ntrop, iters [ch] and the
+    // active count
+    st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
+        lbl_take(m, ch, z.lbl);
+        z.Tb = m.take<double>(ch * NLAY);
+        z.Ts0 = m.take<double>(ch);
+        z.Tp = m.take<double>(ch * NLAY);
+        z.dT = m.take<double>(ch * NLAY);
+        z.Tsp = m.take<double>(ch);
+        z.dTs = m.take<double>(ch);
+        z.Ed0 = m.take<double>(ch * NLEV);
+        z.Eu0 = m.take<double>(ch * NLEV);
+        z.dE0 = m.take<double>(ch * NLAY);
+        z.Ed = m.take<double>(ch * NLEV);
+        z.Eu = m.take<double>(ch * NLEV);
+        z.dE = m.take<double>(ch * NLAY);
+        z.F = m.take<double>(ch * 2);
+        z.Edo = m.take<double>(ch * NLEV);
+        z.Euo = m.take<double>(ch * NLEV);
+        z.J = m.take<double>(ch * FJAC_NJ);
+        z.H = m.take<double>(ch * FJAC_NH);
+        z.part = m.take<double>(nchunks * ch * 2 * NLEV);
+        z.dt = m.take<double>(ch);
+        z.time = m.take<float>(ch);
+        z.ntrop = m.take<int>(ch);
+        z.iters = m.take<int>(ch);
+        z.count = m.take<int>(1);
+    }, false);
+    if (st != RCM_OK) return st;
+    if (!s->h_fdh_count) CU(cudaMallocHost((void**)&s->h_fdh_count, 2 * sizeof(int)));
+    for (int k = 0; k < 2; ++k) slot[k].q = s->dg_stream[k];
+    auto ecs_args = [&](const Slot& z) {
+        EcsArgs e{};
+        e.ncol = z.n;
+        e.iter = z.iter;
+        e.max_iter = max_iter;
+        e.fixed_rh = fixed_rh != 0;
+        e.tol = tol;
+        e.T_floor = s->T_floor;
+        e.f_h2o = sc.f[0];
+        e.Tb = z.Tb;
+        e.Ts0 = z.Ts0;
+        e.rel_hum = z.a.rel_hum;
+        e.Tp = z.Tp;
+        e.Tsp = z.Tsp;
+        e.dT = z.dT;
+        e.dTs = z.dTs;
+        e.T = z.a.Tlayer;
+        e.Ts = z.a.Tsurf;
+        e.sH = z.a.sH;
+        e.h2o_ref = z.a.h2o_ref;
+        e.ntrop = z.ntrop;
+        e.Ed0 = z.Ed0;
+        e.Eu0 = z.Eu0;
+        e.dE0 = z.dE0;
+        e.Ed = z.Ed;
+        e.Eu = z.Eu;
+        e.dE = z.dE;
+        e.J = z.J;
+        e.dE_jac = z.H;
+        e.iters = z.iters;
+        e.F = z.F;
+        e.Ed_out = z.Edo;
+        e.Eu_out = z.Euo;
+        e.nactive = z.count;
+        return e;
+    };
+    // the step's rt and finish kernels on the chunk's copies: E_down, E_up, dE into Ed, Eu, dE
+    auto evaluate = [&](const Slot& z, double* Ed, double* Eu, double* dE) -> int {
+        LblArgs a = z.a;
+        a.E_down = Ed;
+        a.E_up = Eu;
+        a.dE = dE;
+        CU(rcm_launch_lbl_rt(a, z.q, nullptr, nullptr));
+        CU(rcm_launch_lbl_finish(a, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // iterate z.iter: the copies at T_B + dT, T_surf + dTs, their fluxes, the check, the active count into h_fdh_count[k]
+    auto check = [&](Slot& z, int k) -> int {
+        const EcsArgs e = ecs_args(z);
+        CU(rcm_launch_lbl_ecs_retemper(e, z.q));
+        if ((st = evaluate(z, z.Ed, z.Eu, z.dE)) != RCM_OK) return st;
+        CU(rcm_launch_ecs_check(e, z.q));
+        CU(cudaMemcpyAsync(s->h_fdh_count + k, z.count, sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the flux Jacobian at T_B + dT, T_surf + dTs (Tp, Tsp: never the copies the finish has moved) and the Newton step
+    auto newton = [&](Slot& z) -> int {
+        LblArgs a = z.a;
+        a.Tlayer = z.Tp;
+        a.Tsurf = z.Tsp;
+        CU(rcm_launch_lbl_fjac(a, wtau, z.J, z.H, z.q));
+        CU(rcm_launch_ecs_newton(ecs_args(z), z.q));
+        s->launches += 2;
+        return RCM_OK;
+    };
+    // the chunk [c0, c0 + n): prep, T_B and T_surf saved, base evaluation, scaling, iterate 0
+    auto start = [&](Slot& z, int k, int c0) -> int {
+        z.c0 = c0;
+        z.n = std::min((int)ch, col0 + ncol - c0);
+        z.iter = 0;
+        z.live = true;
+        CU(cudaMemcpyAsync(z.ntrop, ntrop + (c0 - col0), z.n * sizeof(int), cudaMemcpyHostToDevice, z.q));
+        if ((st = lbl_prep(s, z.q, c0, z.n, z.state, z.lbl, nullptr, nullptr, z.a)) != RCM_OK) return st;
+        z.a.time_h = z.time;
+        z.a.part = z.part;
+        z.a.dt = z.dt;
+        CU(cudaMemcpyAsync(z.Tb, z.a.Tlayer, z.n * NLAY * D, cudaMemcpyDeviceToDevice, z.q));
+        CU(cudaMemcpyAsync(z.Ts0, z.a.Tsurf, z.n * D, cudaMemcpyDeviceToDevice, z.q));
+        if ((st = evaluate(z, z.Ed0, z.Eu0, z.dE0)) != RCM_OK) return st;
+        if (vmr_scale) {
+            CU(rcm_launch_lbl_scale(z.a, sc.f[0], sc.f[2], z.q));
+            s->launches += 1;
+        }
+        if (tau3) z.a.tau3 = tau3;
+        return check(z, k);
+    };
+    auto download = [&](const Slot& z) -> int {
+        const size_t r = (size_t)(z.c0 - col0);
+        if (F) CU(cudaMemcpyAsync(F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
+        if (dT) CU(cudaMemcpyAsync(dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (dTs) CU(cudaMemcpyAsync(dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
         if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
         if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
         if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));

@@ -25,6 +25,7 @@
 #include "rcm_jac.cuh"
 #include "rcm_fjac.cuh"
 #include "rcm_fdh.cuh"
+#include "rcm_ecs.cuh"
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
@@ -205,6 +206,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_fdh_kernels.cuh"
 #include "rcm_lbl_jac_kernels.cuh"
 #include "rcm_lbl_fjac_kernels.cuh"
+#include "rcm_ecs_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -538,5 +540,25 @@ cudaError_t rcm_launch_lbl_fjac(const LblArgs& a, double wtau, double* J, double
 
 cudaError_t rcm_launch_lbl_fdh_retemper(const FdhArgs& f, double* T, double* Ts, const double* Ts0, cudaStream_t st) {
     rcm_lbl_fdh_retemper_kernel<<<(f.ncol * NLAY + 255) / 256, 256, 0, st>>>(f, T, Ts, Ts0);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_ecs_retemper(const EcsArgs& a, cudaStream_t st) {
+    rcm_ecs_retemper_kernel<<<(a.ncol * NLAY + 255) / 256, 256, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_ecs_retemper(const EcsArgs& a, cudaStream_t st) {
+    rcm_lbl_ecs_retemper_kernel<<<(a.ncol * NLAY + 255) / 256, 256, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_ecs_check(const EcsArgs& a, cudaStream_t st) {
+    rcm_ecs_check_kernel<<<(a.ncol + FDH_CHECK_NT - 1) / FDH_CHECK_NT, FDH_CHECK_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_ecs_newton(const EcsArgs& a, cudaStream_t st) {
+    rcm_ecs_newton_kernel<<<(a.ncol + ECS_NEWTON_WARPS - 1) / ECS_NEWTON_WARPS, ECS_NEWTON_NT, 0, st>>>(a);
     return cudaGetLastError();
 }
