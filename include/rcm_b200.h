@@ -410,6 +410,32 @@ int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_sc
 int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
                              double tol, int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up,
                              int* iters);
+/* Species Jacobians of the columns [col0, col0 + ncol): analytic derivatives of every level's broadband E_down and E_up of the
+ * NEXT step (summed over the wavelengths in index order) and of its heating rates with respect to the ln VMR of each of the five
+ * species in each layer, at exactly the state rcm_flux_jacobian differentiates for the same arguments (sort, water-vapour
+ * feedback, grey or per-column cloud, step-0 rule, vmr_scale applied as there).
+ * Entries [100]: e = 20 s + l, s in ascending species index as vmr_scale (0 H2O, 1 CO2, 2 O3, 3 N2O, 4 CH4), layers l top-down;
+ * entry e is d/d ln x_{s,l}, x_{s,l} the VMR of species s in layer l as the step uses it (W m-2 per unit ln x), at fixed T:
+ * no re-sort, no feedback.  dtau_l/dln x_{s,l} is species s's own term of the step's optical depth, numDens_l x (its three-FMA
+ * K1 term at layer l) x x_{s,l}; the entry is 0.0 where the tau clamp or floor acts and where x_{s,l} = 0.
+ * Outputs (host, either may be NULL; both NULL: RCM_OK without work): J [ncol][2][21][100], J[c][0][k][e] = dE_down[k]/dx_e
+ * and J[c][1][k][e] = dE_up[k]/dx_e; dE_jac [ncol][20][100] from J entry by entry as dE from E (main.cpp:337-341).  Structural
+ * zeros those of the ln q entries of rcm_flux_jacobian: dE_down[k]/dx_{s,l} for l >= k, dE_up[k]/dx_{s,l} for l < k.  The
+ * H2O block (e = 0..19) equals rcm_flux_jacobian's entries 21..40 bit for bit.  Linearised, the change of the fluxes for a
+ * profile perturbation of any species is sum_e J[.][e] dln x_e.  Every value is a function of its column alone: ranges, chunks
+ * and shards give bit-identical rows.  Synchronous; changes nothing.  Device scratch of its own: two sets for chunks of at
+ * most 8,192 columns, each of 6,341 doubles per column plus the tile blocks (about 0.9 GB).  Errors as rcm_flux_jacobian;
+ * also RCM_ERR_STATE with any species_mask other than the default 0x2F.  Each leaves the solver usable. */
+int rcm_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
+/* Species Jacobians of the line-by-line path: rcm_species_jacobian's entries, outputs, structural zeros and properties at the
+ * state rcm_lbl_flux_jacobian differentiates for the same arguments.  dtau_l/dln x_{s,l} is species s's share of tau_l as
+ * rcm_lbl_diagnose_fluxes composes it, one rounded product each: tau_H2O,l x s_H2O,l; (f_CO2 x co2_factor) x tau_CO2,l;
+ * tau_O3,l x s_O3,l; f_N2O x tau_N2O,l; f_CH4 x tau_CH4,l; 0.0 where the tau clamp acts.  The H2O block equals
+ * rcm_lbl_flux_jacobian's entries 21..40 bit for bit.  Device scratch of its own: two sets for chunks of at most 8,192
+ * columns, each of 6,382 doubles per column (about 0.84 GB, independent of the wavelengths); with CO2, CH4 or N2O scaled also
+ * the 3 x nwvl x 20 doubles of rcm_lbl_diagnose_fluxes.  Errors as rcm_lbl_flux_jacobian; also RCM_ERR_STATE with any
+ * species_mask other than the default 0x2F.  Each leaves the solver usable. */
+int rcm_lbl_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

@@ -519,6 +519,35 @@ class Solver:
         _check(_lib.rcm_lbl_flux_jacobian(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(J), _p(H)), self._h)
         return dict(J=J, dE_jac=H)
 
+    SPECIES = ("h2o", "co2", "o3", "n2o", "ch4")   # the species of the species Jacobians' entries, in the order of vmr_scale
+
+    def species_jacobian(self, col0: int = 0, ncol: int | None = None, vmr_scale=None) -> dict:
+        """rcm_species_jacobian: derivatives of the next step's broadband fluxes at every level and of its heating rates with
+        respect to each species' ln VMR in each layer, for columns [col0, col0 + ncol), at the state flux_jacobian
+        differentiates, without changing anything.  vmr_scale as in diagnose_fluxes.  Entry e = 20 s + l: d/dln x of species
+        s (h2o, co2, o3, n2o, ch4) in layer l (top-down), at fixed T.
+        -> J [ncol, 2, 21, 100] (J[:, 0, k] = dE_down[k], J[:, 1, k] = dE_up[k]), dE_jac [ncol, 20, 100] and the views
+        J_h2o, J_co2, J_o3, J_n2o, J_ch4 [ncol, 2, 21, 20]."""
+        return self._species_jacobian(_lib.rcm_species_jacobian, col0, ncol, vmr_scale)
+
+    def lbl_species_jacobian(self, col0: int = 0, ncol: int | None = None, vmr_scale=None) -> dict:
+        """rcm_lbl_species_jacobian: species_jacobian on the line-by-line path, at the state lbl_flux_jacobian
+        differentiates.  vmr_scale as in lbl_diagnose_fluxes; outputs as in species_jacobian."""
+        return self._species_jacobian(_lib.rcm_lbl_species_jacobian, col0, ncol, vmr_scale)
+
+    def _species_jacobian(self, fn, col0, ncol, vmr_scale) -> dict:
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = self._vmr_scale(vmr_scale)
+        m = max(n, 0)
+        ne = len(self.SPECIES) * NLAY
+        J = np.zeros((m, 2, NLEV, ne))
+        H = np.zeros((m, NLAY, ne))
+        _check(fn(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(J), _p(H)), self._h)
+        out = dict(J=J, dE_jac=H)
+        for s, name in enumerate(self.SPECIES):
+            out[f"J_{name}"] = J[..., s * NLAY:(s + 1) * NLAY]
+        return out
+
     def lbl_adjusted_forcing(self, vmr_scale, ntrop, col0: int = 0, ncol: int | None = None, tol: float = 1e-6,
                              max_iter: int = 20) -> dict:
         """rcm_lbl_adjusted_forcing: adjusted_forcing on the line-by-line path (base state: what lbl_diagnose_fluxes

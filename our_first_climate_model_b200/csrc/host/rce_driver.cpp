@@ -14,6 +14,7 @@
 //           [--lbl-bands-out bands.csv [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out kernels.csv]
 //           [--lbl-jacobian-out jacobian.csv] [--lbl-forcing-out forcing.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4]]
 //           [--response-out response.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]
+//           [--species-jacobian-out species.csv] [--lbl-species-jacobian-out species.csv]
 //           [--lbl-response-out response.csv [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]
 //   rcm_rce ... --gpus N                                          the same ensemble sharded over N GPUs of this node
 //
@@ -79,6 +80,14 @@
 // any --gpus N.
 //
 // --lbl-response-out FILE (line-by-line tables only): the same from rcm_lbl_climate_response, in the format of --response-out.
+//
+// --species-jacobian-out FILE (repwvl tables only): after the run, the layer-resolved species kernels of the next step
+// (rcm_species_jacobian) - header "species,layer,p_layer,dOLR_dlnx,dSFC_dlnx,dHeat_dlnx", then one row per species (h2o, co2,
+// o3, n2o, ch4) and layer (top-down; p_layer in hPa) with the ensemble means of the derivatives of the OLR, of the surface
+// downward flux and of the layer's own heating rate dE_l with respect to ln of the species' VMR in that layer (W/m2).  Summed
+// in column order: the file is byte-identical for any --gpus N.
+//
+// --lbl-species-jacobian-out FILE (line-by-line tables only): the same from rcm_lbl_species_jacobian.
 //
 // --steps-exact runs exactly max_steps iterations (the reference's n_steps semantics, main.cpp:83) instead of
 // stopping at stationarity.  Exit code 0, or 1 with the library's error text on stderr.  No CPU fallback.
@@ -152,6 +161,8 @@ struct Job {  // what every shard needs; host arrays cover the WHOLE ensemble
     int fixed_rh;
     double *RF_out, *RdT_out, *RdTs_out;
     int* Riters_out;
+    int species;              // --species-jacobian-out / --lbl-species-jacobian-out: rows [ncol][3][100] of species_rows into S_out
+    double* S_out;
 };
 
 std::atomic<int> g_failed{0};
@@ -244,6 +255,54 @@ int write_jacobian(const std::string& path, int ncol, const double* player, cons
         for (int e = 0; e < KERN_NE; ++e) {
             double sum = 0.0;
             for (size_t c = 0; c < (size_t)ncol; ++c) sum += H[c * JAC_NH + l * KERN_NE + e];
+            std::fprintf(f, ",%.17g", sum / ncol);
+        }
+        std::fprintf(f, "\n");
+    }
+    if (std::fclose(f) != 0) {
+        std::fprintf(stderr, "rcm_rce: short write to %s\n", path.c_str());
+        return 1;
+    }
+    return 0;
+}
+
+constexpr int SPJ_NE = 5 * RCM_NLAYER, SPJ_NJ = 2 * RCM_NLEVEL * SPJ_NE, SPJ_NH = RCM_NLAYER * SPJ_NE;  // rcm_species_jacobian
+
+// rows [n][3][100] of the n columns of s from rcm_species_jacobian (repwvl) or rcm_lbl_species_jacobian (line-by-line): per entry
+// e = 20 s + l, dE_up[0]/dx_e, dE_down[20]/dx_e and d dE_l/dx_e, the layer's own heating rate
+int species_rows(rcm_solver* s, bool lbl, int n, double* R) {
+    constexpr int NLAY = RCM_NLAYER, NLEV = RCM_NLEVEL, CHUNK = 1024;
+    std::vector<double> J((size_t)std::min(n, CHUNK) * SPJ_NJ), H((size_t)std::min(n, CHUNK) * SPJ_NH);
+    for (int c0 = 0; c0 < n; c0 += CHUNK) {
+        const int m = std::min(CHUNK, n - c0);
+        const int st = (lbl ? rcm_lbl_species_jacobian : rcm_species_jacobian)(s, c0, m, nullptr, J.data(), H.data());
+        if (st != RCM_OK) return st;
+        for (size_t c = 0; c < (size_t)m; ++c)
+            for (int e = 0; e < SPJ_NE; ++e) {
+                double* r = R + (c0 + c) * 3 * SPJ_NE + e;
+                r[0] = J[c * SPJ_NJ + (size_t)(NLEV + 0) * SPJ_NE + e];     // E_up[0]
+                r[SPJ_NE] = J[c * SPJ_NJ + (size_t)(NLEV - 1) * SPJ_NE + e];  // E_down[20]
+                r[2 * SPJ_NE] = H[c * SPJ_NH + (size_t)(e % NLAY) * SPJ_NE + e];
+            }
+    }
+    return RCM_OK;
+}
+
+// ensemble means of the species rows, summed in column order
+int write_species(const std::string& path, int ncol, const double* player, const double* R) {
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) {
+        std::fprintf(stderr, "rcm_rce: cannot write %s\n", path.c_str());
+        return 1;
+    }
+    constexpr int NLAY = RCM_NLAYER;
+    const char* names[5] = {"h2o", "co2", "o3", "n2o", "ch4"};  // ascending species index, the entries' order
+    std::fprintf(f, "species,layer,p_layer,dOLR_dlnx,dSFC_dlnx,dHeat_dlnx\n");
+    for (int e = 0; e < SPJ_NE; ++e) {
+        std::fprintf(f, "%s,%d,%.17g", names[e / NLAY], e % NLAY, player[e % NLAY]);
+        for (int o = 0; o < 3; ++o) {
+            double sum = 0.0;
+            for (size_t c = 0; c < (size_t)ncol; ++c) sum += R[(c * 3 + o) * SPJ_NE + e];
             std::fprintf(f, ",%.17g", sum / ncol);
         }
         std::fprintf(f, "\n");
@@ -469,6 +528,10 @@ void run_shard(Shard* sh, const Job* j) {
                                                                          j->Riters_out + lo);
         if (st != RCM_OK) return fail(j->table ? "rcm_climate_response" : "rcm_lbl_climate_response", st);
     }
+    if (j->species) {
+        st = species_rows(sh->s, !j->table, (int)n, j->S_out + lo * 3 * SPJ_NE);
+        if (st != RCM_OK) return fail(j->table ? "rcm_species_jacobian" : "rcm_lbl_species_jacobian", st);
+    }
     if (j->lbl_nband > 0) {
         st = diagnose_lbl_bands(sh->s, (int)n, j->lbl_nband, j->lbl_bstart, j->forcing_scale, j->B_out + lo * j->lbl_nband * 4);
         if (st != RCM_OK) return fail("rcm_lbl_diagnose_fluxes", st);
@@ -480,7 +543,7 @@ void run_shard(Shard* sh, const Job* j) {
 int main(int argc, char** argv) {
     std::string atm_path, table_path, lbl_dir, out_path = "output.txt", ckpt_path, resume_path, spectral_path, kernels_path,
         jacobian_path, forcing_path, forcing_scale_arg = "1,2,1,1,1", trop_layers_arg = "4", bands_path, band_size_arg = "100",
-        lbl_kernels_path, lbl_jacobian_path, lbl_forcing_path, response_path, lbl_response_path;
+        lbl_kernels_path, lbl_jacobian_path, lbl_forcing_path, response_path, lbl_response_path, species_path, lbl_species_path;
     double co2_factor = 1.0;
     int ncol = 1, device = 0, check_every = 250, steps_exact = 0, gpus = 1, fixed_rh = 1;
     long max_steps = 6000;
@@ -518,6 +581,8 @@ int main(int argc, char** argv) {
         else if (a == "--response-out") response_path = val();
         else if (a == "--lbl-response-out") lbl_response_path = val();
         else if (a == "--fixed-q") fixed_rh = 0;
+        else if (a == "--species-jacobian-out") species_path = val();
+        else if (a == "--lbl-species-jacobian-out") lbl_species_path = val();
         else {
             std::fprintf(stderr, "rcm_rce: unknown argument %s\n", a.c_str());
             return 1;
@@ -532,7 +597,8 @@ int main(int argc, char** argv) {
                              "[--lbl-bands-out FILE [--band-size 100] [--forcing-scale 1,2,1,1,1]] [--lbl-kernels-out FILE] "
                              "[--lbl-jacobian-out FILE] [--lbl-forcing-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4]] "
                              "[--response-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]] "
-                             "[--lbl-response-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]]\n");
+                             "[--lbl-response-out FILE [--forcing-scale 1,2,1,1,1] [--trop-layers 4] [--fixed-q]] "
+                             "[--species-jacobian-out FILE] [--lbl-species-jacobian-out FILE]\n");
         return 1;
     }
     if (!lbl_dir.empty() && !spectral_path.empty()) {
@@ -575,6 +641,15 @@ int main(int argc, char** argv) {
         return 1;
     }
     if (!lbl_response_path.empty()) response_path = lbl_response_path;  // the same response file, from the LBL call
+    if (!lbl_dir.empty() && !species_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --species-jacobian-out needs a repwvl table (--table): with --lbl use --lbl-species-jacobian-out\n");
+        return 1;
+    }
+    if (lbl_dir.empty() && !lbl_species_path.empty()) {
+        std::fprintf(stderr, "rcm_rce: --lbl-species-jacobian-out needs line-by-line tables (--lbl)\n");
+        return 1;
+    }
+    if (!lbl_species_path.empty()) species_path = lbl_species_path;  // the same species file, from the LBL call
     if (lbl_dir.empty() && !bands_path.empty()) {
         std::fprintf(stderr, "rcm_rce: --lbl-bands-out needs line-by-line tables (--lbl)\n");
         return 1;
@@ -701,6 +776,7 @@ int main(int argc, char** argv) {
         const bool response = !response_path.empty();
         std::vector<double> Fr(response ? n * 2 : 0), dTr(response ? n * NLAY : 0), dTsr(response ? n : 0);
         std::vector<int> itr(response ? n : 0);
+        std::vector<double> S(species_path.empty() ? 0 : n * 3 * SPJ_NE);
         const std::vector<int> bstart = bands_path.empty() ? std::vector<int>() : lbl_band_starts(nwvl, band_size);
         const int nband = bands_path.empty() ? 0 : (int)bstart.size() - 1;
         std::vector<double> B(n * nband * 4);
@@ -708,7 +784,7 @@ int main(int argc, char** argv) {
                 max_steps, check_every, steps_exact, resume_path, ckpt_path, T.data(), Ts.data(), Eu.data(), time_h.data(),
                 dims[2], olr.data(), sfc.data(), !kernels_path.empty(), K.data(), !jacobian_path.empty(), H.data(),
                 forcing, forcing_scale, ntrop.data(), Ff.data(), dTf.data(), itf.data(), nband, bstart.data(), B.data(),
-                response, fixed_rh, Fr.data(), dTr.data(), dTsr.data(), itr.data()};
+                response, fixed_rh, Fr.data(), dTr.data(), dTsr.data(), itr.data(), !species_path.empty(), S.data()};
         std::vector<Shard> shards((size_t)gpus);
         std::vector<ncclComm_t> comms((size_t)gpus);
         std::vector<int> devs((size_t)gpus);
@@ -759,6 +835,10 @@ int main(int argc, char** argv) {
             return 1;
         }
         if (response && write_response(response_path, ncol, player.data(), Fr.data(), dTr.data(), dTsr.data(), itr.data())) {
+            rcm_table_free(table);
+            return 1;
+        }
+        if (!species_path.empty() && write_species(species_path, ncol, player.data(), S.data())) {
             rcm_table_free(table);
             return 1;
         }
@@ -905,6 +985,12 @@ int main(int argc, char** argv) {
                                                                     nullptr, itr.data());
         if (st != RCM_OK) return die(lbl ? "rcm_lbl_climate_response" : "rcm_climate_response", st, s);
         if (write_response(response_path, ncol, player.data(), Fr.data(), dTr.data(), dTsr.data(), itr.data())) return 1;
+    }
+    if (!species_path.empty()) {
+        std::vector<double> S(m * 3 * SPJ_NE);
+        st = species_rows(s, lbl, ncol, S.data());
+        if (st != RCM_OK) return die(lbl ? "rcm_lbl_species_jacobian" : "rcm_species_jacobian", st, s);
+        if (write_species(species_path, ncol, player.data(), S.data())) return 1;
     }
     if (!bands_path.empty()) {
         const std::vector<int> bstart = lbl_band_starts((int)lbl_wvl.size(), band_size);

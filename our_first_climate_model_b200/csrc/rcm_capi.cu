@@ -17,6 +17,7 @@
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
+#include "rcm_species.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -1787,6 +1788,45 @@ int rcm_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale
         });
 }
 
+// the species of the entries of both species-Jacobian calls, in the order of vmr_scale: H2O, CO2, O3, N2O, CH4
+constexpr unsigned kSpeciesMask = 0x2F;
+
+// Species Jacobians: the flux Jacobian's chunks, prep and layout, rcm_species_fjac_kernel in place of rcm_fjac_kernel.
+int rcm_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac) {
+    if (!s) return RCM_ERR_ARG;
+    DiagScale sc{};
+    const int st = diag_check(s, "rcm_species_jacobian", col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->p.species_mask != kSpeciesMask)
+        return fail(s, RCM_ERR_STATE, "rcm_species_jacobian: needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (!J && !dE_jac) return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    struct Set {
+        DiagState state;
+        double *J, *H;
+    };
+    return diag_chunks<Set>(
+        s, col0, ncol, vmr_scale ? &sc : nullptr,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // J [ch][2][21][100], dE_jac [ch][20][100]
+            z.J = m.take<double>(ch * SPJ_NJ);
+            z.H = m.take<double>(ch * SPJ_NH);
+        },
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) -> int {
+            SpjacArgs g = diag_args<SpjacArgs>(a);
+            g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+            g.J = z.J;
+            g.dE_jac = z.H;
+            CU(rcm_launch_species_fjac(g, q));
+            s->launches += 1;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (J) CU(cudaMemcpyAsync(J + r * SPJ_NJ, z.J, (size_t)n * SPJ_NJ * D, cudaMemcpyDeviceToHost, q));
+            if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * SPJ_NH, z.H, (size_t)n * SPJ_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
 // ------------------------------------------------------------------------------------------
 // Line-by-line calls (rcm_lbl_diagnose_fluxes, rcm_lbl_radiative_kernels): the step's prep kernel on copies of a chunk's T,
 // previous profile, VMRs and T_surf, then the species factors; the state stays as it is.
@@ -2046,6 +2086,48 @@ int rcm_lbl_flux_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_s
         [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
             if (J) CU(cudaMemcpyAsync(J + r * FJAC_NJ, z.J, (size_t)n * FJAC_NJ * D, cudaMemcpyDeviceToHost, q));
             if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * FJAC_NH, z.H, (size_t)n * FJAC_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+// Line-by-line species Jacobians: the LBL flux Jacobian's chunks and prep, rcm_lbl_species_fjac_kernel in place of
+// rcm_lbl_fjac_kernel.  The CO2, CH4 and N2O shares come from the tables' raw planes with the factors lbl_planes composes with.
+int rcm_lbl_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_species_jacobian";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->p.species_mask != kSpeciesMask) return fail(s, RCM_ERR_STATE, fn + ": needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (!J && !dE_jac) return RCM_OK;
+    constexpr size_t D = sizeof(double);
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    const double* raw = s->d_lbl_tau5 + 3 * (size_t)s->lbl_nwvl * NLAY;
+    struct Set {
+        DiagState state;
+        LblState lbl;
+        double *J, *H;
+    };
+    return chunk_loop<Set, LblArgs>(
+        s, col0, ncol, diag_chunk(ncol), false,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // J [ch][2][21][100], dE_jac [ch][20][100]
+            lbl_take(m, ch, z.lbl);
+            z.J = m.take<double>(ch * SPJ_NJ);
+            z.H = m.take<double>(ch * SPJ_NH);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
+            return lbl_prep(s, q, c0, n, z.state, z.lbl, tau3, vmr_scale ? &sc : nullptr, a);
+        },
+        [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
+            CU(rcm_launch_lbl_species_fjac(a, wtau, raw, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3], z.J, z.H, q));
+            s->launches += 1;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            if (J) CU(cudaMemcpyAsync(J + r * SPJ_NJ, z.J, (size_t)n * SPJ_NJ * D, cudaMemcpyDeviceToHost, q));
+            if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * SPJ_NH, z.H, (size_t)n * SPJ_NH * D, cudaMemcpyDeviceToHost, q));
             return RCM_OK;
         });
 }

@@ -29,6 +29,7 @@
 #include "rcm_lbl_diag.cuh"
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
+#include "rcm_species.cuh"
 
 __constant__ DevConst cst;
 
@@ -207,6 +208,8 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_lbl_jac_kernels.cuh"
 #include "rcm_lbl_fjac_kernels.cuh"
 #include "rcm_ecs_kernels.cuh"
+#include "rcm_species_kernels.cuh"
+#include "rcm_lbl_species_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -540,6 +543,23 @@ cudaError_t rcm_launch_lbl_fjac(const LblArgs& a, double wtau, double* J, double
 
 cudaError_t rcm_launch_lbl_fdh_retemper(const FdhArgs& f, double* T, double* Ts, const double* Ts0, cudaStream_t st) {
     rcm_lbl_fdh_retemper_kernel<<<(f.ncol * NLAY + 255) / 256, 256, 0, st>>>(f, T, Ts, Ts0);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_species_fjac(const SpjacArgs& a, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_species_fjac_kernel<true> : rcm_species_fjac_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPJ_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<(a.ncol + SPJ_WARPS - 1) / SPJ_WARPS, SPJ_NT, SPJ_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_species_fjac(const LblArgs& a, double wtau, const double* raw, double f_co2x, double f_ch4,
+                                        double f_n2o, double* J, double* dE_jac, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_lbl_species_fjac_kernel<true> : rcm_lbl_species_fjac_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPJ_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<(a.ncol + SPJ_WARPS - 1) / SPJ_WARPS, SPJ_NT, SPJ_SMEM, st>>>(a, wtau, raw, f_co2x, f_ch4, f_n2o, J, dE_jac);
     return cudaGetLastError();
 }
 
