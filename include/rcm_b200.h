@@ -436,6 +436,43 @@ int rcm_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_sc
  * the 3 x nwvl x 20 doubles of rcm_lbl_diagnose_fluxes.  Errors as rcm_lbl_flux_jacobian; also RCM_ERR_STATE with any
  * species_mask other than the default 0x2F.  Each leaves the solver usable. */
 int rcm_lbl_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vmr_scale, double* J, double* dE_jac);
+/* Adjoint flux gradients of the columns [col0, col0 + ncol): the derivatives of one weighted sum of each column's broadband
+ * fluxes and heating rates of the NEXT step, by one reverse sweep of the radiative transfer instead of full Jacobians.
+ * Row r is column c = col0 + r.  Cotangents (host, each may be NULL = zero): w_E_down, w_E_up [ncol][21], w_dE [ncol][20];
+ * the objective of column c is
+ *   Phi_c = sum_k w_E_down[r][k] E_down[k] + sum_k w_E_up[r][k] E_up[k] + sum_l w_dE[r][l] dE[l],
+ * with E and dE the fluxes and heating rates rcm_diagnose_fluxes returns for the same vmr_scale (dE from E as main.cpp:337-341;
+ * its solar term is constant).
+ * Output (host): grad [ncol][121], grad[r][e] = dPhi_c/dx_e over the entries e = 0..19 T_l (layers top-down), e = 20 T_surf,
+ * e = 21 + 20 s + l ln x_{s,l}, s in the order of vmr_scale (0 H2O, 1 CO2, 2 O3, 3 N2O, 4 CH4).  Entries 0..40 are those of
+ * rcm_flux_jacobian, entries 21..120 those of rcm_species_jacobian offset by 21, with every definition of those calls: the
+ * state they differentiate (sort, water-vapour feedback, grey or per-column cloud, vmr_scale), the step-0 rule for d/dT_l,
+ * fixed T for ln x (no re-sort, no feedback), 0 where the tau clamp or floor acts, where T <= T_floor in the Planck source and
+ * where a species' VMR is 0.  grad is their contraction with the cotangents, to rounding: sum_k w_E_down[k] J[0][k] +
+ * w_E_up[k] J[1][k] + sum_l w_dE[l] dE_jac[l].
+ * The cotangents are folded on the host into level cotangents, b_k on E_down[k] and a_k on E_up[k]: b_k = (w_E_down[k] +
+ * w_dE[k]) - w_dE[k-1], a_k = (w_E_up[k] - w_dE[k]) + w_dE[k-1], each term where it exists.  The sum over the wavelengths is
+ * taken in partials of 5 rounds of 4 wavelengths (wavelengths g, g + 4, ... per group g, the groups in order), then the
+ * partials in order: fixed by the table and the angle schedule.  Every value is a function of its column alone: ranges,
+ * chunks and shards give bit-identical rows.
+ * grad NULL: RCM_OK without work.  All three cotangents NULL: grad filled with 0.0, no launch.  Synchronous; changes nothing.
+ * Device scratch of its own: two sets for chunks of at most 8,192 columns, each of 183 + 121 (1 + nsplit) doubles per column,
+ * nsplit = ceil(ceil(nwvl / 4) / 5), plus the tile blocks (about 0.15 GB for 100 wavelengths).
+ * Errors as rcm_species_jacobian; also RCM_ERR_ARG for a cotangent entry that is not finite (checked on the host before any
+ * work).  Each error leaves the solver usable. */
+int rcm_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const double* w_E_down, const double* w_E_up,
+                      const double* w_dE, double* grad);
+/* Adjoint flux gradients of the line-by-line path: rcm_flux_gradient's cotangents, objective, entries, fold and properties at
+ * the state rcm_lbl_diagnose_fluxes radiates for the same vmr_scale, with the definitions of rcm_lbl_flux_jacobian (d/dT_l
+ * through layer l's Planck source alone, cplkavg_narrow's dB/dT) and rcm_lbl_species_jacobian (each species' share of tau as
+ * the rounded product rcm_lbl_diagnose_fluxes composes).  The sum over the wavelengths is taken in partials of 1,024
+ * wavelengths (wavelengths g, g + 4, ... of a partial per group g, the groups in order), then the partials in order: fixed by
+ * the table.  Device scratch of its own: two sets for chunks of at most 8,192 columns, each of 224 + 121 (1 + ceil(nwvl /
+ * 1,024)) doubles per column (about 0.36 GB at 20,000 wavelengths); with CO2, CH4 or N2O scaled also the 3 x nwvl x 20 doubles
+ * of rcm_lbl_diagnose_fluxes.  Errors as rcm_lbl_species_jacobian; also RCM_ERR_ARG for a cotangent entry that is not
+ * finite.  Each error leaves the solver usable. */
+int rcm_lbl_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const double* w_E_down,
+                          const double* w_E_up, const double* w_dE, double* grad);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

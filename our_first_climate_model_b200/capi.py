@@ -548,6 +548,38 @@ class Solver:
             out[f"J_{name}"] = J[..., s * NLAY:(s + 1) * NLAY]
         return out
 
+    def flux_gradient(self, w_E_down=None, w_E_up=None, w_dE=None, col0: int = 0, ncol: int | None = None,
+                      vmr_scale=None) -> dict:
+        """rcm_flux_gradient: the gradient of Phi = sum_k w_E_down[k] E_down[k] + w_E_up[k] E_up[k] + sum_l w_dE[l] dE[l]
+        (per column, the next step's broadband fluxes and heating rates) by one adjoint sweep, for columns [col0, col0 + ncol),
+        without changing anything.  Cotangents: w_E_down, w_E_up [ncol, 21], w_dE [ncol, 20], None = zero.  vmr_scale as in
+        diagnose_fluxes.
+        -> grad [ncol, 121] (entries 0..40 as flux_jacobian, 21..120 as species_jacobian's 100) with the views dT [ncol, 20],
+        dTs [ncol] and dlnx [ncol, 5, 20] (species in the order of vmr_scale)."""
+        return self._flux_gradient(_lib.rcm_flux_gradient, w_E_down, w_E_up, w_dE, col0, ncol, vmr_scale)
+
+    def lbl_flux_gradient(self, w_E_down=None, w_E_up=None, w_dE=None, col0: int = 0, ncol: int | None = None,
+                          vmr_scale=None) -> dict:
+        """rcm_lbl_flux_gradient: flux_gradient on the line-by-line path, at the state lbl_diagnose_fluxes radiates, with the
+        definitions of lbl_flux_jacobian and lbl_species_jacobian.  Arguments and outputs as flux_gradient."""
+        return self._flux_gradient(_lib.rcm_lbl_flux_gradient, w_E_down, w_E_up, w_dE, col0, ncol, vmr_scale)
+
+    def _flux_gradient(self, fn, w_E_down, w_E_up, w_dE, col0, ncol, vmr_scale) -> dict:
+        n = self.ncol - col0 if ncol is None else int(ncol)
+        sc = self._vmr_scale(vmr_scale)
+        m = max(n, 0)
+        ws = []
+        for name, w, nk in (("w_E_down", w_E_down, NLEV), ("w_E_up", w_E_up, NLEV), ("w_dE", w_dE, NLAY)):
+            if w is not None:
+                w = _f64(w)
+                if w.shape != (m, nk):
+                    raise ValueError(f"{name} needs shape ({m}, {nk}), got {w.shape}")
+            ws.append(w)
+        ns = len(self.SPECIES)
+        g = np.zeros((m, NLEV + ns * NLAY))
+        _check(fn(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(ws[0]), _p(ws[1]), _p(ws[2]), _p(g)), self._h)
+        return dict(grad=g, dT=g[:, :NLAY], dTs=g[:, NLAY], dlnx=g[:, NLEV:].reshape(m, ns, NLAY))
+
     def lbl_adjusted_forcing(self, vmr_scale, ntrop, col0: int = 0, ncol: int | None = None, tol: float = 1e-6,
                              max_iter: int = 20) -> dict:
         """rcm_lbl_adjusted_forcing: adjusted_forcing on the line-by-line path (base state: what lbl_diagnose_fluxes

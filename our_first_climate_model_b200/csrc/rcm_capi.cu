@@ -18,6 +18,7 @@
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
 #include "rcm_species.cuh"
+#include "rcm_grad.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -2128,6 +2129,162 @@ int rcm_lbl_species_jacobian(rcm_solver* s, int col0, int ncol, const double* vm
         [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
             if (J) CU(cudaMemcpyAsync(J + r * SPJ_NJ, z.J, (size_t)n * SPJ_NJ * D, cudaMemcpyDeviceToHost, q));
             if (dE_jac) CU(cudaMemcpyAsync(dE_jac + r * SPJ_NH, z.H, (size_t)n * SPJ_NH * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+// ------------------------------------------------------------------------------------------
+// Flux gradients (rcm_flux_gradient, rcm_lbl_flux_gradient): the species Jacobians' chunks and prep, then one reverse sweep per
+// (column, wavelength, angle) with the chunk's level cotangents, partial sums over fixed wavelength ranges, and their sum.
+// ------------------------------------------------------------------------------------------
+extern "C++" {
+namespace {
+
+// The level cotangents of the rows [0, ncol) into co [ncol][42] = {b_0..b_20, a_0..a_20}, w_dE folded in as the adjoint of dE
+// from E (main.cpp:337-341: dE_l = Ed_l - Ed_{l+1} + Eu_{l+1} - Eu_l for l < 19, dE_19 = Ed_19 - Eu_19):
+//   b_k = (w_Ed[k] + w_dE[k]) - w_dE[k-1],  a_k = (w_Eu[k] - w_dE[k]) + w_dE[k-1],  each term only where it exists.
+// RCM_ERR_ARG for a non-finite entry; *any = false when all three are NULL.
+int grad_fold(rcm_solver* s, const std::string& fn, int ncol, const double* wEd, const double* wEu, const double* wdE,
+              std::vector<double>& co, bool* any) {
+    *any = wEd || wEu || wdE;
+    if (!*any) return RCM_OK;
+    const struct { const double* p; size_t n; const char* name; } in[3] = {
+        {wEd, (size_t)ncol * NLEV, "w_E_down"}, {wEu, (size_t)ncol * NLEV, "w_E_up"}, {wdE, (size_t)ncol * NLAY, "w_dE"}};
+    for (const auto& v : in)
+        if (v.p)
+            for (size_t i = 0; i < v.n; ++i)
+                if (!std::isfinite(v.p[i]))
+                    return fail(s, RCM_ERR_ARG, fn + ": " + v.name + "[" + std::to_string(i / (v.n / ncol)) + "][" +
+                                                    std::to_string(i % (v.n / ncol)) + "] is not finite");
+    co.assign((size_t)ncol * GRAD_NCO, 0.0);
+    for (int r = 0; r < ncol; ++r) {
+        double* b = co.data() + (size_t)r * GRAD_NCO;
+        double* a = b + NLEV;
+        for (int k = 0; k < NLEV; ++k) {
+            double bk = wEd ? wEd[(size_t)r * NLEV + k] : 0.0, ak = wEu ? wEu[(size_t)r * NLEV + k] : 0.0;
+            if (wdE) {
+                const double* w = wdE + (size_t)r * NLAY;
+                if (k < NLAY) {
+                    bk = bk + w[k];
+                    ak = ak - w[k];
+                }
+                if (k >= 1 && k < NLAY) {
+                    bk = bk - w[k - 1];
+                    ak = ak + w[k - 1];
+                }
+            }
+            b[k] = bk;
+            a[k] = ak;
+        }
+    }
+    return RCM_OK;
+}
+
+}  // namespace
+}  // extern "C++"
+
+// Flux gradients: rcm_grad_rt_kernel per (tile, split) unit into partials [ch][nsplit][121], rcm_grad_sum_kernel over the splits.
+int rcm_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const double* w_E_down, const double* w_E_up,
+                      const double* w_dE, double* grad) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_flux_gradient";
+    DiagScale sc{};
+    int st = diag_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->p.species_mask != kSpeciesMask) return fail(s, RCM_ERR_STATE, fn + ": needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (!grad) return RCM_OK;
+    std::vector<double> co;
+    bool any = false;
+    if ((st = grad_fold(s, fn, ncol, w_E_down, w_E_up, w_dE, co, &any)) != RCM_OK) return st;
+    if (!any) {
+        std::fill(grad, grad + (size_t)ncol * GRAD_NE, 0.0);
+        return RCM_OK;
+    }
+    constexpr size_t D = sizeof(double);
+    const int nsplit = split_geom(s, 0).nsplit;
+    struct Set {
+        DiagState state;
+        double *co, *part, *grad;
+    };
+    return chunk_loop<Set, SplitArgs>(
+        s, col0, ncol, diag_chunk(ncol), true,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // co [ch][42], part [ch][nsplit][121], grad [ch][121]
+            z.co = m.take<double>(ch * GRAD_NCO);
+            z.part = m.take<double>(ch * nsplit * GRAD_NE);
+            z.grad = m.take<double>(ch * GRAD_NE);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, SplitArgs& a) -> int {  // diag_chunks' prep, the chunk's cotangents first
+            CU(cudaMemcpyAsync(z.co, co.data() + (size_t)(c0 - col0) * GRAD_NCO, (size_t)n * GRAD_NCO * D, cudaMemcpyHostToDevice, q));
+            return diag_prep(s, q, c0, n, z.state, vmr_scale ? &sc : nullptr, a);
+        },
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) -> int {
+            GradArgs g = unit_args<GradArgs>(a);
+            g.T_floor = a.T_floor;
+            g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+            g.T = a.Tlayer;
+            g.Ts = a.Tsurf;
+            g.co = z.co;
+            g.part = z.part;
+            CU(rcm_launch_grad_rt(g, std::min(g.nunits, rcm_grad_ctas_per_sm() * nsm_of(s)), q));
+            CU(rcm_launch_grad_sum(g.ncol, g.nsplit, z.part, z.grad, q));
+            s->launches += 2;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            CU(cudaMemcpyAsync(grad + r * GRAD_NE, z.grad, (size_t)n * GRAD_NE * D, cudaMemcpyDeviceToHost, q));
+            return RCM_OK;
+        });
+}
+
+// Line-by-line flux gradients: the LBL species Jacobian's chunks, prep, raw planes and factors, then rcm_lbl_grad_kernel into
+// partials [ch][ceil(nwvl / GRAD_LBL_SPAN)][121] and rcm_grad_sum_kernel over the spans.
+int rcm_lbl_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const double* w_E_down,
+                          const double* w_E_up, const double* w_dE, double* grad) {
+    if (!s) return RCM_ERR_ARG;
+    const std::string fn = "rcm_lbl_flux_gradient";
+    DiagScale sc{};
+    int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
+    if (st != RCM_OK) return st;
+    if (s->p.species_mask != kSpeciesMask) return fail(s, RCM_ERR_STATE, fn + ": needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (!grad) return RCM_OK;
+    std::vector<double> co;
+    bool any = false;
+    if ((st = grad_fold(s, fn, ncol, w_E_down, w_E_up, w_dE, co, &any)) != RCM_OK) return st;
+    if (!any) {
+        std::fill(grad, grad + (size_t)ncol * GRAD_NE, 0.0);
+        return RCM_OK;
+    }
+    constexpr size_t D = sizeof(double);
+    const double* tau3 = nullptr;
+    if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
+    const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    const double* raw = s->d_lbl_tau5 + 3 * (size_t)s->lbl_nwvl * NLAY;
+    const int nspan = (s->lbl_nwvl + GRAD_LBL_SPAN - 1) / GRAD_LBL_SPAN;
+    struct Set {
+        DiagState state;
+        LblState lbl;
+        double *co, *part, *grad;
+    };
+    return chunk_loop<Set, LblArgs>(
+        s, col0, ncol, diag_chunk(ncol), false,
+        [&](DiagCarve& m, size_t ch, Set& z) {  // co [ch][42], part [ch][nspan][121], grad [ch][121]
+            lbl_take(m, ch, z.lbl);
+            z.co = m.take<double>(ch * GRAD_NCO);
+            z.part = m.take<double>(ch * nspan * GRAD_NE);
+            z.grad = m.take<double>(ch * GRAD_NE);
+        },
+        [&](const Set& z, int c0, int n, cudaStream_t q, LblArgs& a) -> int {
+            CU(cudaMemcpyAsync(z.co, co.data() + (size_t)(c0 - col0) * GRAD_NCO, (size_t)n * GRAD_NCO * D, cudaMemcpyHostToDevice, q));
+            return lbl_prep(s, q, c0, n, z.state, z.lbl, tau3, vmr_scale ? &sc : nullptr, a);
+        },
+        [&](const Set& z, const LblArgs& a, cudaStream_t q) -> int {
+            CU(rcm_launch_lbl_grad(a, wtau, raw, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3], z.co, z.part, q));
+            CU(rcm_launch_grad_sum(a.ncol, nspan, z.part, z.grad, q));
+            s->launches += 2;
+            return RCM_OK;
+        },
+        [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
+            CU(cudaMemcpyAsync(grad + r * GRAD_NE, z.grad, (size_t)n * GRAD_NE * D, cudaMemcpyDeviceToHost, q));
             return RCM_OK;
         });
 }

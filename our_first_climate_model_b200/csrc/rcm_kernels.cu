@@ -30,6 +30,7 @@
 #include "rcm_lbl_jac.cuh"
 #include "rcm_lbl_fjac.cuh"
 #include "rcm_species.cuh"
+#include "rcm_grad.cuh"
 
 __constant__ DevConst cst;
 
@@ -210,6 +211,8 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_ecs_kernels.cuh"
 #include "rcm_species_kernels.cuh"
 #include "rcm_lbl_species_kernels.cuh"
+#include "rcm_grad_kernels.cuh"
+#include "rcm_lbl_grad_kernels.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Solar setup per column (SURVEY section 8(f)3): doubling_adding + solar_radiative_transfer_setup
@@ -580,5 +583,34 @@ cudaError_t rcm_launch_ecs_check(const EcsArgs& a, cudaStream_t st) {
 
 cudaError_t rcm_launch_ecs_newton(const EcsArgs& a, cudaStream_t st) {
     rcm_ecs_newton_kernel<<<(a.ncol + ECS_NEWTON_WARPS - 1) / ECS_NEWTON_WARPS, ECS_NEWTON_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+int rcm_grad_ctas_per_sm() { return GRAD_CTAS; }
+
+cudaError_t rcm_launch_grad_rt(const GradArgs& a, int grid, cudaStream_t st) {
+    auto kern = a.clampk ? rcm_grad_rt_kernel<true> : rcm_grad_rt_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GRAD_SMEM);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, GRAD_NT, GRAD_SMEM, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_lbl_grad(const LblArgs& a, double wtau, const double* raw, double f_co2x, double f_ch4, double f_n2o,
+                                const double* co, double* part, cudaStream_t st) {
+    constexpr int C = RCM_LBL_C, NT = RCM_LBL_NT;
+    const size_t smem = ((size_t)EXP_TAB * EXP_REP + 3 * TBD_LEN + 2 * C + 2 * (HALF + 1) * NT + (size_t)(NT / (2 * C)) * C * GRAD_NE) *
+                        sizeof(double);
+    auto kern = a.clampk ? rcm_lbl_grad_kernel<C, NT, true> : rcm_lbl_grad_kernel<C, NT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const int nspan = (a.nwvl + GRAD_LBL_SPAN - 1) / GRAD_LBL_SPAN;
+    kern<<<a.ntiles * nspan, NT, smem, st>>>(a, wtau, raw, f_co2x, f_ch4, f_n2o, co, part);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_grad_sum(int ncol, int npart, const double* part, double* grad, cudaStream_t st) {
+    const size_t blocks = ((size_t)ncol * GRAD_NE + 255) / 256;
+    rcm_grad_sum_kernel<<<blocks < 4096 ? (int)blocks : 4096, 256, 0, st>>>(ncol, npart, part, grad);
     return cudaGetLastError();
 }
