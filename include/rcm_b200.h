@@ -473,6 +473,43 @@ int rcm_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale
  * finite.  Each error leaves the solver usable. */
 int rcm_lbl_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const double* w_E_down,
                           const double* w_E_up, const double* w_dE, double* grad);
+/* Climate-response gradients of the columns [col0, col0 + ncol): the derivatives of the equilibrium surface warming dTs in
+ * every species' VMR in every layer of the perturbed state and in an imposed forcing term of every equation, by one adjoint
+ * solve of the converged Newton system and one reverse sweep of the radiative transfer.
+ * The call runs at exactly the solution rcm_climate_response finds for the same vmr_scale, ntrop, fixed_rh, tol and max_iter
+ * (same iterates, same bits).  Write that solution as y = (dT_0 .. dT_{ntrop-1}, dTs), m = ntrop + 1, and the residual as
+ * R(y, p) with the equations and order of rcm_climate_response (i < ntrop: the heating rate of layer i; i = ntrop: the net flux
+ * at level ntrop).  The derivatives are taken in
+ *   p = ln x_{s,l}: a multiplicative perturbation of species s in layer l of the PERTURBED state only (the base state is
+ *     fixed); entry e = 20 s + l, s in the order of vmr_scale (0 H2O, 1 CO2, 2 O3, 3 N2O, 4 CH4), layers l top-down; with the
+ *     definitions of rcm_species_jacobian at the solution state (the tile block's rows at T_B + dT).  With fixed_rh != 0,
+ *     ln x_{H2O,l} is a factor on the feedback's H2O of layer l, i.e. a relative-humidity change;
+ *   q_i: an imposed forcing term added to equation i: for i < ntrop an extra heating of stratospheric layer i (W m-2, the
+ *     units of dE), for i = ntrop an extra net downward flux at the tropopause level.
+ * With A the m x m Newton matrix of rcm_climate_response assembled from the flux Jacobian AT THE SOLUTION (same D_i, gamma_l,
+ * conv_l and index order), s = -A^{-T} e_m, solved by the same elimination (partial pivoting, lowest row on ties, NaN refused):
+ *   dTs_dF [ncol][21]: dTs/dq_i = s_i for i < ntrop, entry 20 = s_m (K per W m-2: the column's local climate sensitivity
+ *     parameter at the tropopause), exactly 0.0 in entries ntrop..19;
+ *   dTs_dlnx [ncol][100]: dTs/dp_e = s^T dR/dp_e, the flux gradient (rcm_flux_gradient's entries 21..120 at the solution
+ *     state) with the cotangents w_dE[i] = s_i (i < ntrop), w_E_down[ntrop] = s_m, w_E_up[ntrop] = -s_m, every other 0.0,
+ *     folded with rcm_flux_gradient's expressions in its order;
+ *   dTs [ncol], iters [ncol]: rcm_climate_response's bytes for the same arguments.
+ * Any output may be NULL; all NULL: RCM_OK without work.  The rows of dTs_dF and dTs_dlnx are quiet NaN where iters == -1 or
+ * where A at the solution has a zero or non-finite pivot (iters keeps the response's value).  Every value is a function of its
+ * column alone: ranges, chunks and shards give bit-identical rows.  Synchronous; changes nothing.  Device scratch of its own:
+ * that of rcm_climate_response plus 184 + 121 nsplit doubles per column of a chunk (nsplit as rcm_flux_gradient), twice.
+ * Errors as rcm_climate_response; also RCM_ERR_STATE with any species_mask other than the default 0x2F.  Each error leaves the
+ * solver usable. */
+int rcm_climate_response_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
+                                  double tol, int max_iter, double* dTs, double* dTs_dF, double* dTs_dlnx, int* iters);
+/* Climate-response gradients of the line-by-line path: rcm_climate_response_gradient at the solution of
+ * rcm_lbl_climate_response, with A from rcm_lbl_flux_jacobian at the solution and the species entries of
+ * rcm_lbl_species_jacobian there (the LBL copies' T_B + dT and s_H2O, each species' rounded share of tau).  Device scratch of its
+ * own: that of rcm_lbl_climate_response plus 184 + 121 ceil(nwvl / 1,024) doubles per column of a chunk, twice.  Errors as
+ * rcm_lbl_climate_response; also RCM_ERR_STATE with any species_mask other than the default 0x2F. */
+int rcm_lbl_climate_response_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop,
+                                      int fixed_rh, double tol, int max_iter, double* dTs, double* dTs_dF, double* dTs_dlnx,
+                                      int* iters);
 /* Batched form of output_conv (main.cpp:102-114): for every column the 20 rows "layer,player,Tlayer,theta,time"
  * ("%d,%f,%f,%f,%f\n", theta = Tlayer * (1000/player)^(2/7) as t_to_theta, main.cpp:123-127; time in hours).
  * column_ids != 0 prefixes every row with the column number ("%d,"); with ncol == 1 and column_ids == 0 the rows are

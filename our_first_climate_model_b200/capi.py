@@ -618,6 +618,37 @@ class Solver:
         return dict(F=F, IRF_toa=F[:, 0], IRF_trop=F[:, 1], dT=dT, dTs=dTs, E_down=Ed, E_up=Eu, iters=it,
                     converged=it >= 0)
 
+    def climate_response_gradient(self, vmr_scale, ntrop, fixed_rh: bool = True, col0: int = 0, ncol: int | None = None,
+                                  tol: float = 1e-6, max_iter: int = 20) -> dict:
+        """rcm_climate_response_gradient: the derivatives of climate_response's surface warming dTs at its solution for the
+        same arguments, by one adjoint solve and one reverse sweep, without changing anything.
+        -> dTs [ncol] and iters [ncol] (climate_response's bytes), converged, dTs_dF [ncol, 21] with the views
+        dTs_dheat [ncol, 20] (K per W/m2 of extra heating of stratospheric layer i < ntrop; 0 below) and lambda_trop [ncol]
+        (K per W/m2 of extra net downward flux at the tropopause), and dTs_dlnx [ncol, 5, 20] (K per unit ln VMR of species s
+        in layer l of the perturbed state, species in the order of vmr_scale; with fixed_rh the H2O entries are per unit
+        ln relative humidity).  Rows of dTs_dF and dTs_dlnx are NaN where iters == -1 or the adjoint solve fails."""
+        return self._response_gradient(_lib.rcm_climate_response_gradient, vmr_scale, ntrop, fixed_rh, col0, ncol, tol,
+                                       max_iter)
+
+    def lbl_climate_response_gradient(self, vmr_scale, ntrop, fixed_rh: bool = True, col0: int = 0,
+                                      ncol: int | None = None, tol: float = 1e-6, max_iter: int = 20) -> dict:
+        """rcm_lbl_climate_response_gradient: climate_response_gradient at the solution of lbl_climate_response, with the
+        definitions of lbl_flux_jacobian and lbl_species_jacobian.  Arguments and results as climate_response_gradient."""
+        return self._response_gradient(_lib.rcm_lbl_climate_response_gradient, vmr_scale, ntrop, fixed_rh, col0, ncol, tol,
+                                       max_iter)
+
+    def _response_gradient(self, fn, vmr_scale, ntrop, fixed_rh, col0, ncol, tol, max_iter) -> dict:
+        """the arguments and results of the two climate-response gradient calls around fn"""
+        n, sc, nt = self._forcing_args(vmr_scale, ntrop, col0, ncol)
+        m = max(n, 0)
+        ns = len(self.SPECIES)
+        dTs, dF, g = np.zeros(m), np.zeros((m, NLEV)), np.zeros((m, ns * NLAY))
+        it = np.zeros(m, dtype=np.int32)
+        _check(fn(self._h, C.c_int(col0), C.c_int(n), _p(sc), _p(nt), C.c_int(1 if fixed_rh else 0), C.c_double(tol),
+                  C.c_int(max_iter), _p(dTs), _p(dF), _p(g), _p(it)), self._h)
+        return dict(dTs=dTs, dTs_dF=dF, dTs_dheat=dF[:, :NLAY], lambda_trop=dF[:, NLAY], dTs_dlnx=g.reshape(m, ns, NLAY),
+                    iters=it, converged=it >= 0)
+
     def _forcing_args(self, vmr_scale, ntrop, col0, ncol):
         """(ncol, vmr_scale, ntrop [ncol] int32) of the adjusted-forcing and climate-response calls"""
         n = self.ncol - col0 if ncol is None else int(ncol)

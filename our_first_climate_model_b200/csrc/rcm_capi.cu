@@ -8,6 +8,7 @@
 #include <cstring>
 #include <new>
 #include <functional>
+#include <limits>
 #include <string>
 #include <vector>
 
@@ -2180,6 +2181,23 @@ int grad_fold(rcm_solver* s, const std::string& fn, int ncol, const double* wEd,
     return RCM_OK;
 }
 
+// rcm_grad_rt_kernel on the tile blocks and units of the prep a, the Planck source at T and Ts, with the level cotangents co:
+// partials [ncol][nsplit][121] into part, then rcm_grad_sum_kernel over the splits into grad [ncol][121]
+int grad_sweep(rcm_solver* s, const SplitArgs& a, cudaStream_t q, const double* T, const double* Ts, const double* co,
+               double* part, double* grad) {
+    GradArgs g = unit_args<GradArgs>(a);
+    g.T_floor = a.T_floor;
+    g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    g.T = T;
+    g.Ts = Ts;
+    g.co = co;
+    g.part = part;
+    CU(rcm_launch_grad_rt(g, std::min(g.nunits, rcm_grad_ctas_per_sm() * nsm_of(s)), q));
+    CU(rcm_launch_grad_sum(g.ncol, g.nsplit, part, grad, q));
+    s->launches += 2;
+    return RCM_OK;
+}
+
 }  // namespace
 }  // extern "C++"
 
@@ -2217,18 +2235,8 @@ int rcm_flux_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale
             CU(cudaMemcpyAsync(z.co, co.data() + (size_t)(c0 - col0) * GRAD_NCO, (size_t)n * GRAD_NCO * D, cudaMemcpyHostToDevice, q));
             return diag_prep(s, q, c0, n, z.state, vmr_scale ? &sc : nullptr, a);
         },
-        [&](const Set& z, const SplitArgs& a, cudaStream_t q) -> int {
-            GradArgs g = unit_args<GradArgs>(a);
-            g.T_floor = a.T_floor;
-            g.wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
-            g.T = a.Tlayer;
-            g.Ts = a.Tsurf;
-            g.co = z.co;
-            g.part = z.part;
-            CU(rcm_launch_grad_rt(g, std::min(g.nunits, rcm_grad_ctas_per_sm() * nsm_of(s)), q));
-            CU(rcm_launch_grad_sum(g.ncol, g.nsplit, z.part, z.grad, q));
-            s->launches += 2;
-            return RCM_OK;
+        [&](const Set& z, const SplitArgs& a, cudaStream_t q) {
+            return grad_sweep(s, a, q, a.Tlayer, a.Tsurf, z.co, z.part, z.grad);
         },
         [&](const Set& z, size_t r, int n, cudaStream_t q) -> int {
             CU(cudaMemcpyAsync(grad + r * GRAD_NE, z.grad, (size_t)n * GRAD_NE * D, cudaMemcpyDeviceToHost, q));
@@ -2623,39 +2631,75 @@ int ecs_check_args(rcm_solver* s, const std::string& fn, int fixed_rh) {
     return RCM_OK;
 }
 
-}  // namespace
-}  // extern "C++"
+// The outputs of a climate-response call (NULL: not wanted).
+struct EcsOut {
+    double *F, *dT, *dTs, *E_down, *E_up;
+    int* iters;
+};
 
-// Equilibrium climate response: rcm_adjusted_forcing's scratch sets, streams, prep, base evaluation, scaling and Newton schedule
-// (fdh_schedule) with one more unknown per column, the uniform potential-temperature increment dTs of the troposphere and the
-// surface.  Per iterate: rcm_ecs_retemper_kernel (tile blocks at T + dT and Ts + dTs, with fixed RH the H2O row), the
-// evaluation and rcm_ecs_check_kernel; while columns are active, the flux Jacobian (rcm_fjac_kernel at T + dT, Ts + dTs) and
-// rcm_ecs_newton_kernel.
-int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh, double tol,
-                         int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up, int* iters) {
-    if (!s) return RCM_ERR_ARG;
-    const std::string fn = "rcm_climate_response";
+// The gradient calls' outputs: dTs_dF [ncol][21] and dTs_dlnx [ncol][100] (NULL: not wanted).
+struct EcsGrad {
+    double *dTs_dF, *dTs_dlnx;
+};
+
+// A slot's scratch for the gradient calls' epilogue: co [ch][42], part [ch][npart][121], sum [ch][121], dF [ch][21] (none for
+// the response alone, so that its scratch layout stays as it was)
+struct EcsGradSet {
+    double *co, *part, *sum, *dF;
+};
+
+void ecs_grad_take(DiagCarve& m, size_t ch, size_t npart, bool grad, EcsGradSet& g) {
+    g.co = m.take<double>(grad ? ch * GRAD_NCO : 0);
+    g.part = m.take<double>(grad ? ch * npart * GRAD_NE : 0);
+    g.sum = m.take<double>(grad ? ch * GRAD_NE : 0);
+    g.dF = m.take<double>(grad ? ch * NLEV : 0);
+}
+
+// the epilogue's downloads of the rows [r, r + n): dTs_dF, and entries 21..120 of the sums into dTs_dlnx
+int ecs_grad_download(rcm_solver* s, const EcsGrad& o, const EcsGradSet& g, size_t r, int n, cudaStream_t q) {
+    constexpr size_t D = sizeof(double);
+    if (o.dTs_dF) CU(cudaMemcpyAsync(o.dTs_dF + r * NLEV, g.dF, (size_t)n * NLEV * D, cudaMemcpyDeviceToHost, q));
+    if (o.dTs_dlnx)
+        CU(cudaMemcpy2DAsync(o.dTs_dlnx + r * SPJ_NE, SPJ_NE * D, g.sum + NLEV, GRAD_NE * D, SPJ_NE * D, n,
+                             cudaMemcpyDeviceToHost, q));
+    return RCM_OK;
+}
+
+// Equilibrium climate response of the repwvl path: rcm_adjusted_forcing's scratch sets, streams, prep, base evaluation, scaling
+// and Newton schedule (fdh_schedule) with one more unknown per column, the uniform potential-temperature increment dTs of the
+// troposphere and the surface.  Per iterate: rcm_ecs_retemper_kernel (tile blocks at T + dT and Ts + dTs, with fixed RH the
+// H2O row), the evaluation and rcm_ecs_check_kernel; while columns are active, the flux Jacobian (rcm_fjac_kernel at T + dT,
+// Ts + dTs) and rcm_ecs_newton_kernel.  With grad (the gradient call) the checks add the species mask, and a chunk whose
+// active count has reached 0 runs an epilogue before its download: the flux Jacobian at the solution, rcm_ecs_adjoint_kernel
+// and the gradient sweep on the retempered tile blocks.
+int ecs_response(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, const int* ntrop,
+                 int fixed_rh, double tol, int max_iter, const EcsOut& o, const EcsGrad* grad) {
     DiagScale sc{};
     int st = diag_check(s, fn, col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     if (s->h2o_slot != 0) return fail(s, RCM_ERR_STATE, fn + ": needs H2O among the active species");
     if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
     if ((st = ecs_check_args(s, fn, fixed_rh)) != RCM_OK) return st;
+    if (grad && s->p.species_mask != kSpeciesMask)
+        return fail(s, RCM_ERR_STATE, fn + ": needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (grad && !o.dTs && !o.iters && !grad->dTs_dF && !grad->dTs_dlnx) return RCM_OK;
     const int nwvl = s->dc.nwvl;
     const bool first = (s->step_index == 0);
     const size_t ch = diag_chunk(ncol), D = sizeof(double);
+    const size_t nsplit = split_geom(s, 0).nsplit;
     struct Slot {
         cudaStream_t q;
         int c0 = 0, n = 0, iter = 0;
         bool live = false;
         DiagState state;
         double *Ttau, *Tp, *dT, *Tsp, *dTs, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *spec_dn, *spec_up;
+        EcsGradSet g;
         int *ntrop, *iters, *count;
         SplitArgs a;
     } slot[2];
     // T_tau, T + dT, dT [ch][20], Ts + dTs, dTs [ch], E_down, E_up [ch][21] and dE [ch][20] of the base and of the current
     // iterate, F [ch][2], the output E_down, E_up [ch][21], J [ch][2][21][41], dE_jac [ch][20][41], spectral [2][ch][nwvl][21];
-    // ntrop, iters [ch] and the active count
+    // the epilogue's scratch; ntrop, iters [ch] and the active count
     st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
         z.Ttau = m.take<double>(ch * NLAY);
         z.Tp = m.take<double>(ch * NLAY);
@@ -2675,6 +2719,7 @@ int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_sc
         z.H = m.take<double>(ch * FJAC_NH);
         z.spec_dn = m.take<double>(ch * nwvl * NLEV);
         z.spec_up = m.take<double>(ch * nwvl * NLEV);
+        ecs_grad_take(m, ch, nsplit, grad, z.g);
         z.ntrop = m.take<int>(ch);
         z.iters = m.take<int>(ch);
         z.count = m.take<int>(1);
@@ -2751,14 +2796,26 @@ int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_sc
         }
         return check(z, k);
     };
+    // the flux Jacobian at the solution (the tile blocks, Tp and Tsp of the last retemper: a frozen column is not retempered),
+    // the adjoint solve and the sweep, then the epilogue's downloads
+    auto epilogue = [&](const Slot& z) -> int {
+        SplitArgs a = z.a;
+        a.Tsurf = z.Tsp;
+        if ((st = flux_jacobian(s, a, z.q, z.Tp, z.J, z.H)) != RCM_OK) return st;
+        CU(rcm_launch_ecs_adjoint(ecs_args(z), z.g.dF, z.g.co, z.q));
+        s->launches += 1;
+        if ((st = grad_sweep(s, z.a, z.q, z.Tp, z.Tsp, z.g.co, z.g.part, z.g.sum)) != RCM_OK) return st;
+        return ecs_grad_download(s, *grad, z.g, (size_t)(z.c0 - col0), z.n, z.q);
+    };
     auto download = [&](const Slot& z) -> int {
+        if (grad && (st = epilogue(z)) != RCM_OK) return st;
         const size_t r = (size_t)(z.c0 - col0);
-        if (F) CU(cudaMemcpyAsync(F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
-        if (dT) CU(cudaMemcpyAsync(dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
-        if (dTs) CU(cudaMemcpyAsync(dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
-        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
-        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
-        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        if (o.F) CU(cudaMemcpyAsync(o.F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.dT) CU(cudaMemcpyAsync(o.dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.dTs) CU(cudaMemcpyAsync(o.dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.E_down) CU(cudaMemcpyAsync(o.E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.E_up) CU(cudaMemcpyAsync(o.E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.iters) CU(cudaMemcpyAsync(o.iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
         return RCM_OK;
     };
     return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
@@ -2767,22 +2824,25 @@ int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_sc
 // Line-by-line equilibrium climate response: rcm_lbl_adjusted_forcing's chunks, prep, saved T_B and T_surf, base evaluation,
 // scaling and Newton schedule; per iterate rcm_lbl_ecs_retemper_kernel (every copy back to T_B + dT, T_surf + dTs, with fixed
 // RH s_H2O at T_B + dT), the evaluation and rcm_ecs_check_kernel; while columns are active, rcm_lbl_fjac_kernel at
-// T_B + dT, T_surf + dTs and rcm_ecs_newton_kernel.
-int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
-                             double tol, int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up,
-                             int* iters) {
-    if (!s) return RCM_ERR_ARG;
-    const std::string fn = "rcm_lbl_climate_response";
+// T_B + dT, T_surf + dTs and rcm_ecs_newton_kernel.  grad as in ecs_response; the epilogue is rcm_lbl_fjac_kernel at the
+// solution, rcm_ecs_adjoint_kernel, then rcm_lbl_grad_kernel on the copies and planes the last evaluation radiated.
+int lbl_ecs_response(rcm_solver* s, const std::string& fn, int col0, int ncol, const double* vmr_scale, const int* ntrop,
+                     int fixed_rh, double tol, int max_iter, const EcsOut& o, const EcsGrad* grad) {
     DiagScale sc{};
     int st = lbl_check(s, fn, col0, ncol, vmr_scale, sc);
     if (st != RCM_OK) return st;
     if ((st = fdh_check_args(s, fn, ncol, ntrop, tol, max_iter)) != RCM_OK) return st;
     if ((st = ecs_check_args(s, fn, fixed_rh)) != RCM_OK) return st;
+    if (grad && s->p.species_mask != kSpeciesMask)
+        return fail(s, RCM_ERR_STATE, fn + ": needs the default species_mask (H2O, CO2, O3, N2O, CH4)");
+    if (grad && !o.dTs && !o.iters && !grad->dTs_dF && !grad->dTs_dlnx) return RCM_OK;
     const double* tau3 = nullptr;
     if ((st = lbl_planes(s, sc, tau3)) != RCM_OK) return st;
     const size_t ch = diag_chunk(ncol), D = sizeof(double);
     const size_t nchunks = (size_t)lbl_args(s, 0).nchunks;
     const double wtau = 2 * M_PI * (1.0 / (double)s->p.nangle);
+    const double* raw = s->d_lbl_tau5 + 3 * (size_t)s->lbl_nwvl * NLAY;
+    const size_t nspan = (s->lbl_nwvl + GRAD_LBL_SPAN - 1) / GRAD_LBL_SPAN;
     struct Slot {
         cudaStream_t q;
         int c0 = 0, n = 0, iter = 0;
@@ -2790,14 +2850,15 @@ int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vm
         DiagState state;
         LblState lbl;
         double *Tb, *Ts0, *Tp, *dT, *Tsp, *dTs, *Ed0, *Eu0, *dE0, *Ed, *Eu, *dE, *F, *Edo, *Euo, *J, *H, *part, *dt;
+        EcsGradSet g;
         float* time;
         int *ntrop, *iters, *count;
         LblArgs a;
     } slot[2];
     // the prep's T_surf, sH, sO; T_B, T_surf as prepared, T_B + dT, dT [ch][20], T_surf + dTs, dTs [ch]; E_down, E_up [ch][21]
     // and dE [ch][20] of the base and of the current iterate, F [ch][2], the output E_down, E_up [ch][21], J [ch][2][21][41],
-    // dE_jac [ch][20][41], the rt kernel's partials [nchunks][ch][42], the finish's dt and time [ch]; ntrop, iters [ch] and the
-    // active count
+    // dE_jac [ch][20][41], the rt kernel's partials [nchunks][ch][42], the finish's dt, the epilogue's scratch, time [ch];
+    // ntrop, iters [ch] and the active count
     st = diag_begin(s, ch, slot, [&](DiagCarve& m, size_t, Slot& z) {
         lbl_take(m, ch, z.lbl);
         z.Tb = m.take<double>(ch * NLAY);
@@ -2819,6 +2880,7 @@ int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vm
         z.H = m.take<double>(ch * FJAC_NH);
         z.part = m.take<double>(nchunks * ch * 2 * NLEV);
         z.dt = m.take<double>(ch);
+        ecs_grad_take(m, ch, nspan, grad, z.g);
         z.time = m.take<float>(ch);
         z.ntrop = m.take<int>(ch);
         z.iters = m.take<int>(ch);
@@ -2915,17 +2977,88 @@ int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vm
         if (tau3) z.a.tau3 = tau3;
         return check(z, k);
     };
+    // the flux Jacobian at the solution (Tp, Tsp: never the copies the finish has moved; sH and sO as the last retemper and
+    // the scaling left them), the adjoint solve and the sweep with the composed planes, then the epilogue's downloads
+    auto epilogue = [&](const Slot& z) -> int {
+        LblArgs a = z.a;
+        a.Tlayer = z.Tp;
+        a.Tsurf = z.Tsp;
+        CU(rcm_launch_lbl_fjac(a, wtau, z.J, z.H, z.q));
+        CU(rcm_launch_ecs_adjoint(ecs_args(z), z.g.dF, z.g.co, z.q));
+        CU(rcm_launch_lbl_grad(a, wtau, raw, sc.f[1] * s->lbl_co2_factor, sc.f[4], sc.f[3], z.g.co, z.g.part, z.q));
+        CU(rcm_launch_grad_sum(a.ncol, (int)nspan, z.g.part, z.g.sum, z.q));
+        s->launches += 4;
+        return ecs_grad_download(s, *grad, z.g, (size_t)(z.c0 - col0), z.n, z.q);
+    };
     auto download = [&](const Slot& z) -> int {
+        if (grad && (st = epilogue(z)) != RCM_OK) return st;
         const size_t r = (size_t)(z.c0 - col0);
-        if (F) CU(cudaMemcpyAsync(F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
-        if (dT) CU(cudaMemcpyAsync(dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
-        if (dTs) CU(cudaMemcpyAsync(dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
-        if (E_down) CU(cudaMemcpyAsync(E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
-        if (E_up) CU(cudaMemcpyAsync(E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
-        if (iters) CU(cudaMemcpyAsync(iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
+        if (o.F) CU(cudaMemcpyAsync(o.F + r * 2, z.F, z.n * 2 * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.dT) CU(cudaMemcpyAsync(o.dT + r * NLAY, z.dT, z.n * NLAY * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.dTs) CU(cudaMemcpyAsync(o.dTs + r, z.dTs, z.n * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.E_down) CU(cudaMemcpyAsync(o.E_down + r * NLEV, z.Edo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.E_up) CU(cudaMemcpyAsync(o.E_up + r * NLEV, z.Euo, z.n * NLEV * D, cudaMemcpyDeviceToHost, z.q));
+        if (o.iters) CU(cudaMemcpyAsync(o.iters + r, z.iters, z.n * sizeof(int), cudaMemcpyDeviceToHost, z.q));
         return RCM_OK;
     };
     return fdh_schedule(s, slot, col0, ncol, ch, start, check, newton, download);
+}
+
+// The gradient calls around ecs_response / lbl_ecs_response (run): dTs_dF into a buffer of their own when the caller wants
+// dTs_dlnx alone, and after the call a row of quiet NaN in dTs_dlnx wherever the adjoint kernel wrote one in dTs_dF (the
+// response did not converge, or A at the solution could not be solved).
+template <class Run>
+int ecs_gradient(int ncol, double* dTs_dF, double* dTs_dlnx, Run run) {
+    std::vector<double> own;
+    if (!dTs_dF && dTs_dlnx && ncol > 0) {
+        own.resize((size_t)ncol * NLEV);
+        dTs_dF = own.data();
+    }
+    const EcsGrad g{dTs_dF, dTs_dlnx};
+    const int st = run(g);
+    if (st != RCM_OK || !dTs_dlnx) return st;
+    for (int c = 0; c < ncol; ++c)
+        if (std::isnan(dTs_dF[(size_t)c * NLEV + NLAY]))
+            std::fill(dTs_dlnx + (size_t)c * SPJ_NE, dTs_dlnx + (size_t)(c + 1) * SPJ_NE, std::numeric_limits<double>::quiet_NaN());
+    return RCM_OK;
+}
+
+}  // namespace
+}  // extern "C++"
+
+int rcm_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh, double tol,
+                         int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up, int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    return ecs_response(s, "rcm_climate_response", col0, ncol, vmr_scale, ntrop, fixed_rh, tol, max_iter,
+                        EcsOut{F, dT, dTs, E_down, E_up, iters}, nullptr);
+}
+
+int rcm_lbl_climate_response(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
+                             double tol, int max_iter, double* F, double* dT, double* dTs, double* E_down, double* E_up,
+                             int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    return lbl_ecs_response(s, "rcm_lbl_climate_response", col0, ncol, vmr_scale, ntrop, fixed_rh, tol, max_iter,
+                            EcsOut{F, dT, dTs, E_down, E_up, iters}, nullptr);
+}
+
+// Climate-response gradients: the response with its epilogue, of the response's outputs only dTs and iters.
+int rcm_climate_response_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop, int fixed_rh,
+                                  double tol, int max_iter, double* dTs, double* dTs_dF, double* dTs_dlnx, int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    return ecs_gradient(ncol, dTs_dF, dTs_dlnx, [&](const EcsGrad& g) {
+        return ecs_response(s, "rcm_climate_response_gradient", col0, ncol, vmr_scale, ntrop, fixed_rh, tol, max_iter,
+                            EcsOut{nullptr, nullptr, dTs, nullptr, nullptr, iters}, &g);
+    });
+}
+
+int rcm_lbl_climate_response_gradient(rcm_solver* s, int col0, int ncol, const double* vmr_scale, const int* ntrop,
+                                      int fixed_rh, double tol, int max_iter, double* dTs, double* dTs_dF, double* dTs_dlnx,
+                                      int* iters) {
+    if (!s) return RCM_ERR_ARG;
+    return ecs_gradient(ncol, dTs_dF, dTs_dlnx, [&](const EcsGrad& g) {
+        return lbl_ecs_response(s, "rcm_lbl_climate_response_gradient", col0, ncol, vmr_scale, ntrop, fixed_rh, tol,
+                                max_iter, EcsOut{nullptr, nullptr, dTs, nullptr, nullptr, iters}, &g);
+    });
 }
 
 // ------------------------------------------------------------------------------------------

@@ -44,5 +44,8 @@ cudaError_t rcm_launch_ecs_retemper(const EcsArgs& a, cudaStream_t st);
 cudaError_t rcm_launch_lbl_ecs_retemper(const EcsArgs& a, cudaStream_t st);
 cudaError_t rcm_launch_ecs_check(const EcsArgs& a, cudaStream_t st);
 cudaError_t rcm_launch_ecs_newton(const EcsArgs& a, cudaStream_t st);
+// the adjoint of the converged response (rcm_ecs_adj_kernels.cuh): dF [ncol][21] = dTs / d(forcing term of equation i) and
+// co [ncol][42], the level cotangents of the gradient sweep that give dTs / dp
+cudaError_t rcm_launch_ecs_adjoint(const EcsArgs& a, double* dF, double* co, cudaStream_t st);
 
 #endif

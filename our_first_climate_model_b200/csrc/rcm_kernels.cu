@@ -209,6 +209,7 @@ __global__ void __launch_bounds__(256) rcm_microbench_kernel(double* out, long i
 #include "rcm_lbl_jac_kernels.cuh"
 #include "rcm_lbl_fjac_kernels.cuh"
 #include "rcm_ecs_kernels.cuh"
+#include "rcm_ecs_adj_kernels.cuh"
 #include "rcm_species_kernels.cuh"
 #include "rcm_lbl_species_kernels.cuh"
 #include "rcm_grad_kernels.cuh"
@@ -583,6 +584,11 @@ cudaError_t rcm_launch_ecs_check(const EcsArgs& a, cudaStream_t st) {
 
 cudaError_t rcm_launch_ecs_newton(const EcsArgs& a, cudaStream_t st) {
     rcm_ecs_newton_kernel<<<(a.ncol + ECS_NEWTON_WARPS - 1) / ECS_NEWTON_WARPS, ECS_NEWTON_NT, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t rcm_launch_ecs_adjoint(const EcsArgs& a, double* dF, double* co, cudaStream_t st) {
+    rcm_ecs_adjoint_kernel<<<(a.ncol + ECS_NEWTON_WARPS - 1) / ECS_NEWTON_WARPS, ECS_NEWTON_NT, 0, st>>>(a, dF, co);
     return cudaGetLastError();
 }
 
